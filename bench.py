@@ -6,6 +6,7 @@
   python bench.py --impl reference --steps 100 --warmup 5              # the CPU arm: the UNMODIFIED reference (baseline/_ref),
                                                                        #   one process per host core; C port of it as a second figure
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+  python bench.py --steps 100 --warmup 5 --dump-outputs bench_outputs   # also writes what the last timed step returned, as .npy
 
 Default workload (config.workload): BASELINE.json configs[2] — Knuffingen map, 480x640 `classes` observations (5x480x640 u8 =
 1 536 000 B per env-step), Stanley-controller actions with lanepath CTE / heading info consumed every step, auto-reset of
@@ -13,12 +14,18 @@ finished envs; 16384 envs per GPU (weak scaling: per-GPU work is fixed, envs sha
 all-gathers episode statistics).
 
 A "step" is one lockstep pass of the hot path over all envs of the rank. `value` is measured with the action tensors already on
-the device (CUDA events on the launching stream, max over ranks); `sustained` repeats that for --min-seconds; `e2e` drives the
+the device (CUDA events on the launching stream, max over ranks) over exactly --steps steps; `sustained` (only with --min-seconds)
+repeats that for a clock-determined number of steps; `e2e` drives the
 same step from pinned HOST buffers (actions in, reward / flags / CTE / heading out, stream synchronised every step; observations
 stay device-resident as the vectorised API defines); `e2e_obs_to_host` additionally brings the observations to the host
 (bit-packed); `roofline` is the render kernel's algorithmic bytes over its own event-timed duration.
+
+--dump-outputs DIR writes what the headline's last timed step returned to its caller (observations, reward, terminated,
+truncated, every info tensor; rank 0's envs) as DIR/<name>.npy in float32 / float64, at most 64 MB in all. Inputs depend only on
+the arguments (seeded resets and policy), so two builds of the library can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -27,6 +34,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the tree may be read-only: bench.py writes nothing into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "baseline"))
@@ -79,6 +87,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "50", "-i",
                                           str(self.gpu)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # no sampler outlives a run that fails before stop()
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -279,6 +288,33 @@ def build_env(w, N, dev, rank, world):
     return env, [base], max_steer
 
 
+DUMP_BUDGET = {"obs": 47_000_000, "rest": 16_000_000}   # bytes; with the .npy headers the whole dump stays under 64 MB
+
+
+def sample_outputs(ret):
+    """Host copies of what env.step() returned -> {name: ndarray}: obs (obs_g<i> per resolution group), reward, terminated,
+    truncated, info_<key>. float64 data and 32/64-bit integers become float64, everything else float32 (both exact). An array
+    over its share of the budget keeps a fixed, seeded sample of its envs (dim 0), whose indices are stored as <name>_rows."""
+    import torch
+    obs, reward, term, trunc, info = ret
+    groups = {"obs": obs} if torch.is_tensor(obs) else {f"obs_g{i}": o for i, o in enumerate(obs)}
+    rest = {"reward": reward, "terminated": term, "truncated": trunc, **{f"info_{k}": v for k, v in info.items()}}
+    out = {}
+    for part, arrays in (("obs", groups), ("rest", rest)):
+        share = DUMP_BUDGET[part] // len(arrays)
+        for name, t in arrays.items():
+            dt = torch.float64 if t.dtype in (torch.float64, torch.int32, torch.int64) else torch.float32
+            n = t.shape[0]
+            row_bytes = (t.numel() // max(n, 1)) * dt.itemsize
+            k = min(n, max(share // (row_bytes + 8), 1))
+            if k < n:
+                rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+                t = t[torch.from_numpy(rows).to(t.device)]
+                out[name + "_rows"] = rows.astype(np.float64)
+            out[name] = t.to(dt).cpu().numpy()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -288,13 +324,17 @@ def main():
     ap.add_argument("--config", type=int, default=3, choices=[1, 2, 3, 4, 5], help="BASELINE.json config (1-based); 3 is the one the metric is quoted on")
     ap.add_argument("--envs-per-gpu", type=int, default=0, help="override the config's env count per GPU")
     ap.add_argument("--graph-steps", type=int, default=5, help="env steps captured per CUDA-graph replay (launch-bound configs)")
-    ap.add_argument("--min-seconds", type=float, default=3.0, help="length of the sustained device-timed run reported next to the K-step one")
+    ap.add_argument("--min-seconds", type=float, default=0.0, help="length of a sustained device-timed run reported next to the K-step one "
+                    "(0: none, so that --steps alone sets how many steps are timed)")
     ap.add_argument("--cpu-envs", type=int, default=0, help="envs of the C-port sample (default: 128 x host threads, at most 2048: 3 GB of frames)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="length of the cpu_baseline samples")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-fill-context", action="store_true", help="skip the memset / zero-fill context numbers (keeps ncu launch lists clean)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -343,7 +383,8 @@ def main():
         return {"car_control": cc, "maneuver": maneuver}
 
     def step_device():
-        _, reward, term, trunc, info = env.step(act())
+        state["ret"] = env.step(act())
+        _, reward, term, trunc, info = state["ret"]
         state["info"] = info
         stats.update(reward, term, trunc)
         state["t"] += 1
@@ -387,25 +428,12 @@ def main():
         dist.all_reduce(elapsed_ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(elapsed_ms.item()) / args.steps
     value = N * world / (ms_per_step * 1e-3)
+    dump = None
+    if args.dump_outputs and rank == 0 and not graph_stepped(w, N):
+        dump = sample_outputs(state["ret"])
 
-    # ---- the same loop for at least --min-seconds (clocks and power settle): the sustained figure
-    sustained = None
-    if args.min_seconds > 0:
-        chunk = max(args.steps, 10)
-        n_chunks = max(int(np.ceil(args.min_seconds * 1e3 / (ms_per_step * chunk))), 1)
-        barrier()
-        e0.record()
-        for _ in range(n_chunks * chunk):
-            step_device()
-        e1.record()
-        barrier()
-        s_ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
-        if world > 1:
-            dist.all_reduce(s_ms, op=dist.ReduceOp.MAX)
-        sustained = {"value": N * world * n_chunks * chunk / (float(s_ms.item()) * 1e-3), "unit": UNIT, "seconds": float(s_ms.item()) * 1e-3,
-                     "steps": n_chunks * chunk}
-
-    # ---- launch-bound configs: the policy + step captured in a CUDA graph (TinyCarloVecEnv.capture), replayed
+    # ---- launch-bound configs: the policy + step captured in a CUDA graph (TinyCarloVecEnv.capture), replayed. It runs before
+    # the clock-determined sustained loop, so that its last step, the headline's, depends on the arguments only.
     graph = None
     if graph_stepped(w, N):
         per = args.graph_steps if args.graph_steps > 0 and args.steps % args.graph_steps == 0 else 1   # env steps per replay; K stays exact
@@ -423,6 +451,25 @@ def main():
             dist.all_reduce(g_ms, op=dist.ReduceOp.MAX)
         graph = {"value": N * world * args.steps / (float(g_ms.item()) * 1e-3), "unit": UNIT, "ms_per_step": float(g_ms.item()) / args.steps,
                  "note": f"policy ops + step captured once with TinyCarloVecEnv.capture(steps={per}) and replayed: one graph launch per {per} step(s)"}
+        if args.dump_outputs and rank == 0:   # the replays wrote into the buffers the eager step returned views of
+            dump = sample_outputs(state["ret"])
+
+    # ---- the same loop for at least --min-seconds (clocks and power settle): the sustained figure
+    sustained = None
+    if args.min_seconds > 0:
+        chunk = max(args.steps, 10)
+        n_chunks = max(int(np.ceil(args.min_seconds * 1e3 / (ms_per_step * chunk))), 1)
+        barrier()
+        e0.record()
+        for _ in range(n_chunks * chunk):
+            step_device()
+        e1.record()
+        barrier()
+        s_ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(s_ms, op=dist.ReduceOp.MAX)
+        sustained = {"value": N * world * n_chunks * chunk / (float(s_ms.item()) * 1e-3), "unit": UNIT, "seconds": float(s_ms.item()) * 1e-3,
+                     "steps": n_chunks * chunk}
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- config 5: per-group kernel times from a serial pass (the groups normally overlap on separate streams)
@@ -617,6 +664,10 @@ def main():
             "sustained": sustained, "cuda_graph": graph, "clocks": clocks, "e2e": e2e, "e2e_obs_to_host": e2e_obs, "gpu_launches": n_launch,
             "roofline": roofline, "cpu_baseline": cpu_baseline, "cpu_baseline_port": cpu_port, "library": {"so_hash": so_hash}, "setup": SETUP or None,
             "episode_stats": {"finished": st[0], "truncated": st[1], "reward_sum": st[2], "env_steps": st[3]}}
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

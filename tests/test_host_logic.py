@@ -212,6 +212,40 @@ def test_bench_reference_arm_prints_the_contract_line(config):
         assert d["config"] == bench.config_dict(WL.WORKLOADS[3], A, 1)      # what the CUDA arm prints: the driver's same_config check
 
 
+def test_bench_dump_sample_is_exact_fixed_and_bounded():
+    """bench.py --dump-outputs: the arrays a step returned, as float32 / float64 holding the same values, under 64 MB for the
+    largest configurations (16384 envs of 5x480x640 frames; three resolution groups), and the same env sample on every run."""
+    import sys
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n = 16384
+    ids = torch.arange(n)
+    obs = (ids % 251).to(torch.uint8).view(n, 1, 1, 1).expand(n, 5, 480, 640)     # frame of env i is i % 251 everywhere
+    flags = (ids % 3 == 0)
+    info = {"cte": ids.to(torch.float32) / 7, "nearest_edge": (ids.to(torch.int32) * 131071).view(n, 1).expand(n, 5),
+            "local_path": torch.rand(n, 4, 2)}
+
+    def nbytes(d):
+        return sum(a.nbytes + 128 for a in d.values())   # + the .npy header
+    d = bench.sample_outputs((obs, ids.to(torch.float32), flags, ~flags, info))
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values()) and nbytes(d) <= 64_000_000
+    rows = d["obs_rows"].astype(np.int64)
+    assert 0 < len(rows) < n and np.all(np.diff(rows) > 0)
+    assert np.array_equal(d["obs"], np.broadcast_to((rows % 251).reshape(-1, 1, 1, 1), (len(rows), 5, 480, 640)).astype(np.float32))
+    assert np.array_equal(d["reward"], np.arange(n, dtype=np.float32)) and np.array_equal(d["terminated"], (np.arange(n) % 3 == 0).astype(np.float32))
+    assert d["info_nearest_edge"].dtype == np.float64 and d["info_nearest_edge"][n - 1, 4] == (n - 1) * 131071
+    assert np.array_equal(d["info_cte"], info["cte"].numpy()) and np.array_equal(d["info_local_path"], info["local_path"].numpy())
+    assert np.array_equal(bench.sample_outputs((obs, ids.to(torch.float32), flags, ~flags, info))["obs_rows"], d["obs_rows"])
+    # config 5: one observation tensor per resolution group
+    sizes, res = [10880, 10880, 11008], [(84, 84), (128, 160), (240, 320)]
+    groups = [torch.zeros((1, 5, h, w), dtype=torch.uint8).expand(s, 5, h, w) for s, (h, w) in zip(sizes, res)]
+    m = sum(sizes)
+    d = bench.sample_outputs((groups, torch.zeros(m), torch.zeros(m, dtype=torch.bool), torch.zeros(m, dtype=torch.bool),
+                              {"local_path_nodes": torch.zeros((m, 4, 2), dtype=torch.int32)}))
+    assert {"obs_g0", "obs_g1", "obs_g2", "info_local_path_nodes"} <= set(d) and nbytes(d) <= 64_000_000
+
+
 def test_shard_groups_partition_every_group():
     from tinycarlo_b200.distributed import shard_groups
     sizes = [10922, 10922, 10924]
