@@ -79,16 +79,12 @@ struct TcHandle {
     int rows_per_band_rgb = 0, n_bands_rgb = 0, plane_words_rgb = 0;
     size_t track_smem = 0, proj_smem = 0, render_smem = 0;
     int max_edges = 0, plane_words_full = 0;
-    int stagger_ns = 0, n_sms = 148;
+    int n_sms = 148;
     int track_group = 32;       // lanes per env of tc_track_kernel (32 or 8)
     int track_per_thread = 1;   // tc_track_thread_kernel (one thread per env) instead of tc_track_kernel (a warp per env)
     long long *timeline = nullptr;
-    bool fused_ok = false;
-    int render_threads = 256;
-    // fused kernel geometry: per class (large frames) or all classes per block (small frames)
-    int fused_all = 0, fused_nodes = 0, fused_edges = 0, fused_cblob = 0, fused_words = 0;
-    TcClassBlob all_desc{};
-    int32_t edge_off_h[TC_MAX_CLASSES + 1] = {0};
+    bool fused_ok = false;      // tc_render_classes_kernel's block fits (or fused_all)
+    int fused_all = 0;          // small frames: a block per env renders all classes (tc_render_env_kernel / tc_render_envs_kernel)
     // block-per-env kernel: visible-set tables (tc_cull.h), rebuilt when the camera parameters change
     std::vector<int32_t> m_node_off, m_edge_off, m_edges; // host copy of the laneline tables (the builder's input)
     std::vector<double> m_nodes;
@@ -107,12 +103,11 @@ struct TcHandle {
     size_t env_smem = 0;     // tc_render_env_kernel (small frames)
     // two-kernel path of large bit-packed frames (tc_prims_kernel + tc_draw_class_kernel): buffers allocated at first use
     TcPrimsOut prims{};
-    int prims_on = 1;
     int env_blocks = 0;      // resident blocks per SM of the packed kernel as chosen (diagnostics)
     int env_pack = 0, env_chunks = 1;   // > 0: tc_render_envs_kernel with that many envs per block
     size_t envs_smem = 0;
     size_t envb_smem = 0;    // tc_render_env_banded_kernel (large frames, RGB / 1 bit per pixel); 0: not available
-    int envb_rows = 0, envb_bands = 0, envb_words = 0, envb_on = 1;
+    int envb_rows = 0, envb_bands = 0, envb_words = 0;
     double cull_radius = -1.0, cull_mean_nodes = 0.0;
     bool cull_built_once = false;
     int cull_cells = 0, cull_max_nodes = 0;
@@ -186,9 +181,7 @@ static int tc_install_cull(TcHandle *h, double radius) {
     const auto t0 = std::chrono::steady_clock::now();
     TcCull cull;
     TcMapDesc m = tc_host_map(h);
-    double cell = 0.25;
-    if (const char *cs = getenv("TC_CULL_CELL")) cell = atof(cs) > 0 ? atof(cs) : cell;
-    tc_build_cull(&m, radius, cell, 0.05, cull);
+    tc_build_cull(&m, radius, 0.25, 0.05, cull);
     TcCullSet c;
     c.key = radius;
     const size_t np = tc_env_np(cull.max_nodes, cull.max_edges);
@@ -206,7 +199,7 @@ static int tc_install_cull(TcHandle *h, double radius) {
         // The packed small-frame kernel (tc_render_envs_kernel, 3 blocks of 256 threads per SM): E envs per block and 1 or 2
         // 32-segment chunks of primitive slots, chosen for the most envs in flight per SM without dropping below 3 blocks per SM
         // (fewer blocks hide the latency-bound phases worse than fuller lanes gain); E = 1 never beats tc_render_env_kernel
-        // (measured), which stays the fallback. TC_ENV_PACK=0|2|4 and TC_ENV_CHUNKS=1|2 override.
+        // (measured), which stays the fallback. TC_ENV_PACK=0 selects the one-env kernel, so that tests reach it where the packed one would run.
         int pack = 0, chunks = 1, nblocks = 0;
         if (h->fused_all) {
             int best = 0;
@@ -221,12 +214,7 @@ static int tc_install_cull(TcHandle *h, double radius) {
                     // (at 2 blocks per SM the packed kernel loses to the one-env kernel at 4: config 5's wide cameras, 0.42 vs 0.35 ms)
                     if (blocks >= 3 && ee * blocks > best) { best = ee * blocks; pack = ee; chunks = cc; nblocks = blocks; }
                 }
-            if (const char *pe = getenv("TC_ENV_PACK")) {
-                const int v = atoi(pe);
-                pack = (v == 1 || v == 2 || v == 4) ? v : 0;
-            }
-            if (const char *pc = getenv("TC_ENV_CHUNKS")) chunks = atoi(pc) == 2 ? 2 : 1;
-            if (pack && tc_envs_smem_bytes(pack, np, cull.max_bytes, h->env_words, chunks) > 200 * 1024) pack = 0;
+            if (const char *pe = getenv("TC_ENV_PACK")) if (atoi(pe) == 0) pack = 0;
         }
         c.pack = pack; c.chunks = chunks; c.blocks = nblocks;
         c.envs_smem = pack ? tc_envs_smem_bytes(pack, np, cull.max_bytes, h->env_words, chunks) : 0;
@@ -324,16 +312,13 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     TC_TRYH(tc_dev_alloc(h, &h->d_cblob_desc, (size_t)C));
     TC_CUDAH(cudaMemcpy(h->d_cblob_desc, pk.cblob_desc.data(), sizeof(TcClassBlob) * C, cudaMemcpyHostToDevice));
     h->max_cblob_bytes = pk.max_cblob_bytes;
-    h->all_desc = pk.all_desc;
-    for (int c = 0; c <= C; c++) h->edge_off_h[c] = map->ll_edge_off[c];
     TC_TRYH(tc_dev_alloc(h, &h->d_edge_off, (size_t)C + 1));
     TC_CUDAH(cudaMemcpy(h->d_edge_off, map->ll_edge_off, (size_t)(C + 1) * 4, cudaMemcpyHostToDevice));
 
     {
         // nearest-laneline index: ~16k ground cells over the laneline bounding box + 1 m (farther out the kernel scans all edges)
         TcNear nr;
-        const char *ne = getenv("TC_NEAR_INDEX");
-        if (!(ne && atoi(ne) == 0)) tc_build_near(map, 1.0, 16384, nr);
+        tc_build_near(map, 1.0, 16384, nr);
         if (nr.nx > 0) {
             TC_TRYH(tc_dev_alloc(h, &h->d_near_off, nr.off.size()));
             TC_CUDAH(cudaMemcpy(h->d_near_off, nr.off.data(), nr.off.size() * 4, cudaMemcpyHostToDevice));
@@ -370,18 +355,13 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     h->proj_smem = tc_proj_smem_bytes(h->max_nodes);
     const size_t plane_budget = 48 * 1024;
     tc_band_geometry(h->H, h->W, 1, plane_budget, &h->rows_per_band_cls, &h->n_bands_cls, &h->plane_words_cls);
-    {
-        size_t rgb_budget = 64 * 1024;   // measured on 480x640: 24/32/40/48/64/96 KB -> 3.02/2.64/2.64/2.49/2.32/4.84 ms per 8192 envs
-        if (const char *kb = getenv("TC_RGB_PLANE_KB")) rgb_budget = (size_t)std::max(4, atoi(kb)) * 1024;
-        tc_band_geometry(h->H, h->W, C, rgb_budget, &h->rows_per_band_rgb, &h->n_bands_rgb, &h->plane_words_rgb);
-    }
+    // measured on 480x640: 24/32/40/48/64/96 KB -> 3.02/2.64/2.64/2.49/2.32/4.84 ms per 8192 envs
+    tc_band_geometry(h->H, h->W, C, 64 * 1024, &h->rows_per_band_rgb, &h->n_bands_rgb, &h->plane_words_rgb);
     for (int c = 0; c < C; c++) h->max_edges = std::max(h->max_edges, map->ll_edge_off[c + 1] - map->ll_edge_off[c]);
     {
         cudaDeviceProp prop;
         TC_CUDAH(cudaGetDeviceProperties(&prop, device));
         h->n_sms = prop.multiProcessorCount;
-        const char *sg = getenv("TC_STAGGER_NS"); // tuning knob for the first-wave stagger of the fused render kernel
-        if (sg) h->stagger_ns = atoi(sg);
     }
     h->plane_words_full = (int)(((size_t)h->H * h->W + 31) / 32) + 1;
     {
@@ -395,19 +375,12 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
         // measured (Knuffingen 240x320, 8192 envs): block per env 0.56 ms against 1.05 ms for the per-class blocks, which pay the
         // camera pass and the set-up once per class; beyond ~75 KB a block (3 per SM) the per-class kernel's finer blocks win again
         // (the camera reach, hence the size of the visible-set tables, is not known yet: the plane is what decides)
-        bool all = smem_all <= 100 * 1024 && (size_t)words_all * 4 <= 50 * 1024;
-        if (const char *fa = getenv("TC_FUSED_ALL")) all = atoi(fa) != 0 && smem_all <= 200 * 1024;
+        const bool all = smem_all <= 100 * 1024 && (size_t)words_all * 4 <= 50 * 1024;
         h->fused_all = all ? 1 : 0;
-        h->fused_nodes = h->max_nodes; h->fused_edges = h->max_edges;
-        h->fused_cblob = h->max_cblob_bytes; h->fused_words = h->plane_words_full;
         h->render_smem = smem_one;
         h->env_words = words_all;
-        {
-            size_t eb = 30 * 1024;   // C band planes + their OR; with 24*np and the primitive slots of 48 segments: 4 blocks per SM on Knuffingen
-            if (const char *kb = getenv("TC_ENVB_PLANE_KB")) eb = (size_t)std::max(4, atoi(kb)) * 1024;
-            tc_band_geometry(h->H, h->W, C + 1, eb, &h->envb_rows, &h->envb_bands, &h->envb_words);
-            if (const char *on = getenv("TC_ENV_BANDED")) h->envb_on = atoi(on) != 0;
-        }
+        // C band planes + their OR in 30 KB; with 24*np and the primitive slots of 48 segments: 4 blocks per SM on Knuffingen
+        tc_band_geometry(h->H, h->W, C + 1, 30 * 1024, &h->envb_rows, &h->envb_bands, &h->envb_words);
         h->fused_ok = all || smem_one <= 56 * 1024; // >= 4 blocks per SM; larger frames take the banded two-kernel path
     }
 #define TC_PREP_RENDER(K)                 \
@@ -417,15 +390,12 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     TC_PREP_RENDER((tc_render_env_banded_kernel<TC_FMT_BITS>));
     TC_PREP_RENDER((tc_prims_kernel<256, 2>));
     TC_PREP_RENDER((tc_draw_class_kernel<256, TC_FMT_BITS>));
-    if (const char *po = getenv("TC_PRIMS_PATH")) h->prims_on = atoi(po) != 0;
     if (h->fused_ok) {
-        if (const char *rt = getenv("TC_RENDER_THREADS")) h->render_threads = atoi(rt) == 128 ? 128 : 256;
-        TC_PREP_RENDER((tc_render_env_kernel<128, TC_FMT_U8>));
         TC_PREP_RENDER((tc_render_env_kernel<256, TC_FMT_U8>));
         TC_PREP_RENDER((tc_render_env_kernel<256, TC_FMT_RGB>));
         TC_PREP_RENDER((tc_render_env_kernel<256, TC_FMT_BITS>));
         TC_PREP_RENDER((tc_render_env_kernel<256, TC_FMT_BF16>));
-#define TC_PREP_ENVS(F) TC_PREP_RENDER((tc_render_envs_kernel<256, F, 1>)); TC_PREP_RENDER((tc_render_envs_kernel<256, F, 2>)); TC_PREP_RENDER((tc_render_envs_kernel<256, F, 4>))
+#define TC_PREP_ENVS(F) TC_PREP_RENDER((tc_render_envs_kernel<256, F, 2>)); TC_PREP_RENDER((tc_render_envs_kernel<256, F, 4>))
         TC_PREP_ENVS(TC_FMT_U8); TC_PREP_ENVS(TC_FMT_RGB); TC_PREP_ENVS(TC_FMT_BITS); TC_PREP_ENVS(TC_FMT_BF16);
 #undef TC_PREP_ENVS
         TC_PREP_RENDER((tc_render_classes_kernel<256, TC_FMT_U8>));
@@ -442,14 +412,12 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     TC_CUDAH(tc_allow_max_smem(tc_track_kernel<8>));
     TC_CUDAH(tc_allow_max_smem(tc_track_thread_kernel));
     TC_CUDAH(cudaFuncSetAttribute(tc_track_thread_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    // a warp per env pays off only when there are too few envs to fill the SMs with one thread each (TC_TRACK_MODE=warp|thread overrides)
+    // a warp per env pays off only when there are too few envs to fill the SMs with one thread each
     // measured: 4096 envs 0.033 (8 lanes per env) vs 0.062 ms (thread), 8192 envs 0.035 vs 0.062, 32768 envs 0.187 (warp) vs 0.044 ms:
     // a thread per env once 8 lanes per env would need more than one wave of warps (3 blocks x 8 warps per SM)
     h->track_per_thread = num_envs / 4 > 3 * 8 * h->n_sms ? 1 : 0;
-    if (const char *tm = getenv("TC_TRACK_MODE")) h->track_per_thread = (tm[0] == 't' || tm[0] == '1') ? 1 : 0;
     // below that: 8 lanes per env once a warp per env would need more than one wave of warps (3 blocks x 8 warps per SM), else a warp per env
     h->track_group = num_envs > 3 * 8 * h->n_sms / 2 ? 8 : 32;
-    if (const char *tg = getenv("TC_TRACK_GROUP")) h->track_group = atoi(tg) == 8 ? 8 : 32;
     TC_CUDAH(tc_allow_max_smem(tc_project_kernel));
     TC_CUDAH(tc_allow_max_smem(tc_raster_classes_kernel));
     TC_CUDAH(tc_allow_max_smem(tc_raster_rgb_kernel));
@@ -536,74 +504,94 @@ int tc_set_wrapped(TcHandle *h, int32_t wrapped) {
     return TC_OK;
 }
 
+enum class TcRenderPath {
+    ENVS,      // tc_render_envs_kernel: small frames, E envs per block
+    ENV,       // tc_render_env_kernel: small frames, one env per block
+    PRIMS,     // tc_prims_kernel + tc_draw_class_kernel (+ the banded kernel for overflowing envs): large bit-packed frames
+    BANDED,    // tc_render_env_banded_kernel: large RGB / bit-packed frames, bands walked inside a block per env
+    CLASSES,   // tc_render_classes_kernel: a block per (env, class), the frame in one plane
+    UNFUSED,   // tc_project_kernel + a raster kernel: segment export, frames too large for the fused kernels
+};
+
+// The render kernels a launch runs, from the handle's geometry (tc_create, tc_install_cull), the format and what is asked for.
+// timeline: per-block phase clocks are wanted (tools/timeline.py), which the packed kernel does not write.
+static TcRenderPath tc_render_path(const TcHandle *h, int obs_format, bool segments, bool timeline) {
+    using P = TcRenderPath;
+    const bool bits = obs_format == TC_OBS_CLASSES_BITS;
+    if (segments) return P::UNFUSED;
+    if (h->fused_all) return h->env_pack > 0 && !timeline ? P::ENVS : P::ENV;
+    if (h->envb_smem > 0 && bits && (h->H * h->W) % 128 == 0 && (size_t)h->plane_words_full * 4 <= 64 * 1024) return P::PRIMS;
+    if (h->envb_smem > 0 && (bits || obs_format == TC_OBS_RGB)) return P::BANDED;
+    if (h->fused_ok && obs_format != TC_OBS_RGB) return P::CLASSES;
+    return P::UNFUSED;
+}
+
+// arguments of the block-per-env kernels; plane_words: words of the stacked plane of the small-frame kernels, 0 for the others
+static TcRenderEnvArgs tc_render_env_args(const TcHandle *h, const uint8_t *mask, uint8_t *obs, int plane_words) {
+    TcRenderEnvArgs ea;
+    ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = h->n_envs; ea.n_classes = h->C;
+    ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = plane_words;
+    ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = obs;
+    memcpy(ea.colors, h->colors, sizeof(ea.colors));
+    ea.timeline = nullptr;
+    ea.rows_per_band = h->envb_rows; ea.n_bands = h->envb_bands; ea.band_words = h->envb_words;
+    ea.region_bytes = (int)tc_envs_region_bytes((size_t)h->env_np, h->env_max_bytes, plane_words);
+    ea.prim_chunks = 1;
+    return ea;
+}
+
 static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int obs_format, int32_t *seg_count_out, int32_t *seg_out,
                             cudaStream_t st, cudaEvent_t after_project = nullptr) {
+    using P = TcRenderPath;
     const int N = h->n_envs, C = h->C;
+    long long *timeline = mask ? nullptr : h->timeline;
+    const P path = tc_render_path(h, obs_format, seg_count_out || seg_out, timeline != nullptr);
     if (obs_format == TC_OBS_CLASSES_BITS || obs_format == TC_OBS_CLASSES_BF16) {
-        const bool banded = obs_format == TC_OBS_CLASSES_BITS && !h->fused_all && h->envb_on && h->envb_smem > 0;
-        if ((!h->fused_ok && !banded) || seg_count_out || seg_out) return tc_fail(TC_ERR_INVALID, "bit-packed / bf16 observations need the fused render path (frame too large or debug segments requested)");
+        if (path == P::UNFUSED) return tc_fail(TC_ERR_INVALID, "bit-packed / bf16 observations need the fused render path (frame too large or debug segments requested)");
         if (obs_format == TC_OBS_CLASSES_BF16 && (h->H * h->W) % 8 != 0) return tc_fail(TC_ERR_INVALID, "bf16 observations need H*W to be a multiple of 8");
-        if (obs_format == TC_OBS_CLASSES_BITS && h->fused_all && (h->H * h->W) % 32 != 0) return tc_fail(TC_ERR_INVALID, "bit-packed observations of small frames need H*W to be a multiple of 32");
+        if (obs_format == TC_OBS_CLASSES_BITS && (path == P::ENVS || path == P::ENV) && (h->H * h->W) % 32 != 0) return tc_fail(TC_ERR_INVALID, "bit-packed observations of small frames need H*W to be a multiple of 32");
     }
-    if (obs && h->fused_ok && h->fused_all && !seg_count_out && !seg_out) {
-        TcRenderEnvArgs ea;
-        ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = N; ea.n_classes = C;
-        ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = h->env_words;
-        ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = obs;
-        memcpy(ea.colors, h->colors, sizeof(ea.colors));
-        ea.timeline = mask ? nullptr : h->timeline;
-        if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
-        const size_t sm = h->env_smem;
-        if (h->env_pack > 0 && !ea.timeline) {
-            const int E = h->env_pack, grid = (N + E - 1) / E;
-            const size_t sme = h->envs_smem;
-            ea.region_bytes = (int)tc_envs_region_bytes((size_t)h->env_np, h->env_max_bytes, h->env_words);
-            ea.prim_chunks = h->env_chunks;
+    const P launch = obs ? path : P::UNFUSED;   // without a frame only the camera pass runs
+    if (launch == P::PRIMS && !h->prims.prims) {
+        TC_TRY(tc_dev_alloc(h, &h->prims.prims, (size_t)N * TC_PRIMS_CAP * TC_PRIMS_SEG_WORDS));
+        TC_TRY(tc_dev_alloc(h, &h->prims.cls_info, (size_t)N * C));
+        TC_TRY(tc_dev_alloc(h, &h->prims.overflow, (size_t)N));
+        TC_CUDA(cudaMemsetAsync(h->prims.cls_info, 0, (size_t)N * C * 4, st));
+        TC_CUDA(cudaMemsetAsync(h->prims.overflow, 0, (size_t)N, st));
+    }
+    if (launch != P::UNFUSED && after_project) TC_CUDA(cudaEventRecord(after_project, st));
+    switch (launch) {
+    case P::ENVS: {
+        TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, h->env_words);
+        ea.prim_chunks = h->env_chunks;
+        const int E = h->env_pack, grid = (N + E - 1) / E;
+        const size_t sm = h->envs_smem;
 #define TC_LAUNCH_ENVS(F)                                                                             \
     do {                                                                                              \
-        if (E == 4) tc_render_envs_kernel<256, F, 4><<<grid, 256, sme, st>>>(ea);                     \
-        else if (E == 2) tc_render_envs_kernel<256, F, 2><<<grid, 256, sme, st>>>(ea);                \
-        else tc_render_envs_kernel<256, F, 1><<<grid, 256, sme, st>>>(ea);                            \
+        if (E == 4) tc_render_envs_kernel<256, F, 4><<<grid, 256, sm, st>>>(ea);                      \
+        else tc_render_envs_kernel<256, F, 2><<<grid, 256, sm, st>>>(ea);                             \
     } while (0)
-            if (obs_format == TC_OBS_RGB) TC_LAUNCH_ENVS(TC_FMT_RGB);
-            else if (obs_format == TC_OBS_CLASSES_BITS) TC_LAUNCH_ENVS(TC_FMT_BITS);
-            else if (obs_format == TC_OBS_CLASSES_BF16) TC_LAUNCH_ENVS(TC_FMT_BF16);
-            else TC_LAUNCH_ENVS(TC_FMT_U8);
+        if (obs_format == TC_OBS_RGB) TC_LAUNCH_ENVS(TC_FMT_RGB);
+        else if (obs_format == TC_OBS_CLASSES_BITS) TC_LAUNCH_ENVS(TC_FMT_BITS);
+        else if (obs_format == TC_OBS_CLASSES_BF16) TC_LAUNCH_ENVS(TC_FMT_BF16);
+        else TC_LAUNCH_ENVS(TC_FMT_U8);
 #undef TC_LAUNCH_ENVS
-            h->launches++;
-            TC_CUDA(cudaGetLastError());
-            return TC_OK;
-        }
+        break;
+    }
+    case P::ENV: {
+        TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, h->env_words);
+        ea.timeline = timeline;
+        const size_t sm = h->env_smem;
         if (obs_format == TC_OBS_RGB) tc_render_env_kernel<256, TC_FMT_RGB><<<N, 256, sm, st>>>(ea);
         else if (obs_format == TC_OBS_CLASSES_BITS) tc_render_env_kernel<256, TC_FMT_BITS><<<N, 256, sm, st>>>(ea);
         else if (obs_format == TC_OBS_CLASSES_BF16) tc_render_env_kernel<256, TC_FMT_BF16><<<N, 256, sm, st>>>(ea);
-        else if (h->render_threads == 128) tc_render_env_kernel<128, TC_FMT_U8><<<N, 128, sm, st>>>(ea);
         else tc_render_env_kernel<256, TC_FMT_U8><<<N, 256, sm, st>>>(ea);
-        h->launches++;
-        TC_CUDA(cudaGetLastError());
-        return TC_OK;
+        break;
     }
-    if (obs && !h->fused_all && h->envb_on && h->envb_smem > 0 && h->prims_on && !seg_count_out && !seg_out && obs_format == TC_OBS_CLASSES_BITS &&
-        (h->H * h->W) % 128 == 0 && (size_t)h->plane_words_full * 4 <= 64 * 1024) {
+    case P::PRIMS: {
         // large frames, 1 bit per pixel: geometry + set-up once per env (primitives to L2), then a block per (env, class) draws and stores;
-        // envs with more segments than the primitive buffer holds are flagged and rendered by the banded kernel below
-        if (!h->prims.prims) {
-            TC_TRY(tc_dev_alloc(h, &h->prims.prims, (size_t)N * TC_PRIMS_CAP * TC_PRIMS_SEG_WORDS));
-            TC_TRY(tc_dev_alloc(h, &h->prims.cls_info, (size_t)N * C));
-            TC_TRY(tc_dev_alloc(h, &h->prims.overflow, (size_t)N));
-            TC_CUDA(cudaMemsetAsync(h->prims.cls_info, 0, (size_t)N * C * 4, st));
-            TC_CUDA(cudaMemsetAsync(h->prims.overflow, 0, (size_t)N, st));
-        }
-        TcRenderEnvArgs ea;
-        ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = N; ea.n_classes = C;
-        ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = 0;
-        ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = nullptr;
-        memcpy(ea.colors, h->colors, sizeof(ea.colors));
-        ea.timeline = nullptr;
-        ea.rows_per_band = h->envb_rows; ea.n_bands = h->envb_bands; ea.band_words = h->envb_words;
-        ea.region_bytes = (int)tc_envs_region_bytes((size_t)h->env_np, h->env_max_bytes, 0);
-        ea.prim_chunks = 1;
-        if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
+        // envs with more segments than the primitive buffer holds are flagged and rendered by the banded kernel
+        TcRenderEnvArgs ea = tc_render_env_args(h, mask, nullptr, 0);
         const size_t sm1 = tc_envs_smem_bytes(2, (size_t)h->env_np, h->env_max_bytes, 0, 1);
         tc_prims_kernel<256, 2><<<(N + 1) / 2, 256, sm1, st>>>(ea, h->prims);
         h->launches++;
@@ -615,67 +603,53 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
         TC_CUDA(cudaGetLastError());
         ea.mask = h->prims.overflow; ea.obs = obs;   // (the flag is only set for envs the caller's mask selected)
         tc_render_env_banded_kernel<TC_FMT_BITS><<<std::min(N, 2 * h->n_sms), 256, h->envb_smem, st>>>(ea);   // few blocks scan the (sparse) flags
-        h->launches++;
-        TC_CUDA(cudaGetLastError());
-        return TC_OK;
+        break;
     }
-    if (obs && !h->fused_all && h->envb_on && h->envb_smem > 0 && !seg_count_out && !seg_out && (obs_format == TC_OBS_RGB || obs_format == TC_OBS_CLASSES_BITS)) {
+    case P::BANDED: {
         // large frames whose stores are not the bound: a block per env, bands walked inside the block
-        TcRenderEnvArgs ea;
-        ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = N; ea.n_classes = C;
-        ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = 0;
-        ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = obs;
-        memcpy(ea.colors, h->colors, sizeof(ea.colors));
-        ea.timeline = nullptr;
-        ea.rows_per_band = h->envb_rows; ea.n_bands = h->envb_bands; ea.band_words = h->envb_words;
-        if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
+        const TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, 0);
         if (obs_format == TC_OBS_RGB) tc_render_env_banded_kernel<TC_FMT_RGB><<<N, 256, h->envb_smem, st>>>(ea);
         else tc_render_env_banded_kernel<TC_FMT_BITS><<<N, 256, h->envb_smem, st>>>(ea);
-        h->launches++;
-        TC_CUDA(cudaGetLastError());
-        return TC_OK;
+        break;
     }
-    if (obs && h->fused_ok && !seg_count_out && !seg_out && obs_format != TC_OBS_RGB) {
+    case P::CLASSES: {
         TcRenderArgs fa;
-        fa.cblob_desc = h->d_cblob_desc; fa.cblob = h->d_cblob; fa.max_cblob_bytes = h->fused_cblob; fa.n_envs = N; fa.n_classes = C;
-        fa.max_nodes = h->fused_nodes; fa.max_edges = h->fused_edges;
-        fa.H = h->H; fa.W = h->W; fa.plane_words = h->fused_words; fa.all_classes = 0; fa.all_desc = h->all_desc;
-        memcpy(fa.edge_off, h->edge_off_h, sizeof(fa.edge_off));
-        fa.rgb = 0;
-        memcpy(fa.colors, h->colors, sizeof(fa.colors)); fa.pose = h->d_pose; fa.cam = h->d_cam; fa.thickness = h->d_thick;
-        fa.mask = mask; fa.obs = obs;
-        fa.stagger_ns = mask ? 0 : h->stagger_ns; fa.n_sms = h->n_sms;
-        fa.timeline = mask ? nullptr : h->timeline;
-        if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
+        fa.cblob_desc = h->d_cblob_desc; fa.cblob = h->d_cblob; fa.max_cblob_bytes = h->max_cblob_bytes; fa.n_envs = N; fa.n_classes = C;
+        fa.max_nodes = h->max_nodes; fa.max_edges = h->max_edges;
+        fa.H = h->H; fa.W = h->W; fa.plane_words = h->plane_words_full;
+        fa.pose = h->d_pose; fa.cam = h->d_cam; fa.thickness = h->d_thick; fa.mask = mask; fa.obs = obs;
+        fa.timeline = timeline;
         const int grid = N * C;
         const size_t sm = h->render_smem;
         if (obs_format == TC_OBS_CLASSES_BITS) tc_render_classes_kernel<256, TC_FMT_BITS><<<grid, 256, sm, st>>>(fa);
         else if (obs_format == TC_OBS_CLASSES_BF16) tc_render_classes_kernel<256, TC_FMT_BF16><<<grid, 256, sm, st>>>(fa);
         else tc_render_classes_kernel<256, TC_FMT_U8><<<grid, 256, sm, st>>>(fa);
+        break;
+    }
+    case P::UNFUSED: {
+        TcProjArgs pa;
+        pa.classes = h->d_classes; pa.n_envs = N; pa.n_classes = C; pa.sum_edges = h->sum_edges; pa.max_nodes = h->max_nodes;
+        pa.H = h->H; pa.W = h->W; pa.edge_off = h->d_edge_off; pa.pose = h->d_pose; pa.cam = h->d_cam; pa.mask = mask;
+        pa.seg = seg_out ? seg_out : h->d_seg;
+        pa.seg_count = seg_count_out ? seg_count_out : h->d_seg_count;
+        tc_project_kernel<<<N * C, TC_PROJ_THREADS, h->proj_smem, st>>>(pa);
         h->launches++;
         TC_CUDA(cudaGetLastError());
-        return TC_OK;
+        if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
+        if (!obs) return TC_OK;
+        TcRasterArgs ra;
+        ra.n_envs = N; ra.n_classes = C; ra.sum_edges = h->sum_edges; ra.H = h->H; ra.W = h->W;
+        ra.edge_off = h->d_edge_off; ra.thickness = h->d_thick; ra.mask = mask; ra.seg = pa.seg; ra.seg_count = pa.seg_count; ra.obs = obs;
+        memcpy(ra.colors, h->colors, sizeof(ra.colors));
+        if (obs_format == TC_OBS_CLASSES) {
+            ra.rows_per_band = h->rows_per_band_cls; ra.n_bands = h->n_bands_cls; ra.plane_words = h->plane_words_cls;
+            tc_raster_classes_kernel<<<N * C * ra.n_bands, TC_RASTER_THREADS, (size_t)ra.plane_words * 4, st>>>(ra);
+        } else {
+            ra.rows_per_band = h->rows_per_band_rgb; ra.n_bands = h->n_bands_rgb; ra.plane_words = h->plane_words_rgb;
+            tc_raster_rgb_kernel<<<N * ra.n_bands, TC_RASTER_THREADS, tc_raster_rgb_smem_bytes(C, ra.plane_words), st>>>(ra);
+        }
+        break;
     }
-    TcProjArgs pa;
-    pa.classes = h->d_classes; pa.n_envs = N; pa.n_classes = C; pa.sum_edges = h->sum_edges; pa.max_nodes = h->max_nodes;
-    pa.H = h->H; pa.W = h->W; pa.edge_off = h->d_edge_off; pa.pose = h->d_pose; pa.cam = h->d_cam; pa.mask = mask;
-    pa.seg = seg_out ? seg_out : h->d_seg;
-    pa.seg_count = seg_count_out ? seg_count_out : h->d_seg_count;
-    tc_project_kernel<<<N * C, TC_PROJ_THREADS, h->proj_smem, st>>>(pa);
-    h->launches++;
-    TC_CUDA(cudaGetLastError());
-    if (after_project) TC_CUDA(cudaEventRecord(after_project, st));
-    if (!obs) return TC_OK;
-    TcRasterArgs ra;
-    ra.n_envs = N; ra.n_classes = C; ra.sum_edges = h->sum_edges; ra.H = h->H; ra.W = h->W;
-    ra.edge_off = h->d_edge_off; ra.thickness = h->d_thick; ra.mask = mask; ra.seg = pa.seg; ra.seg_count = pa.seg_count; ra.obs = obs;
-    memcpy(ra.colors, h->colors, sizeof(ra.colors));
-    if (obs_format == TC_OBS_CLASSES) {
-        ra.rows_per_band = h->rows_per_band_cls; ra.n_bands = h->n_bands_cls; ra.plane_words = h->plane_words_cls;
-        tc_raster_classes_kernel<<<N * C * ra.n_bands, TC_RASTER_THREADS, (size_t)ra.plane_words * 4, st>>>(ra);
-    } else {
-        ra.rows_per_band = h->rows_per_band_rgb; ra.n_bands = h->n_bands_rgb; ra.plane_words = h->plane_words_rgb;
-        tc_raster_rgb_kernel<<<N * ra.n_bands, TC_RASTER_THREADS, tc_raster_rgb_smem_bytes(C, ra.plane_words), st>>>(ra);
     }
     h->launches++;
     TC_CUDA(cudaGetLastError());

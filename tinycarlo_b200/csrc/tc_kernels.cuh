@@ -91,6 +91,48 @@ struct TcTrackArgs {
     TcOutputs out;
 };
 
+// The end of a tracking step, shared by both tracking kernels (one thread per env calls it): autoreset flags, state, the pose for
+// the camera pass and the outputs the caller asked for.
+__device__ __forceinline__ void tc_track_store(const TcTrackArgs &a, const TcTrackTables &t, int env, double *sf, int32_t *si, const TcCarState &s,
+                                               const TcInfo &info, bool truncated, bool auto_reset, const double *dist, const int *nearest) {
+    const int C = t.n_classes;
+    if (a.mode == 0 && a.done) a.done[env] = (info.terminated || truncated) ? 1 : 0;
+    if (a.mode == 0 && a.was_reset) a.was_reset[env] = auto_reset ? 1 : 0;
+    tc_store_state(sf, si, s);
+    // pose for the camera pass: front-axle update already evaluated cos/sin(rot); recomputing keeps the code simple
+    tc_camera_pose(a.cam + (size_t)env * TC_CAM_N + TC_CAM_E, s.x, s.y, cos(s.rot), sin(s.rot), a.pose + (size_t)env * 12);
+    const TcOutputs &o = a.out;
+    if (o.cte) o.cte[env] = (float)info.cte;
+    if (o.heading_error) o.heading_error[env] = (float)info.heading;
+    if (o.velocity) o.velocity[env] = (float)info.velocity;
+    if (o.position) { o.position[2 * env] = (float)s.x; o.position[2 * env + 1] = (float)s.y; }
+    if (o.orientation) o.orientation[env] = (float)s.rot;
+    if (o.laneline_distances) for (int c = 0; c < C; c++) o.laneline_distances[(size_t)env * C + c] = (float)dist[c];
+    if (o.nearest_edge) for (int c = 0; c < C; c++) o.nearest_edge[(size_t)env * C + c] = nearest[c];
+    // car.py:66 builds local_path coordinates only when the info is non-empty (len >= 2)
+    int plen = s.path_len >= 2 ? s.path_len : 0;
+    if (o.local_path)
+        for (int i = 0; i < 4; i++) {
+            bool ok = i < plen;
+            o.local_path[(size_t)env * 8 + 2 * i] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1]] : 0.0f;
+            o.local_path[(size_t)env * 8 + 2 * i + 1] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1] + 1] : 0.0f;
+        }
+    if (o.local_path_nodes)
+        for (int i = 0; i < 8; i++) o.local_path_nodes[(size_t)env * 8 + i] = (i >> 1) < s.path_len ? s.pn[i] : -1;
+    if (o.path_len) o.path_len[env] = s.path_len;
+    if (o.info_f64) {
+        double *r = o.info_f64 + (size_t)env * (4 + C);
+        r[TC_INFO_CTE] = info.cte; r[TC_INFO_HEADING] = info.heading; r[TC_INFO_VELOCITY] = info.velocity;
+        if (a.mode == 0) r[TC_INFO_REWARD] = info.reward;
+        for (int c = 0; c < C; c++) r[TC_INFO_DIST0 + c] = dist[c];
+    }
+    if (a.mode == 0) {
+        if (o.reward) o.reward[env] = (float)info.reward;
+        if (o.terminated) o.terminated[env] = info.terminated ? 1 : 0;
+        if (o.truncated) o.truncated[env] = truncated ? 1 : 0;
+    }
+}
+
 // G lanes per env (a power of two <= 32): the scalar part of a step is computed redundantly by the G lanes, the scans are spread
 // over them. 32 = a warp per env; 8 = four envs per warp, a quarter of the warps for the same envs - the better choice when a few
 // thousand envs cannot fill the SMs with one thread each (4096 envs: 1024 instead of 4096 warps, one wave instead of two).
@@ -116,7 +158,6 @@ __global__ void __launch_bounds__(TC_TRACK_THREADS, 3) tc_track_kernel(const TcT
     TcTrackTables t = tc_track_tables(smem_blob, a.layout);
     t.near_x0 = a.near_x0; t.near_y0 = a.near_y0; t.near_inv_cell = a.near_inv_cell; t.near_nx = a.near_nx; t.near_ny = a.near_ny;
     t.near_off = a.near_off; t.near_edge = a.near_edge;
-    const int C = t.n_classes;
     const double *cp = a.car + (size_t)env * TC_CP_N;
     double *sf = a.sf + (size_t)env * TC_SF_N;
     int32_t *si = a.si + (size_t)env * TC_SI_N;
@@ -157,41 +198,7 @@ __global__ void __launch_bounds__(TC_TRACK_THREADS, 3) tc_track_kernel(const TcT
     TcInfo info = tc_get_info(g, t, cp, s, a.wrapped != 0, dist, nearest);
     if (auto_reset) { info.reward = 0; info.terminated = false; }
     if (g.lane != 0) return;
-    if (a.mode == 0 && a.done) a.done[env] = (info.terminated || truncated) ? 1 : 0;
-    if (a.mode == 0 && a.was_reset) a.was_reset[env] = auto_reset ? 1 : 0;
-    tc_store_state(sf, si, s);
-    // pose for the camera pass: front-axle update already evaluated cos/sin(rot); recomputing keeps the code simple
-    tc_camera_pose(a.cam + (size_t)env * TC_CAM_N + TC_CAM_E, s.x, s.y, cos(s.rot), sin(s.rot), a.pose + (size_t)env * 12);
-    const TcOutputs &o = a.out;
-    if (o.cte) o.cte[env] = (float)info.cte;
-    if (o.heading_error) o.heading_error[env] = (float)info.heading;
-    if (o.velocity) o.velocity[env] = (float)info.velocity;
-    if (o.position) { o.position[2 * env] = (float)s.x; o.position[2 * env + 1] = (float)s.y; }
-    if (o.orientation) o.orientation[env] = (float)s.rot;
-    if (o.laneline_distances) for (int c = 0; c < C; c++) o.laneline_distances[(size_t)env * C + c] = (float)dist[c];
-    if (o.nearest_edge) for (int c = 0; c < C; c++) o.nearest_edge[(size_t)env * C + c] = nearest[c];
-    // car.py:66 builds local_path coordinates only when the info is non-empty (len >= 2)
-    int plen = s.path_len >= 2 ? s.path_len : 0;
-    if (o.local_path)
-        for (int i = 0; i < 4; i++) {
-            bool ok = i < plen;
-            o.local_path[(size_t)env * 8 + 2 * i] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1]] : 0.0f;
-            o.local_path[(size_t)env * 8 + 2 * i + 1] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1] + 1] : 0.0f;
-        }
-    if (o.local_path_nodes)
-        for (int i = 0; i < 8; i++) o.local_path_nodes[(size_t)env * 8 + i] = (i >> 1) < s.path_len ? s.pn[i] : -1;
-    if (o.path_len) o.path_len[env] = s.path_len;
-    if (o.info_f64) {
-        double *r = o.info_f64 + (size_t)env * (4 + C);
-        r[TC_INFO_CTE] = info.cte; r[TC_INFO_HEADING] = info.heading; r[TC_INFO_VELOCITY] = info.velocity;
-        if (a.mode == 0) r[TC_INFO_REWARD] = info.reward;
-        for (int c = 0; c < C; c++) r[TC_INFO_DIST0 + c] = dist[c];
-    }
-    if (a.mode == 0) {
-        if (o.reward) o.reward[env] = (float)info.reward;
-        if (o.terminated) o.terminated[env] = info.terminated ? 1 : 0;
-        if (o.truncated) o.truncated[env] = truncated ? 1 : 0;
-    }
+    tc_track_store(a, t, env, sf, si, s, info, truncated, auto_reset, dist, nearest);
 }
 
 // The same step with ONE THREAD PER ENV. The warp-per-env kernel above computes the scalar part of a step (bicycle model, path
@@ -285,39 +292,7 @@ __global__ void __launch_bounds__(TC_TRACK1_THREADS) tc_track_thread_kernel(cons
     int nearest[TC_MAX_CLASSES];
     TcInfo info = tc_get_info(g1, t, cp, s, a.wrapped != 0, dist, nearest, scan ? pre : nullptr);
     if (auto_reset) { info.reward = 0; info.terminated = false; }
-    if (a.mode == 0 && a.done) a.done[env] = (info.terminated || truncated) ? 1 : 0;
-    if (a.mode == 0 && a.was_reset) a.was_reset[env] = auto_reset ? 1 : 0;
-    tc_store_state(sf, si, s);
-    tc_camera_pose(a.cam + (size_t)env * TC_CAM_N + TC_CAM_E, s.x, s.y, cos(s.rot), sin(s.rot), a.pose + (size_t)env * 12);
-    const TcOutputs &o = a.out;
-    if (o.cte) o.cte[env] = (float)info.cte;
-    if (o.heading_error) o.heading_error[env] = (float)info.heading;
-    if (o.velocity) o.velocity[env] = (float)info.velocity;
-    if (o.position) { o.position[2 * env] = (float)s.x; o.position[2 * env + 1] = (float)s.y; }
-    if (o.orientation) o.orientation[env] = (float)s.rot;
-    if (o.laneline_distances) for (int c = 0; c < C; c++) o.laneline_distances[(size_t)env * C + c] = (float)dist[c];
-    if (o.nearest_edge) for (int c = 0; c < C; c++) o.nearest_edge[(size_t)env * C + c] = nearest[c];
-    int plen = s.path_len >= 2 ? s.path_len : 0;   // car.py:66: local_path coordinates only when the info is non-empty
-    if (o.local_path)
-        for (int i = 0; i < 4; i++) {
-            bool ok = i < plen;
-            o.local_path[(size_t)env * 8 + 2 * i] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1]] : 0.0f;
-            o.local_path[(size_t)env * 8 + 2 * i + 1] = ok ? (float)t.lp_nodes[2 * s.pn[2 * i + 1] + 1] : 0.0f;
-        }
-    if (o.local_path_nodes)
-        for (int i = 0; i < 8; i++) o.local_path_nodes[(size_t)env * 8 + i] = (i >> 1) < s.path_len ? s.pn[i] : -1;
-    if (o.path_len) o.path_len[env] = s.path_len;
-    if (o.info_f64) {
-        double *r = o.info_f64 + (size_t)env * (4 + C);
-        r[TC_INFO_CTE] = info.cte; r[TC_INFO_HEADING] = info.heading; r[TC_INFO_VELOCITY] = info.velocity;
-        if (a.mode == 0) r[TC_INFO_REWARD] = info.reward;
-        for (int c = 0; c < C; c++) r[TC_INFO_DIST0 + c] = dist[c];
-    }
-    if (a.mode == 0) {
-        if (o.reward) o.reward[env] = (float)info.reward;
-        if (o.terminated) o.terminated[env] = info.terminated ? 1 : 0;
-        if (o.truncated) o.truncated[env] = truncated ? 1 : 0;
-    }
+    tc_track_store(a, t, env, sf, si, s, info, truncated, auto_reset, dist, nearest);
 }
 
 // ------------------------------------------------------------------------------------------------ camera pass
@@ -784,16 +759,11 @@ struct TcRenderArgs {
     const int32_t *thickness;  // [N]
     const uint8_t *mask;       // optional
     uint8_t *obs;              // [N,C,H,W]
-    int rgb;                   // informational; the kernel is instantiated per format (needs all_classes): compose [H,W,3] layer colours, later classes on top (renderer.py:41-43)
-    uint8_t colors[TC_MAX_CLASSES * 3];
-    int all_classes;           // 1: a block renders all C classes of an env (stacked C*H-row plane), 0: one class
-    TcClassBlob all_desc;      // the union graph of all classes (all_classes == 1)
-    int32_t edge_off[TC_MAX_CLASSES + 1];
-    int stagger_ns, n_sms;     // first-wave phase stagger (see the kernel)
     long long *timeline;       // optional debug [N*C][10]: smid, clock at start / tables landed / geometry done / raster done / end
 };
 
-// shared memory: [union{ camera-pass scratch + the class's tables (TMA) | bit plane }][segment list]
+// shared memory: [union{ camera-pass scratch + the class's tables (TMA) | bit plane }][segment list][primitive slots][one byte per
+// edge, unused: it keeps the block's footprint, which decides the blocks per SM and (tc_create) which frames take this kernel]
 __host__ __device__ inline size_t tc_render_scratch_bytes(int max_nodes) { return (tc_proj_smem_bytes(max_nodes) + 127) & ~(size_t)127; }
 __host__ __device__ inline size_t tc_render_union_bytes(int max_nodes, int max_cblob_bytes, int plane_words) {
     size_t a = tc_render_scratch_bytes(max_nodes) + (size_t)max_cblob_bytes, b = (size_t)plane_words * 4;
@@ -805,35 +775,16 @@ __host__ __device__ inline size_t tc_render_smem_bytes(int max_nodes, int max_ed
            (size_t)TC_SETUP_CHUNK * TC_MAX_PRIMS_PER_SEG * sizeof(TcPrim) + (size_t)((max_edges + 15) & ~15);
 }
 
-// NT threads per block: 256 for large frames (4 blocks/SM, stores dominate), 128 for small ones (8 blocks/SM: the block's
-// work is then the latency-bound camera pass, and twice as many independent blocks hide it better)
+// NT = 256 threads per block, 4 blocks/SM: the stores dominate
 template <int NT, int FMT>
 __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const TcRenderArgs a) {
-    constexpr bool RGB = FMT == TC_FMT_RGB;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int seg_cnt;
     __shared__ __align__(8) uint64_t bar;
     __shared__ double s_pose[12], s_cam[TC_CAM_N];
-    __shared__ uint32_t s_color24[TC_MAX_CLASSES];
-    const int env = a.all_classes ? blockIdx.x : blockIdx.x / a.n_classes, c = a.all_classes ? 0 : blockIdx.x % a.n_classes;
+    const int env = blockIdx.x / a.n_classes, c = blockIdx.x % a.n_classes;
     if (a.mask && !a.mask[env]) return;
     const int tid = threadIdx.x;
-    // Every block does a latency-bound geometry phase and then a bandwidth-bound store phase. Blocks that share an SM
-    // start together and, sharing the SM's store bandwidth equally, finish together, so their successors start together
-    // again: the SM's HBM share idles during every geometry phase (measured: ~10% of the kernel). Delaying the k-th
-    // resident block of the first wave by k * stagger_ns puts the co-resident blocks out of phase once; the staggered
-    // state then sustains itself (a block in its geometry phase lends its bandwidth share to the others).
-    if (a.stagger_ns > 0 && (int)blockIdx.x < 4 * a.n_sms) {
-        const unsigned slot = blockIdx.x / a.n_sms;
-        if (slot) {
-            unsigned long long t0, t1;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-            do {
-                __nanosleep(500);
-                asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-            } while (t1 - t0 < (unsigned long long)slot * a.stagger_ns);
-        }
-    }
 // per-block phase clocks for tools/timeline.py: compiled in only with -DTC_TIMELINE (the seven 64-bit counters cost
 // registers and spills in the production build)
 #ifdef TC_TIMELINE
@@ -843,7 +794,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
 #define TC_TL(stmt) do { } while (0)
 #endif
     TC_TL(tl0 = clock64());
-    const TcClassBlob cb = a.all_classes ? a.all_desc : a.cblob_desc[c];
+    const TcClassBlob cb = a.cblob_desc[c];
     unsigned char *tab_smem = smem_raw + tc_render_scratch_bytes(a.max_nodes);
     if (tid == 0) {
         seg_cnt = 0;
@@ -854,7 +805,6 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
     }
     const int n = cb.n_nodes, m = cb.n_edges;
     int4 *segs = (int4 *)(smem_raw + tc_render_union_bytes(a.max_nodes, a.max_cblob_bytes, a.plane_words));
-    uint8_t *seg_cls = (uint8_t *)segs + tc_render_segs_bytes(a.max_edges) + (size_t)TC_SETUP_CHUNK * TC_MAX_PRIMS_PER_SEG * sizeof(TcPrim);
     uint32_t *plane = (uint32_t *)smem_raw;
     {
         const size_t np = (size_t)((a.max_nodes + 15) & ~15);
@@ -865,10 +815,6 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
         sc.vis = rB + np; sc.front = fA; sc.inr = rA;
         // pose and intrinsics go through shared memory: 17 doubles held in registers by every thread across the whole
         // camera pass would push the kernel over 64 registers, and spills are local-memory traffic behind the stores
-        if (RGB && tid >= 64 && tid < 64 + TC_MAX_CLASSES) {
-            const int cc = tid - 64;
-            s_color24[cc] = tc_color24_of(a.colors, cc);
-        }
         if (tid < 12) s_pose[tid] = a.pose[(size_t)env * 12 + tid];
         else if (tid < 12 + (TC_CAM_MAX_RANGE - TC_CAM_FX + 1)) s_cam[TC_CAM_FX + tid - 12] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + tid - 12];
         __syncthreads();      // barrier init, pose and intrinsics visible to all threads
@@ -908,20 +854,12 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
             if (sc.vis[n0] || sc.vis[n1]) {
                 int slot = atomicAdd(&seg_cnt, 1);
                 segs[slot] = make_int4(sc.ix[n0], sc.iy[n0], sc.ix[n1], sc.iy[n1]);
-                if (a.all_classes) {   // class of the edge = plane it is drawn into
-                    int cls = 0;
-                    while (cls + 1 < a.n_classes && e >= a.edge_off[cls + 1]) cls++;
-                    seg_cls[slot] = (uint8_t)cls;
-                }
             }
         }
         __syncthreads(); // scratch and tables are dead from here on; the plane takes their place
     }
     const int cnt = seg_cnt;
     TC_TL(tl2 = clock64());
-    const int n_planes = a.all_classes ? a.n_classes : 1;
-    uint8_t *out = RGB ? a.obs + (size_t)env * a.H * a.W * 3 : a.obs + ((size_t)env * a.n_classes + c) * a.H * a.W;
-    const size_t nbytes = (size_t)n_planes * a.H * a.W;
     if (cnt > 0) {
         for (int i = tid; i < a.plane_words; i += NT) plane[i] = 0;
         __syncthreads();
@@ -947,8 +885,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
             // pixels: the primitives go round-robin to the warps, the pixels / rows of a primitive to the lanes
             for (int p = warp; p < nseg * TC_MAX_PRIMS_PER_SEG; p += (NT / 32))
                 if (prims[p].kind != TC_PRIM_NONE) {
-                    const int cls = a.all_classes ? seg_cls[base + p / TC_MAX_PRIMS_PER_SEG] : 0;
-                    TcPlane pl = {plane, a.H, a.W, 0, a.H, -cls * a.H};
+                    TcPlane pl = {plane, a.H, a.W, 0, a.H, 0};
                     tc_prim_draw(g, pl, prims[p]);
                 }
             __syncthreads();
@@ -956,14 +893,15 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
         }
     }
     TC_TL(tl3 = clock64());
-    if (FMT == TC_FMT_RGB) tc_store_rgb<NT>(out, (uint32_t)(a.H * a.W), plane, (uint32_t)(a.H * a.W), a.n_classes, s_color24, cnt > 0);
-    else if (FMT == TC_FMT_BITS) {
-        // planes are whole words here (the host only selects this format when H*W % 32 == 0 or one class per block)
-        const int words = (int)(((size_t)a.H * a.W + 31) / 32) * n_planes;
-        tc_store_bits<NT>((uint32_t *)a.obs + ((size_t)env * a.n_classes + c) * (((size_t)a.H * a.W + 31) / 32), words, plane, cnt > 0);
+    // block (env, class) writes plane blockIdx.x = env * C + class; addressed from blockIdx.x here rather than kept live across
+    // the raster phase, which at exactly 64 registers brings spills back
+    const size_t hw = (size_t)a.H * a.W;
+    if (FMT == TC_FMT_BITS) {
+        const int words = (int)((hw + 31) / 32);
+        tc_store_bits<NT>((uint32_t *)a.obs + (size_t)blockIdx.x * words, words, plane, cnt > 0);
     } else if (FMT == TC_FMT_BF16)
-        tc_store_bf16<NT>((uint16_t *)a.obs + ((size_t)env * a.n_classes + c) * a.H * a.W, (uint32_t)(n_planes * a.H * a.W), plane, cnt > 0);
-    else tc_store_plane<NT>(out, nbytes, plane, cnt > 0);
+        tc_store_bf16<NT>((uint16_t *)a.obs + blockIdx.x * hw, (uint32_t)hw, plane, cnt > 0);
+    else tc_store_plane<NT>(a.obs + blockIdx.x * hw, hw, plane, cnt > 0);
 #ifdef TC_TIMELINE
     if (a.timeline && tid == 0) {
         unsigned smid;
@@ -1575,7 +1513,7 @@ struct TcDrawArgs {
 template <int NT, int FMT>
 __global__ void __launch_bounds__(NT) tc_draw_class_kernel(const TcDrawArgs a) {
     extern __shared__ __align__(128) uint32_t plane[];
-    const int env = blockIdx.x / a.n_classes, c = blockIdx.x - env * a.n_classes;
+    const int env = blockIdx.x / a.n_classes, c = blockIdx.x % a.n_classes;
     const int info = a.in.cls_info[blockIdx.x];   // issued before the mask test: one round trip for both
     if (a.mask && !a.mask[env]) return;
     if (info < 0) return;                  // the env overflowed the primitive buffer: the fallback kernel renders it

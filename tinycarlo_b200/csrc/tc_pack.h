@@ -17,8 +17,6 @@ struct TcPacked {
     std::vector<TcClassBlob> cblob_desc;  // per class
     std::vector<unsigned char> cblob;     // all class blobs, each 16-byte aligned
     int max_cblob_bytes = 0;
-    TcClassBlob all_desc{};               // the disjoint union of all classes as ONE graph (global node ids); its blob
-                                          // is appended to cblob (small frames: one block renders all classes of an env)
 };
 
 static inline int32_t tc_align16(int32_t x) { return (x + 15) & ~15; }
@@ -117,38 +115,6 @@ static inline std::string tc_pack_map(const TcMapDesc *map, TcPacked &pk) {
         pk.adj.insert(pk.adj.end(), oe.begin(), oe.end());
         pk.adj.insert(pk.adj.end(), io.begin(), io.end());
         pk.adj.insert(pk.adj.end(), ie.begin(), ie.end());
-    }
-    {
-        // union graph: nodes of all classes concatenated, edges / adjacency with global node ids, edge order = class order
-        const int n = sumN, m = sumE;
-        std::vector<int32_t> ed(2 * (size_t)std::max(m, 1)), oo(n + 1, 0), io(n + 1, 0), oe(std::max(m, 1)), ie(std::max(m, 1));
-        for (int c = 0; c < C; c++)
-            for (int e = map->ll_edge_off[c]; e < map->ll_edge_off[c + 1]; e++) {
-                ed[2 * e] = map->ll_edges[2 * e] + map->ll_node_off[c];
-                ed[2 * e + 1] = map->ll_edges[2 * e + 1] + map->ll_node_off[c];
-            }
-        for (int e = 0; e < m; e++) { oo[ed[2 * e] + 1]++; io[ed[2 * e + 1] + 1]++; }
-        for (int i = 0; i < n; i++) { oo[i + 1] += oo[i]; io[i + 1] += io[i]; }
-        std::vector<int32_t> oc(oo.begin(), oo.end() - 1), ic(io.begin(), io.end() - 1);
-        for (int e = 0; e < m; e++) { oe[oc[ed[2 * e]]++] = e; ie[ic[ed[2 * e + 1]]++] = e; }
-        TcClassBlob d;
-        d.n_nodes = n; d.n_edges = m;
-        int32_t o = 0;
-        auto sec = [&](int32_t bytes) { int32_t at = o; o = tc_align16(o + bytes); return at; };
-        sec(n * 16);
-        d.off_edges = sec(m * 8); d.off_out_off = sec((n + 1) * 4); d.off_out_edge = sec(m * 4);
-        d.off_in_off = sec((n + 1) * 4); d.off_in_edge = sec(m * 4);
-        d.bytes = o;
-        d.offset = (int32_t)pk.cblob.size();
-        pk.cblob.resize(pk.cblob.size() + (size_t)o, 0);
-        unsigned char *cb = pk.cblob.data() + d.offset;
-        memcpy(cb, map->ll_nodes, (size_t)n * 16);
-        memcpy(cb + d.off_edges, ed.data(), (size_t)m * 8);
-        memcpy(cb + d.off_out_off, oo.data(), (size_t)(n + 1) * 4);
-        memcpy(cb + d.off_out_edge, oe.data(), (size_t)m * 4);
-        memcpy(cb + d.off_in_off, io.data(), (size_t)(n + 1) * 4);
-        memcpy(cb + d.off_in_edge, ie.data(), (size_t)m * 4);
-        pk.all_desc = d;
     }
     return "";
 }

@@ -1,5 +1,4 @@
-"""Knuffingen 480x640 as 1 bit per pixel (obs_format="classes_bits"), 16384 envs: step and per-kernel times. TC_PRIMS_PATH=0 selects
-the banded block-per-env kernel instead of the two-kernel path."""
+"""Knuffingen 480x640 as 1 bit per pixel (obs_format="classes_bits"), 16384 envs: step and per-kernel times."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -34,5 +33,5 @@ e1.record(); torch.cuda.synchronize()
 k, ks = env.profile_end()
 ms = e0.elapsed_time(e1) / steps
 nb = env.obs[0].numel() * env.obs.element_size()
-print(f"prims_path={os.environ.get('TC_PRIMS_PATH', '1')} N={n} step {ms:.3f} ms track {k['track'] / ks:.3f} render {(k['project'] + k['raster']) / ks:.3f}  -> {n / ms / 1e3:.2f} M env-steps/s  "
+print(f"N={n} step {ms:.3f} ms track {k['track'] / ks:.3f} render {(k['project'] + k['raster']) / ks:.3f}  -> {n / ms / 1e3:.2f} M env-steps/s  "
       f"{n * nb / ms / 1e6:.0f} GB/s  set pixels per env {int((env.obs != 0).sum().item()) / n:.0f} words")

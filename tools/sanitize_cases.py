@@ -1,7 +1,8 @@
-"""A small pass through every kernel of the library for compute-sanitizer (memcheck / racecheck / initcheck / synccheck): few envs,
-few steps, each render path once - the packed and one-env block-per-env kernels, the per-class headline kernel, the banded
-kernel (RGB), the two-kernel path of bit-packed frames with its overflow fallback, the unfused debug path, both tracking kernels
-(warp- and thread-per-env) incl. u-turn scans and in-kernel autoreset, the noise kernel - every frame compared with the CPU oracle.
+"""A small pass through every kernel of the library for compute-sanitizer (memcheck / racecheck / initcheck / synccheck): few envs
+(except where the thread-per-env tracking kernel needs many), few steps, each render path once - the packed and one-env
+block-per-env kernels, the per-class headline kernel, the banded kernel (RGB), the two-kernel path of bit-packed frames with its
+overflow fallback, the unfused debug path, both tracking kernels (warp- and thread-per-env, chosen by the env count) incl. u-turn
+scans and in-kernel autoreset, the noise kernel - every frame compared with the CPU oracle.
 
   compute-sanitizer --tool racecheck python tools/sanitize_cases.py
 """
@@ -17,6 +18,10 @@ from pair_util import make_config, oracle_env  # noqa: E402
 from tinycarlo_b200 import TinyCarloVecEnv  # noqa: E402
 
 STEPS = int(os.environ.get("TC_SAN_STEPS", 3))
+# tc_create's choice of tracking kernel: one thread per env once n / 4 > 3 * 8 * SMs, below that a warp per env (8 lanes per env
+# above 3 * 8 * SMs / 2 envs)
+SMS = torch.cuda.get_device_properties(0).multi_processor_count
+N_THREAD_TRACK = 4 * (3 * 8 * SMS + 1)
 
 
 def run(name, cfg, n, env_kw=None, setenv=None, check="u8"):
@@ -70,11 +75,10 @@ run("banded kernel rgb 480x640", simple("rgb", [480, 640]), 3)
 run("bits 480x640: prims + draw kernels", knuff("classes", [480, 640]), 4, env_kw={"obs_format": "classes_bits"}, check="bits")
 run("bits 480x640 long range: overflow fallback", simple("classes", [480, 640], max_range=3.0, orientation=[30, 0, 0]), 3,
     env_kw={"obs_format": "classes_bits"}, check="bits")
-run("bits 480x640 banded only", knuff("classes", [480, 640]), 3, env_kw={"obs_format": "classes_bits"}, setenv={"TC_PRIMS_PATH": "0"}, check="bits")
 run("unfused project + raster (debug segments)", knuff("classes", [96, 128]), 4, env_kw={"debug_segments": True})
-run("thread-per-env tracking", knuff("classes", [32, 48]), 70, setenv={"TC_TRACK_MODE": "thread"})
-run("warp-per-env tracking", knuff("classes", [32, 48]), 20, setenv={"TC_TRACK_MODE": "warp"})
-run("autoreset next_step (thread tracking)", knuff("classes", [32, 48]), 40, env_kw={"autoreset": "next_step"}, setenv={"TC_TRACK_MODE": "thread"})
+run("thread-per-env tracking", knuff("classes", [32, 48]), N_THREAD_TRACK)
+run("warp-per-env tracking", knuff("classes", [32, 48]), 20)
+run("autoreset next_step (thread tracking)", knuff("classes", [32, 48]), N_THREAD_TRACK, env_kw={"autoreset": "next_step"})
 # the noise kernel (NoiseObservationWrapper on the device)
 from tinycarlo_b200.wrapper import NoiseObservationWrapper  # noqa: E402
 e = TinyCarloVecEnv(knuff("classes", [64, 96]), 6, device="cuda:0")
