@@ -185,6 +185,35 @@ TC_API int tc_step_host_obs(TcHandle *h, const float *host_car_control, const in
 TC_API int tc_noise_blobs(TcHandle *h, uint8_t *dev_obs, uint64_t seed, uint32_t step, int32_t n_blobs, int32_t max_radius,
                           int32_t env_index_offset, const uint8_t *dev_mask, void *stream);
 
+/* Ego-centric bird's-eye view (BEV): top-down lane masks around every car, P = C + route planes. For env i with state
+ * x = sf[TC_SF_X], y = sf[TC_SF_Y], θ = sf[TC_SF_ROT] (the rear axle, in map metres; map coordinates are image-like, y down):
+ *
+ *   c = cos θ, s = sin θ, k = pixel_per_meter, (col0, row0) = car_pixel
+ *   for a map point (px, py):  dx = px - x;  dy = py - y
+ *       u = col0 + k * (dy*c - dx*s)        # car's right  -> +u (image right)
+ *       v = row0 - k * (dx*c + dy*s)        # car's heading -> -v (image up)
+ *
+ * evaluated in float64, in exactly this order, with no FMA, then truncated with tc_np_int32 (numpy's np.int32). Plane p < C
+ * is laneline class p: for every edge of that class in JSON order, cv2.polylines(plane, [[u0,v0],[u1,v1]], False, 255,
+ * line_thickness) on a zero plane. With route on, plane C holds the car's tracked local path instead: the path_len lanepath
+ * edges (si[2+2j], si[3+2j]) with lp_nodes coordinates, drawn the same way (what the overview draws in blue). The mapping is
+ * a rotation, not a mirror: the BEV is the reference overview turned so that the car points up. */
+typedef struct {
+    int32_t height, width;       /* BEV resolution H, W */
+    double pixel_per_meter;      /* k */
+    double car_col, car_row;     /* (col0, row0): where the rear axle lands in the BEV */
+    int32_t line_thickness;      /* 1..8 */
+    int32_t route;               /* 1: plane C holds the tracked local path */
+    int32_t format;              /* TC_OBS_CLASSES: u8 [N,P,H,W] 0/255; TC_OBS_CLASSES_BITS: u32 [N,P,H*W/32] (needs H*W % 32 == 0) */
+} TcBevDesc;
+/* Registers the BEV description and a caller-owned device buffer of N frames in desc->format, which must stay alive (like
+ * tc_set_autoreset's buffer). From then on tc_step / tc_step_f64 re-render the BEV after the tracking kernel (one launch; it
+ * reads the post-step state, so next-step autoresets need nothing extra) and tc_reset renders it for the masked envs, whether
+ * or not they render the camera. dev_bev NULL switches the BEV off. */
+TC_API int tc_set_bev(TcHandle *h, const TcBevDesc *desc, uint8_t *dev_bev);
+/* Re-renders the BEV of the envs with dev_mask[i] != 0 (NULL = all) at the current state (after tc_set_state). */
+TC_API int tc_render_bev(TcHandle *h, const uint8_t *dev_mask, void *stream);
+
 /* Number of kernel launches issued through this handle since creation (bench.py reports it). */
 TC_API int64_t tc_launch_count(const TcHandle *h);
 

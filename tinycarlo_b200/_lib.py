@@ -31,6 +31,11 @@ class TcSimDesc(C.Structure):
     _fields_ = [("height", C.c_int32), ("width", C.c_int32), ("obs_format", C.c_int32)]
 
 
+class TcBevDesc(C.Structure):
+    _fields_ = [("height", C.c_int32), ("width", C.c_int32), ("pixel_per_meter", C.c_double), ("car_col", C.c_double),
+                ("car_row", C.c_double), ("line_thickness", C.c_int32), ("route", C.c_int32), ("format", C.c_int32)]
+
+
 OUTPUT_FIELDS = ["obs", "cte", "heading_error", "velocity", "reward", "position", "orientation", "laneline_distances",
                  "nearest_edge", "local_path", "local_path_nodes", "path_len", "terminated", "truncated", "info_f64", "seg_count",
                  "seg_i32"]
@@ -121,6 +126,8 @@ def lib():
     L.tc_set_wrapped.argtypes = [vp, i32]
     L.tc_set_autoreset.argtypes = [vp, vp]
     L.tc_set_reset_mask.argtypes = [vp, vp]
+    L.tc_set_bev.argtypes = [vp, C.POINTER(TcBevDesc), vp]
+    L.tc_render_bev.argtypes = [vp, vp, vp]
     L.tc_set_spawn_rng.argtypes = [vp, vp, vp, i32, vp]
     L.tc_debug_set_timeline.argtypes = [vp, vp]
     L.tc_debug_cull_info.argtypes = [vp, C.POINTER(C.c_double)]
@@ -140,7 +147,7 @@ def lib():
     L.tc_profile_begin.argtypes = [vp, i32]
     L.tc_profile_end.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32)]
     L.tc_debug_layer_query.argtypes = [vp, i32, C.c_double, C.c_double, C.c_double, i32, i32, vp, vp, vp]
-    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_create", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
+    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_create", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
                  "tc_render", "tc_get_state", "tc_set_state", "tc_step_host", "tc_debug_layer_query", "tc_profile_begin", "tc_profile_end"):
         getattr(L, name).restype = C.c_int
     if L.tc_abi_version() != 1:

@@ -2,6 +2,7 @@
 camera.py:16-21, map.py:13-17). A config is a path to a .yaml file, a directory holding config.yaml, or a dict with
 the mandatory sections sim / car / camera / map (a missing section raises KeyError, as in the reference)."""
 import math
+import numbers
 import os
 from typing import Any, Dict, Optional, Tuple, Union
 
@@ -68,6 +69,57 @@ def camera_params(camera_config: Dict[str, Any]) -> Dict[str, Any]:
     if not cam["max_range"]:
         raise ValueError("camera.max_range must be a positive number (the reference raises on the first frame when it is None)")
     return cam
+
+
+BEV_MAX_CLASSES = 16              # TC_MAX_CLASSES: planes of one BEV
+BEV_SMEM_MAX = 200 * 1024         # TC_BEV_SMEM_MAX: shared memory of the BEV kernel's stacked bit plane
+BEV_FORMATS = ("classes", "classes_bits")
+
+
+def bev_params(config: Dict[str, Any], n_classes: int) -> Optional[Dict[str, Any]]:
+    """The optional `bev` section (an extension: an ego-centric bird's-eye view of the lanes, include/tinycarlo_b200.h
+    tc_set_bev) with its defaults, or None when the config has none. Raises ValueError for a bad section."""
+    bev = config.get("bev")
+    if bev is None:
+        return None
+    if not isinstance(bev, dict):
+        raise ValueError("bev must be a mapping")
+
+    def integer(v):
+        return isinstance(v, numbers.Integral) and not isinstance(v, bool)
+
+    def finite(v):
+        return isinstance(v, numbers.Real) and not isinstance(v, bool) and math.isfinite(v)
+    res = bev.get("resolution", [128, 128])
+    if not (isinstance(res, (list, tuple)) and len(res) == 2 and all(integer(v) for v in res)
+            and all(0 < v <= 4096 for v in res)):
+        raise ValueError(f"bev.resolution must be [H, W] with integers in 1..4096, got {res!r}")
+    H, W = int(res[0]), int(res[1])
+    ppm = bev.get("pixel_per_meter", 128)
+    if not (finite(ppm) and ppm > 0):
+        raise ValueError(f"bev.pixel_per_meter must be a finite number > 0, got {ppm!r}")
+    car = bev.get("car_pixel", [W / 2, 7 * H / 8])
+    if not (isinstance(car, (list, tuple)) and len(car) == 2 and all(finite(v) for v in car)):
+        raise ValueError(f"bev.car_pixel must be [col, row] with finite numbers, got {car!r}")
+    t = bev.get("line_thickness", 1)
+    if not (integer(t) and 1 <= t <= 8):
+        raise ValueError(f"bev.line_thickness must be an integer in 1..8, got {t!r}")
+    route = bev.get("route", False)
+    if not isinstance(route, bool):
+        raise ValueError(f"bev.route must be true or false, got {route!r}")
+    fmt = bev.get("format", "classes")
+    if fmt not in BEV_FORMATS:
+        raise ValueError(f"bev.format must be one of {BEV_FORMATS}, got {fmt!r}")
+    if fmt == "classes_bits" and (H * W) % 32 != 0:
+        raise ValueError("bev.format classes_bits needs H*W to be a multiple of 32")
+    planes = n_classes + int(route)
+    if planes > BEV_MAX_CLASSES:
+        raise ValueError(f"bev: {planes} planes (classes + route) exceed {BEV_MAX_CLASSES}")
+    words = (planes * H * W + 31) // 32 + 1
+    if (words * 4 + 15) // 16 * 16 > BEV_SMEM_MAX:
+        raise ValueError(f"bev: {planes} planes of {H}x{W} do not fit the kernel's shared memory ({BEV_SMEM_MAX} bytes of bit planes)")
+    return {"resolution": [H, W], "pixel_per_meter": float(ppm), "car_pixel": [float(car[0]), float(car[1])], "line_thickness": int(t),
+            "route": route, "format": fmt, "planes": planes}
 
 
 # ------------------------------------------------------------------------------------------------ shipped configurations

@@ -117,6 +117,9 @@ struct TcHandle {
     const int32_t *spawn_points = nullptr;
     int n_spawn_points = 0;
     int32_t *last_spawn = nullptr;
+    TcBevDesc bev{};            // bird's-eye view (tc_set_bev): off while bev_out is NULL
+    uint8_t *bev_out = nullptr; // caller-owned
+    int bev_planes = 0, bev_plane_words = 0;
     // optional per-kernel CUDA-event timing (tc_profile_begin/end)
     bool profiling = false;
     int prof_cap = 0, prof_used = 0; // step slots
@@ -681,6 +684,51 @@ static int tc_launch_track(TcHandle *h, int mode, const float *cc, const int32_t
     return TC_OK;
 }
 
+static int tc_launch_bev(TcHandle *h, const uint8_t *mask, cudaStream_t st) {
+    TcBevArgs a;
+    a.blob = h->d_blob; a.layout = h->layout; a.sf = h->d_sf; a.si = h->d_si;
+    a.g.k = h->bev.pixel_per_meter; a.g.col0 = h->bev.car_col; a.g.row0 = h->bev.car_row;
+    a.g.H = h->bev.height; a.g.W = h->bev.width; a.g.thickness = h->bev.line_thickness; a.g.route = h->bev.route;
+    a.n_envs = h->n_envs; a.planes = h->bev_planes; a.plane_words = h->bev_plane_words; a.format = h->bev.format;
+    a.mask = mask; a.out = h->bev_out;
+    tc_bev_kernel<<<h->n_envs, TC_BEV_THREADS, tc_bev_smem_bytes(h->bev_plane_words), st>>>(a);
+    h->launches++;
+    TC_CUDA(cudaGetLastError());
+    return TC_OK;
+}
+
+int tc_set_bev(TcHandle *h, const TcBevDesc *desc, uint8_t *dev_bev) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_set_bev: null handle");
+    if (!dev_bev) {
+        h->bev_out = nullptr;
+        return TC_OK;
+    }
+    if (!desc) return tc_fail(TC_ERR_INVALID, "tc_set_bev: null description");
+    const TcBevDesc &d = *desc;
+    if (d.height <= 0 || d.width <= 0 || d.height > 4096 || d.width > 4096) return tc_fail(TC_ERR_INVALID, "tc_set_bev: bad resolution");
+    if (!(std::isfinite(d.pixel_per_meter) && d.pixel_per_meter > 0)) return tc_fail(TC_ERR_INVALID, "tc_set_bev: pixel_per_meter must be finite and > 0");
+    if (!std::isfinite(d.car_col) || !std::isfinite(d.car_row)) return tc_fail(TC_ERR_INVALID, "tc_set_bev: car pixel must be finite");
+    if (d.line_thickness < 1 || d.line_thickness > 8) return tc_fail(TC_ERR_INVALID, "tc_set_bev: line_thickness must be in 1..8");
+    if (d.route != 0 && d.route != 1) return tc_fail(TC_ERR_INVALID, "tc_set_bev: route must be 0 or 1");
+    if (d.format != TC_OBS_CLASSES && d.format != TC_OBS_CLASSES_BITS) return tc_fail(TC_ERR_INVALID, "tc_set_bev: format must be TC_OBS_CLASSES or TC_OBS_CLASSES_BITS");
+    if (d.format == TC_OBS_CLASSES_BITS && ((size_t)d.height * d.width) % 32 != 0) return tc_fail(TC_ERR_INVALID, "tc_set_bev: the bit-packed format needs H*W to be a multiple of 32");
+    const int planes = h->C + d.route;
+    if (planes > TC_MAX_CLASSES) return tc_fail(TC_ERR_INVALID, "tc_set_bev: more than 16 planes");
+    const size_t words = ((size_t)planes * d.height * d.width + 31) / 32 + 1;
+    if (tc_bev_smem_bytes((int)std::min<size_t>(words, 1 << 28)) > TC_BEV_SMEM_MAX) return tc_fail(TC_ERR_INVALID, "tc_set_bev: the BEV planes do not fit the kernel's shared memory");
+    TC_CUDA(cudaSetDevice(h->device));
+    TC_CUDA(tc_allow_max_smem(tc_bev_kernel));
+    h->bev = d; h->bev_out = dev_bev; h->bev_planes = planes; h->bev_plane_words = (int)words;
+    return TC_OK;
+}
+
+int tc_render_bev(TcHandle *h, const uint8_t *dev_mask, void *stream) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_render_bev: null handle");
+    if (!h->bev_out) return tc_fail(TC_ERR_STATE, "tc_render_bev: no BEV set (tc_set_bev)");
+    TC_CUDA(cudaSetDevice(h->device));
+    return tc_launch_bev(h, dev_mask, (cudaStream_t)stream);
+}
+
 int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_nodes, const TcOutputs *outs, void *stream) {
     if (!h) return tc_fail(TC_ERR_INVALID, "tc_reset: null handle");
     if (!dev_spawn_nodes && !h->rng) return tc_fail(TC_ERR_STATE, "tc_reset: no spawn nodes given and no spawn streams set (tc_set_spawn_rng)");
@@ -690,6 +738,7 @@ int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_node
     TC_TRY(tc_launch_track(h, 1, nullptr, nullptr, dev_mask, dev_spawn_nodes, outs, st));
     if (outs && (outs->obs || outs->seg_count || outs->seg_i32))
         TC_TRY(tc_launch_render(h, dev_mask, outs->obs, h->obs_format, outs->seg_count, outs->seg_i32, st));
+    if (h->bev_out) TC_TRY(tc_launch_bev(h, dev_mask, st));
     return TC_OK;
 }
 
@@ -724,6 +773,7 @@ static int tc_step_impl(TcHandle *h, const float *dev_car_control, const double 
         TC_CUDA(cudaEventRecord(ev[3], st));
         h->prof_used++;
     }
+    if (h->bev_out) TC_TRY(tc_launch_bev(h, nullptr, st));
     return TC_OK;
 }
 

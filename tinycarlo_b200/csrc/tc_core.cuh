@@ -1065,3 +1065,47 @@ TC_HD void tc_polyline2(const TcLanes &g, const TcPlane &pl, int32_t x0, int32_t
     for (int i = 0; i < TC_MAX_PRIMS_PER_SEG; i++)
         if (prims[i].kind != TC_PRIM_NONE) tc_prim_draw(g, pl, prims[i]);
 }
+
+// ------------------------------------------------------------------------------------------------ bird's-eye view
+// The BEV contract (include/tinycarlo_b200.h, tc_set_bev): a map point -> BEV pixel, float64 in the contract's order (the
+// library is built without FMA contraction), truncated like np.int32
+TC_HD void tc_bev_point(double x, double y, double c, double s, double k, double col0, double row0, double px, double py, int32_t &u,
+                        int32_t &v) {
+    const double dx = px - x, dy = py - y;
+    u = tc_np_int32(col0 + k * (dy * c - dx * s));
+    v = tc_np_int32(row0 - k * (dx * c + dy * s));
+}
+
+struct TcBevGeom {
+    double k, col0, row0;
+    int H, W, thickness, route;
+};
+
+// BEV segment i of one env: laneline edges 0..sumE-1 in table order (plane = their class), then - route on - the local-path
+// edges sumE..sumE+3 (plane C). Returns false when there is no such segment or when cv2.polylines provably draws nothing for
+// it: both endpoints lie beyond the same side of the frame grown by t+1 pixels (a thick line reaches at most (t+1)/2 + 1
+// pixels beyond the segment between its endpoints).
+TC_HD bool tc_bev_segment(const TcTrackTables &tt, const TcBevGeom &g, double x, double y, double c, double s, const int32_t *si, int i,
+                          int32_t (&p)[4], int &plane) {
+    const int C = tt.n_classes, sumE = tt.ll_edge_off[C];
+    double ax, ay, bx, by;
+    if (i < sumE) {
+        int cls = 0;
+        while (i >= tt.ll_edge_off[cls + 1]) cls++;
+        const double *nodes = tt.ll_nodes + 2 * tt.ll_node_off[cls];
+        const int32_t n0 = tt.ll_edges[2 * i], n1 = tt.ll_edges[2 * i + 1];
+        ax = nodes[2 * n0]; ay = nodes[2 * n0 + 1]; bx = nodes[2 * n1]; by = nodes[2 * n1 + 1];
+        plane = cls;
+    } else {
+        const int j = i - sumE;
+        if (!g.route || j >= 4 || j >= si[TC_SI_PATH_LEN]) return false;
+        const int32_t n0 = si[TC_SI_PATH_NODES + 2 * j], n1 = si[TC_SI_PATH_NODES + 2 * j + 1];
+        if (n0 < 0 || n0 >= tt.lp_n_nodes || n1 < 0 || n1 >= tt.lp_n_nodes) return false;
+        ax = tt.lp_nodes[2 * n0]; ay = tt.lp_nodes[2 * n0 + 1]; bx = tt.lp_nodes[2 * n1]; by = tt.lp_nodes[2 * n1 + 1];
+        plane = C;
+    }
+    tc_bev_point(x, y, c, s, g.k, g.col0, g.row0, ax, ay, p[0], p[1]);
+    tc_bev_point(x, y, c, s, g.k, g.col0, g.row0, bx, by, p[2], p[3]);
+    const int64_t m = g.thickness + 1, r = (int64_t)g.W - 1 + m, b = (int64_t)g.H - 1 + m;
+    return !((p[0] < -m && p[2] < -m) || (p[1] < -m && p[3] < -m) || (p[0] > r && p[2] > r) || (p[1] > b && p[3] > b));
+}

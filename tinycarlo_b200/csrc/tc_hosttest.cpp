@@ -181,6 +181,30 @@ HT_API void ht_polyline(uint8_t *img, int H, int W, int32_t x0, int32_t y0, int3
         if ((plane[p >> 5] >> (p & 31)) & 1) img[(size_t)y_lo * W + p] = 255;
 }
 
+// mirrors tc_bev_kernel for n envs at state rows sf [n,TC_SF_N] / si [n,TC_SI_N] (the route planes read the local path from
+// si); out: u8 [n,P,H,W] 0/255, P = C + route (cos / sin are the host libm's)
+HT_API void ht_bev(const HtMap *m, int n, const double *sf, const int32_t *si, const TcBevDesc *d, uint8_t *out) {
+    const TcTrackTables tt = tc_track_tables(m->pk.blob.data(), m->pk.L);
+    const TcBevGeom g = {d->pixel_per_meter, d->car_col, d->car_row, d->height, d->width, d->line_thickness, d->route};
+    const int P = m->C + (d->route ? 1 : 0), H = d->height, W = d->width;
+    const size_t npx = (size_t)P * H * W;
+    const TcLanes lanes = {0, 1};
+    for (int env = 0; env < n; env++) {
+        const double *s = sf + (size_t)env * TC_SF_N;
+        const int32_t *r = si + (size_t)env * TC_SI_N;
+        const double c = cos(s[TC_SF_ROT]), sn = sin(s[TC_SF_ROT]);
+        std::vector<uint32_t> plane(npx / 32 + 2, 0);
+        for (int i = 0; i < m->sumE + 4; i++) {
+            int32_t p[4];
+            int q = 0;
+            if (!tc_bev_segment(tt, g, s[TC_SF_X], s[TC_SF_Y], c, sn, r, i, p, q)) continue;
+            const TcPlane pl = {plane.data(), H, W, 0, H, -q * H};
+            tc_polyline2(lanes, pl, p[0], p[1], p[2], p[3], g.thickness);
+        }
+        for (size_t b = 0; b < npx; b++) out[(size_t)env * npx + b] = ((plane[b >> 5] >> (b & 31)) & 1) ? 255 : 0;
+    }
+}
+
 // the reset paths' spawn draws (tc_spawn_draw): k consecutive draws of n env streams, states advanced in place
 HT_API void ht_spawn_draws(const HtMap *m, int n, uint64_t *rng_state, const int32_t *spawn_points, int n_spawn_points, int k, int32_t *out) {
     TcTrackTables t = tc_track_tables(m->pk.blob.data(), m->pk.L);

@@ -1729,6 +1729,61 @@ __global__ void __launch_bounds__(256, TC_ENVB_MIN_BLOCKS) tc_render_env_banded_
     }
 }
 
+// ------------------------------------------------------------------------------------------------ bird's-eye view
+// tc_set_bev's contract (include/tinycarlo_b200.h). A block per env: every warp takes 32 segments at a time (lane = segment),
+// transforms their endpoints straight from the map tables (a few hundred edges: a brute-force pass, no visible-set tables),
+// drops the ones cv2 provably draws nothing for (tc_bev_segment) and draws each survivor with all 32 lanes (tc_polyline2)
+// into the stacked P*H-row bit plane in shared memory; then the block stores the planes.
+#define TC_BEV_THREADS 256
+#define TC_BEV_SMEM_MAX (200 * 1024)   // the stacked plane (tinycarlo_b200/config.py bev_params checks the same bound)
+struct TcBevArgs {
+    const unsigned char *blob;   // map tables (tc_track_tables)
+    TcBlobLayout layout;
+    const double *sf;            // [N,TC_SF_N]
+    const int32_t *si;           // [N,TC_SI_N]
+    TcBevGeom g;
+    int n_envs, planes, plane_words, format;   // plane_words: words of the stacked plane incl. the pad word
+    const uint8_t *mask;         // optional
+    uint8_t *out;
+};
+__host__ __device__ inline size_t tc_bev_smem_bytes(int plane_words) { return ((size_t)plane_words * 4 + 15) & ~(size_t)15; }
+
+__global__ void __launch_bounds__(TC_BEV_THREADS) tc_bev_kernel(const TcBevArgs a) {
+    extern __shared__ __align__(16) uint32_t plane[];
+    __shared__ int drew;
+    const int env = blockIdx.x, tid = threadIdx.x;
+    if (a.mask && !a.mask[env]) return;
+    const TcTrackTables tt = tc_track_tables(a.blob, a.layout);
+    const double *sf = a.sf + (size_t)env * TC_SF_N;
+    const int32_t *si = a.si + (size_t)env * TC_SI_N;
+    const double x = sf[TC_SF_X], y = sf[TC_SF_Y], c = cos(sf[TC_SF_ROT]), s = sin(sf[TC_SF_ROT]);
+    for (int i = tid; i < a.plane_words; i += TC_BEV_THREADS) plane[i] = 0;
+    if (tid == 0) drew = 0;
+    __syncthreads();
+    const int H = a.g.H, W = a.g.W, n_seg = a.layout.sum_edges + (a.g.route ? 4 : 0);
+    const TcLanes g = {(int)(tid & 31), 32};
+    for (int base = (tid >> 5) * 32; base < n_seg; base += TC_BEV_THREADS) {   // uniform trip count within a warp
+        int32_t p[4] = {0, 0, 0, 0};
+        int pl_idx = 0;
+        const bool keep = base + g.lane < n_seg && tc_bev_segment(tt, a.g, x, y, c, s, si, base + g.lane, p, pl_idx);
+        unsigned todo = __ballot_sync(0xffffffffu, keep);
+        if (todo && g.lane == 0) drew = 1;
+        while (todo) {
+            const int src = __ffs(todo) - 1;
+            todo &= todo - 1;
+            const int q = __shfl_sync(0xffffffffu, pl_idx, src);
+            const TcPlane pl = {plane, H, W, 0, H, -q * H};
+            tc_polyline2(g, pl, __shfl_sync(0xffffffffu, p[0], src), __shfl_sync(0xffffffffu, p[1], src), __shfl_sync(0xffffffffu, p[2], src),
+                         __shfl_sync(0xffffffffu, p[3], src), a.g.thickness);
+        }
+    }
+    __syncthreads();
+    const size_t npx = (size_t)a.planes * H * W;
+    if (a.format == TC_OBS_CLASSES_BITS)   // H*W % 32 == 0 (tc_set_bev): the planes are whole words
+        tc_store_bits<TC_BEV_THREADS>((uint32_t *)a.out + (size_t)env * (npx / 32), (int)(npx / 32), plane, drew != 0);
+    else tc_store_plane_sparse<TC_BEV_THREADS>(a.out + (size_t)env * npx, npx, plane, drew != 0);
+}
+
 // ------------------------------------------------------------------------------------------------ blob noise
 // NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) on the device: per class, n_blobs filled circles that
 // either erase the class mask or OR in the pixels of a randomly chosen class, applied in the reference's order (classes

@@ -162,8 +162,11 @@ class TinyCarloEnv(gc.Env):
             cte, he, vel = float(i64[0]), float(i64[1]), float(i64[2])
         else:
             local_path, dist, cte, he, vel = [], {n: 0 for n in names}, 0, 0, 0.0
-        return {"cte": cte, "heading_error": he, "position": [float(sf[0]), float(sf[1])], "orientation": float(sf[2]),
+        info = {"cte": cte, "heading_error": he, "position": [float(sf[0]), float(sf[1])], "orientation": float(sf[2]),
                 "laneline_distances": dist, "local_path": local_path, "velocity": vel}
+        if v.bev is not None:   # the config's `bev` section (an extension): this env's bird's-eye view
+            info["bev"] = v.bev[0].cpu().numpy()
+        return info
 
     def reset(self, seed: Optional[int] = None, options: Optional[Any] = None) -> Tuple[np.ndarray, Dict[str, Any]]:
         super().reset(seed=seed)

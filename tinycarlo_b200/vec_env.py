@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from .camera_params import camera_row
-from .config import camera_params, car_param_row, load_config, resolve_map_path, sim_params
+from .config import bev_params, camera_params, car_param_row, load_config, resolve_map_path, sim_params
 from .maptables import MapTables
 from .spawn import spawn_stream_states
 
@@ -99,6 +99,19 @@ class TinyCarloVecEnv:
             if debug_segments:
                 self.out["seg_count"] = torch.zeros((N, Cn), dtype=torch.int32, device=dev)
                 self.out["seg_i32"] = torch.zeros((N, max(int(m.ll_edge_off[-1]), 1), 4), dtype=torch.int32, device=dev)
+            # bird's-eye view (config section `bev`, tc_set_bev): [N,P,H,W] u8 or [N,P,H*W/32] int32, rewritten by every
+            # step() / reset() whatever no_observation says; None without the section
+            self.bev_cfg = bev_params(self.config, Cn)
+            self.bev = None
+            if self.bev_cfg is not None:
+                b = self.bev_cfg
+                bh, bw = b["resolution"]
+                bits = b["format"] == "classes_bits"
+                self.bev = torch.zeros((N, b["planes"]) + ((bh * bw // 32,) if bits else (bh, bw)), dtype=torch.int32 if bits else torch.uint8,
+                                       device=dev)
+                bdesc = _lib.TcBevDesc(bh, bw, b["pixel_per_meter"], b["car_pixel"][0], b["car_pixel"][1], b["line_thickness"], int(b["route"]),
+                                       _lib.TC_OBS_CLASSES_BITS if bits else _lib.TC_OBS_CLASSES)
+                _lib.check(self._L.tc_set_bev(self._h, C.byref(bdesc), _ptr(self.bev)), "tc_set_bev")
             self._spawn_nodes = torch.full((N,), -1, dtype=torch.int32, device=dev)   # node of each env's latest reset
             self._mask_all = torch.ones(N, dtype=torch.uint8, device=dev)
         self._outs = self._make_outputs(with_obs=True)
@@ -266,9 +279,12 @@ class TinyCarloVecEnv:
     # ------------------------------------------------------------------------------------------------ gym-like API
     def _info(self) -> Dict[str, torch.Tensor]:
         o = self.out
-        return {"cte": o["cte"], "heading_error": o["heading_error"], "position": o["position"], "orientation": o["orientation"],
+        info = {"cte": o["cte"], "heading_error": o["heading_error"], "position": o["position"], "orientation": o["orientation"],
                 "laneline_distances": o["laneline_distances"], "local_path": o["local_path"], "velocity": o["velocity"],
                 "nearest_edge": o["nearest_edge"], "local_path_nodes": o["local_path_nodes"], "path_len": o["path_len"]}
+        if self.bev is not None:
+            info["bev"] = self.bev
+        return info
 
     def reset(self, seed: Optional[int] = None, mask: Optional[torch.Tensor] = None, spawn_nodes: Optional[torch.Tensor] = None):
         """env.py:101-113 for the envs selected by `mask` (bool/uint8 [N]; None = all). seed re-seeds every env's spawn
@@ -417,6 +433,15 @@ class TinyCarloVecEnv:
         return self._overview.render([float(sf[0]), float(sf[1])], float(sf[2]), float(sf[3]), float(self._car_rows[env_index, 0]),
                                      float(self._car_rows[env_index, 1]), path)
 
+    def render_bev(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Re-render self.bev (the config's `bev` section) at the current poses for the envs in `mask` (None = all)."""
+        if self.bev is None:
+            raise ValueError("render_bev: the config has no `bev` section")
+        with torch.cuda.device(self.device):
+            m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            _lib.check(self._L.tc_render_bev(self._h, _ptr(m), self._stream()), "tc_render_bev")
+        return self.bev
+
     def render_obs(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Re-render self.obs at the current poses (after load_state_dict / set_camera_params)."""
         with torch.cuda.device(self.device):
@@ -455,6 +480,8 @@ class TinyCarloVecEnv:
         if "done_flags" in ck and self.autoreset:
             self.done_flags.copy_(ck["done_flags"])
         self.render_obs()
+        if self.bev is not None:
+            self.render_bev()
 
     def load_state_dict(self, state: Dict[str, torch.Tensor]):
         with torch.cuda.device(self.device):
