@@ -122,7 +122,9 @@ TC_API int tc_destroy(TcHandle *h);
 
 TC_API int tc_set_car_params(TcHandle *h, const double *dev_params /*[N,TC_CP_N]*/, void *stream);
 /* Handles that render small frames with one block per env (C*H*W <= 128 KB) read the rows back in this call and rebuild
- * their visible-set tables when the cameras' reach changed: the call then synchronises the stream (it is a set-up call). */
+ * their visible-set tables when the cameras' reach changed: the call then synchronises the stream (it is a set-up call).
+ * dev_thickness: line thickness per env in 1..255, as cv2.polylines draws it; the rasteriser's 16.16 fixed-point set-up needs
+ * max(H, W) + 2 * thickness < 2^15. The device array is not checked here: the Python env validates it (ValueError). */
 TC_API int tc_set_camera_params(TcHandle *h, const double *dev_cam /*[N,TC_CAM_N]*/, const int32_t *dev_thickness /*[N]*/, void *stream);
 /* The same with the caller's HOST copy of the rows (host_cam [N,TC_CAM_N], may be NULL): how far the cameras see decides which
  * visible-set tables the small-frame render kernels use, and with the host copy that decision needs no read-back, so the

@@ -57,9 +57,17 @@ def car_param_row(car_config: Dict[str, Any], T: float):
             g("steering_speed", None), g("max_acceleration", None), g("max_deceleration", None), float(T)]
 
 
+LINE_THICKNESS_MAX = 255   # the rasteriser's 16.16 fixed-point set-up needs max(H, W) + 2 * thickness < 2^15
+
+
+def is_line_thickness(t) -> bool:
+    """camera line thickness: an integer in 1..LINE_THICKNESS_MAX (cv2.polylines rejects 0 and negative values)"""
+    return isinstance(t, numbers.Integral) and not isinstance(t, bool) and 1 <= t <= LINE_THICKNESS_MAX
+
+
 def camera_params(camera_config: Dict[str, Any]) -> Dict[str, Any]:
     """camera.py:16-21 defaults. max_range=None crashes the reference on the first frame (camera.py:80-82, SURVEY
-    section 5); it is rejected here at construction."""
+    section 5); it is rejected here at construction, as is a line_thickness outside 1..255."""
     cam = {"resolution": list(camera_config.get("resolution", [128, 160])),
            "position": list(camera_config.get("position", [0, 0, 0])),
            "orientation": list(camera_config.get("orientation", [0, 0, 0])),
@@ -68,6 +76,9 @@ def camera_params(camera_config: Dict[str, Any]) -> Dict[str, Any]:
            "line_thickness": camera_config.get("line_thickness", 1)}
     if not cam["max_range"]:
         raise ValueError("camera.max_range must be a positive number (the reference raises on the first frame when it is None)")
+    if not is_line_thickness(cam["line_thickness"]):
+        raise ValueError(f"camera.line_thickness must be an integer in 1..{LINE_THICKNESS_MAX}, got {cam['line_thickness']!r}")
+    cam["line_thickness"] = int(cam["line_thickness"])
     return cam
 
 

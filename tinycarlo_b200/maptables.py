@@ -9,6 +9,8 @@ from typing import Any, Dict, List, Optional
 
 import numpy as np
 
+MAX_CLASSES = 16   # TC_MAX_CLASSES (include/tinycarlo_b200.h): laneline layers a map may have
+
 
 class MapTables:
     def __init__(self, map_json, pixel_per_meter, spawn_points: Optional[List[int]] = None):
@@ -61,6 +63,9 @@ class MapTables:
             bad("top level must be an object")
         if not isinstance(data.get("lanelines"), dict) or not data["lanelines"]:
             bad("'lanelines' must be a non-empty object of laneline layers")
+        if len(data["lanelines"]) > MAX_CLASSES:
+            bad(f"{len(data['lanelines'])} laneline layers; the render kernels support at most {MAX_CLASSES} (one observation "
+                "plane and one colour per layer)")
         if not isinstance(data.get("lanepath"), dict):
             bad("'lanepath' layer is missing")
 

@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from .camera_params import camera_row
-from .config import bev_params, camera_params, car_param_row, load_config, resolve_map_path, sim_params
+from .config import LINE_THICKNESS_MAX, bev_params, camera_params, car_param_row, load_config, resolve_map_path, sim_params
 from .maptables import MapTables
 from .spawn import spawn_stream_states
 
@@ -227,11 +227,21 @@ class TinyCarloVecEnv:
             if not np.all(np.isfinite(v)) or (positive and not np.all(v > 0)):
                 raise ValueError(f"car.{name} must be finite" + (" and > 0" if positive else ""))
 
+    @staticmethod
+    def _thickness_rows(v, shape) -> np.ndarray:
+        """Per-env line thicknesses as int32 of `shape`: integers in 1..255 like the config's camera.line_thickness (0 and
+        negative values would draw 1-pixel lines where cv2.polylines raises; larger ones leave the rasteriser's 16.16 range)."""
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer) or not ((a >= 1) & (a <= LINE_THICKNESS_MAX)).all():
+            raise ValueError(f"camera.line_thickness must be integers in 1..{LINE_THICKNESS_MAX}, got {v!r}")
+        return np.broadcast_to(a, shape).astype(np.int32)
+
     def set_camera_params(self, position=None, orientation=None, fov=None, max_range=None, line_thickness=None, env_ids=None):
         """Per-env camera parameters (camera.py:48-50 update_params, vectorised). Arrays are [n,3] / [n] for the envs in
         env_ids (default: all), or a single value broadcast. E and K are rebuilt on the host with the reference's calls."""
         ids = np.arange(self.num_envs) if env_ids is None else np.asarray(env_ids).reshape(-1)
         n = len(ids)
+        thickness = None if line_thickness is None else self._thickness_rows(line_thickness, (n,))
         if not hasattr(self, "_cam_src"):
             cc = self.cam_cfg
             self._cam_src = {"position": np.tile(np.asarray(cc["position"], np.float64), (self.num_envs, 1)),
@@ -249,8 +259,8 @@ class TinyCarloVecEnv:
             self._cam_src["fov"][ids] = bc(fov, (n,))
         if max_range is not None:
             self._cam_src["max_range"][ids] = bc(max_range, (n,))
-        if line_thickness is not None:
-            self._thickness[ids] = bc(line_thickness, (n,)).astype(np.int32)
+        if thickness is not None:
+            self._thickness[ids] = thickness
         res = [self.H, self.W]
         s = self._cam_src
         cache = {}
@@ -264,9 +274,10 @@ class TinyCarloVecEnv:
 
     def set_camera_rows(self, cam_rows: np.ndarray, line_thickness=None):
         """Raw per-env camera rows [N,20] (E 3x4 row-major, fx, fy, cx, cy, max_range, pad) — include/tinycarlo_b200.h TC_CAM_*."""
+        thickness = None if line_thickness is None else self._thickness_rows(line_thickness, (self.num_envs,))
         self._cam_rows[:] = np.asarray(cam_rows, np.float64).reshape(self.num_envs, _lib.TC_CAM_N)
-        if line_thickness is not None:
-            self._thickness[:] = np.asarray(line_thickness, np.int32)
+        if thickness is not None:
+            self._thickness[:] = thickness
         self._upload_params()
 
     # ------------------------------------------------------------------------------------------------ spawn draws
