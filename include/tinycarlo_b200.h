@@ -5,6 +5,7 @@
  * What each entry point replaces in the reference (paths relative to the reference checkout):
  *   tc_create              TinyCarloEnv.__init__ staging: Map.__init__ (tinycarlo/map.py:9-37), Layer tables
  *                          (tinycarlo/layer.py:15-19), Car.__init__ (tinycarlo/car.py:10-32)
+ *   tc_create_rig          the same with several cameras per car (the reference has one), each rendered as its own view
  *   tc_set_car_params      Car.__init__ parameters (tinycarlo/car.py:12-18), one row per env
  *   tc_set_camera_params   Camera.__init__/update_params (tinycarlo/camera.py:12-27,48-50): E (3x4), K, max_range,
  *                          line_thickness per env; E and K are built on the host (camera.py:145-178)
@@ -118,6 +119,23 @@ TC_API const char *tc_last_error(void);
 TC_API const char *tc_build_info(void);
 
 TC_API int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int32_t device, TcHandle **out);
+/* Camera rig: a handle of N envs with M = n_cameras >= 1 cameras per car (tc_create is tc_create_rig with M = 1). View
+ * v = i*M + m is camera m of env i; the order is env-major, so observations read as [N, M, ...].
+ *
+ *   camera rows, thicknesses   dev_cam [N*M, TC_CAM_N], dev_thickness [N*M] of tc_set_camera_params(_host): row v for view v
+ *   pose of view v             tc_camera_pose(E of row v, state of env i): a view's frame is exactly what a one-camera handle
+ *                              renders for that camera row and that car state
+ *   obs                        N*M frames in the handle's format, all of one resolution: u8 [N,M,C,H,W], RGB [N,M,H,W,3],
+ *                              bits [N,M,C,ceil(H*W/32)], bf16 [N,M,C,H,W]
+ *   masks                      of tc_reset, tc_render and tc_render_bev stay per env [N]: an env's mask selects all its views
+ *   per-env outputs            state, TcOutputs except seg_*, flags, spawn draws and the BEV stay per env [N]
+ *   per-view outputs           seg_count [N*M, C], seg_i32 [N*M, sumE, 4], the tc_debug_set_timeline buffer [N*M*C][10]
+ *   tc_noise_blobs             obs [N*M, C, H, W]; Philox counter (env_index_offset + i, step, c * n_blobs + blob, m)
+ *   tc_step_host_obs           obs_bytes covers all views
+ *
+ * The visible-set tables of the small-frame kernels are built for the largest reach over all N*M camera rows. Fails with
+ * TC_ERR_INVALID for n_cameras < 1 or num_envs * n_cameras * C > 2^31 - 1 (the per-class grids index blocks with an int). */
+TC_API int tc_create_rig(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int32_t n_cameras, int32_t device, TcHandle **out);
 TC_API int tc_destroy(TcHandle *h);
 
 TC_API int tc_set_car_params(TcHandle *h, const double *dev_params /*[N,TC_CP_N]*/, void *stream);
@@ -182,7 +200,8 @@ TC_API int tc_step_host_obs(TcHandle *h, const float *host_car_control, const in
  * n_blobs filled circles (centre uniform in the frame, radius uniform in [1, max_radius)), each with probability 0.3 ORs in
  * the pixels of a random class inside the circle, else erases the circle; classes ascending, blobs in sequence, like the
  * reference. The reference draws from numpy's unseeded global RNG; here the draw of (env, step, class, blob) is
- * Philox4x32-10 with key = seed and counter = (env_index_offset + env, step, class * n_blobs + blob, 0):
+ * Philox4x32-10 with key = seed and counter = (env_index_offset + env, step, class * n_blobs + blob, camera) (camera 0
+ * without a rig, see tc_create_rig; dev_mask is per env):
  * x = r0 % W, y = r1 % H, radius = 1 + r2 % (max_radius - 1), copy = (r3 & 0xffff) < 19661, source class = (r3 >> 16) % C. */
 TC_API int tc_noise_blobs(TcHandle *h, uint8_t *dev_obs, uint64_t seed, uint32_t step, int32_t n_blobs, int32_t max_radius,
                           int32_t env_index_offset, const uint8_t *dev_mask, void *stream);

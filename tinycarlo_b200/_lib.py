@@ -118,6 +118,7 @@ def lib():
     L.tc_last_error.restype = C.c_char_p
     L.tc_build_info.restype = C.c_char_p
     L.tc_create.argtypes = [C.POINTER(TcMapDesc), C.POINTER(TcSimDesc), i32, i32, C.POINTER(vp)]
+    L.tc_create_rig.argtypes = [C.POINTER(TcMapDesc), C.POINTER(TcSimDesc), i32, i32, i32, C.POINTER(vp)]
     L.tc_destroy.argtypes = [vp]
     L.tc_set_car_params.argtypes = [vp, vp, vp]
     L.tc_set_camera_params.argtypes = [vp, vp, vp, vp]
@@ -147,7 +148,7 @@ def lib():
     L.tc_profile_begin.argtypes = [vp, i32]
     L.tc_profile_end.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32)]
     L.tc_debug_layer_query.argtypes = [vp, i32, C.c_double, C.c_double, C.c_double, i32, i32, vp, vp, vp]
-    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_create", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
+    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_create", "tc_create_rig", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
                  "tc_render", "tc_get_state", "tc_set_state", "tc_step_host", "tc_debug_layer_query", "tc_profile_begin", "tc_profile_end"):
         getattr(L, name).restype = C.c_int
     if L.tc_abi_version() != 1:

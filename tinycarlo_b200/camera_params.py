@@ -32,3 +32,11 @@ def camera_row(position, orientation, fov, resolution, max_range) -> np.ndarray:
     row[12], row[13], row[14], row[15] = K[0, 0], K[1, 1], K[0, 2], K[1, 2]
     row[16] = float(max_range)
     return row
+
+
+def view_rows(cam_cfgs, n_envs: int):
+    """Camera rows [n_envs*M, 20] and line thicknesses int32 [n_envs*M] for M camera sections (config.camera_params), one per
+    view in env-major order: view v = env * M + m has camera m (include/tinycarlo_b200.h tc_create_rig)."""
+    rows = np.stack([camera_row(c["position"], c["orientation"], c["fov"], c["resolution"], c["max_range"]) for c in cam_cfgs])
+    thickness = np.array([int(c["line_thickness"]) for c in cam_cfgs], np.int32)
+    return np.tile(rows, (n_envs, 1)), np.tile(thickness, n_envs)

@@ -4,7 +4,7 @@ the mandatory sections sim / car / camera / map (a missing section raises KeyErr
 import math
 import numbers
 import os
-from typing import Any, Dict, Optional, Tuple, Union
+from typing import Any, Dict, List, Optional, Tuple, Union
 
 MAPS_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "maps")
 
@@ -80,6 +80,34 @@ def camera_params(camera_config: Dict[str, Any]) -> Dict[str, Any]:
         raise ValueError(f"camera.line_thickness must be an integer in 1..{LINE_THICKNESS_MAX}, got {cam['line_thickness']!r}")
     cam["line_thickness"] = int(cam["line_thickness"])
     return cam
+
+
+RIG_KEYS = ("position", "orientation", "fov", "max_range", "line_thickness")
+
+
+def camera_rig(config: Dict[str, Any]) -> Optional[List[Dict[str, Any]]]:
+    """The optional top-level `cameras` list (an extension: several cameras per car, include/tinycarlo_b200.h tc_create_rig):
+    one camera_params() section per entry, each the config's `camera` section with the entry's keys overriding it ({} is that
+    camera itself), or None when the config has no such key. All cameras share camera.resolution: an entry with its own
+    resolution raises ValueError, as do unknown keys (per-camera resolutions are what TinyCarloGroupedVecEnv's groups are for)."""
+    rig = config.get("cameras")
+    if rig is None:
+        return None
+    if not isinstance(rig, list) or not rig:
+        raise ValueError(f"cameras must be a non-empty list of mappings, got {rig!r}")
+    out = []
+    for k, entry in enumerate(rig):
+        if not isinstance(entry, dict):
+            raise ValueError(f"cameras[{k}] must be a mapping, got {entry!r}")
+        if "resolution" in entry:
+            raise ValueError(f"cameras[{k}]: all cameras share camera.resolution (use TinyCarloGroupedVecEnv for several resolutions)")
+        unknown = sorted(set(entry) - set(RIG_KEYS))
+        if unknown:
+            raise ValueError(f"cameras[{k}]: unknown keys {unknown} (allowed: {list(RIG_KEYS)})")
+        merged = dict(config["camera"])
+        merged.update(entry)
+        out.append(camera_params(merged))
+    return out
 
 
 BEV_MAX_CLASSES = 16              # TC_MAX_CLASSES: planes of one BEV

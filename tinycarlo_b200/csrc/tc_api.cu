@@ -52,6 +52,7 @@ struct TcCullSet {
 struct TcHandle {
     int device = 0;
     int n_envs = 0, C = 0, H = 0, W = 0, obs_format = 0;
+    int n_cams = 1, n_views = 0;   // cameras per env; views v = env * n_cams + m, what the render kernels see as their "envs"
     int sum_nodes = 0, sum_edges = 0, max_nodes = 0;
     int wrapped = 0;
     bool car_set = false, cam_set = false;
@@ -66,8 +67,9 @@ struct TcHandle {
     int32_t *d_edge_off = nullptr;
     double *d_sf = nullptr;
     int32_t *d_si = nullptr;
-    double *d_car = nullptr, *d_cam = nullptr, *d_pose = nullptr;
+    double *d_car = nullptr, *d_cam = nullptr, *d_pose = nullptr;   // d_cam, d_pose, d_thick: per view
     int32_t *d_thick = nullptr;
+    uint8_t *d_view_mask = nullptr;   // [n_views]: the caller's per-env mask spread over the views (rigs only)
     int32_t *d_seg = nullptr, *d_seg_count = nullptr;
     float *d_act_cc = nullptr; // staging for tc_step_host
     int32_t *d_act_man = nullptr;
@@ -252,10 +254,17 @@ int tc_destroy(TcHandle *h) {
 }
 
 int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int32_t device, TcHandle **out) {
+    return tc_create_rig(map, sim, num_envs, 1, device, out);
+}
+
+int tc_create_rig(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int32_t n_cameras, int32_t device, TcHandle **out) {
     if (!map || !sim || !out) return tc_fail(TC_ERR_INVALID, "tc_create: null argument");
     if (num_envs <= 0) return tc_fail(TC_ERR_INVALID, "tc_create: num_envs must be positive");
+    if (n_cameras < 1) return tc_fail(TC_ERR_INVALID, "tc_create_rig: n_cameras must be >= 1");
     const int C = map->n_classes;
     if (C <= 0 || C > TC_MAX_CLASSES) return tc_fail(TC_ERR_INVALID, "tc_create: n_classes out of range (1..16)");
+    // the per-class render grids index their blocks (view, class) with an int
+    if ((int64_t)num_envs * n_cameras * C > INT32_MAX) return tc_fail(TC_ERR_INVALID, "tc_create_rig: num_envs * n_cameras * n_classes exceeds 2^31 - 1");
     if (sim->height <= 0 || sim->width <= 0) return tc_fail(TC_ERR_INVALID, "tc_create: bad resolution");
     if (sim->obs_format < TC_OBS_CLASSES || sim->obs_format > TC_OBS_CLASSES_BF16) return tc_fail(TC_ERR_INVALID, "tc_create: bad obs_format");
     TcPacked pk;
@@ -270,7 +279,7 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     TC_CUDA(cudaSetDevice(device));
 
     TcHandle *h = new TcHandle();
-    h->device = device; h->n_envs = num_envs; h->C = C; h->H = sim->height; h->W = sim->width; h->obs_format = sim->obs_format;
+    h->device = device; h->n_envs = num_envs; h->n_cams = n_cameras; h->n_views = num_envs * n_cameras; h->C = C; h->H = sim->height; h->W = sim->width; h->obs_format = sim->obs_format;
     h->sum_nodes = sumN; h->sum_edges = sumE;
     memcpy(h->colors, map->ll_colors, (size_t)3 * C);
     h->m_node_off.assign(map->ll_node_off, map->ll_node_off + C + 1);
@@ -333,15 +342,16 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     }
 
     // ---- per-env buffers
-    const size_t N = (size_t)num_envs;
+    const size_t N = (size_t)num_envs, V = (size_t)h->n_views;
     TC_TRYH(tc_dev_alloc(h, &h->d_sf, N * TC_SF_N));
     TC_TRYH(tc_dev_alloc(h, &h->d_si, N * TC_SI_N));
     TC_TRYH(tc_dev_alloc(h, &h->d_car, N * TC_CP_N));
-    TC_TRYH(tc_dev_alloc(h, &h->d_cam, N * TC_CAM_N));
-    TC_TRYH(tc_dev_alloc(h, &h->d_pose, N * 12));
-    TC_TRYH(tc_dev_alloc(h, &h->d_thick, N));
-    TC_TRYH(tc_dev_alloc(h, &h->d_seg, N * (size_t)std::max(sumE, 1) * 4));
-    TC_TRYH(tc_dev_alloc(h, &h->d_seg_count, N * C));
+    TC_TRYH(tc_dev_alloc(h, &h->d_cam, V * TC_CAM_N));
+    TC_TRYH(tc_dev_alloc(h, &h->d_pose, V * 12));
+    TC_TRYH(tc_dev_alloc(h, &h->d_thick, V));
+    if (n_cameras > 1) TC_TRYH(tc_dev_alloc(h, &h->d_view_mask, V));
+    TC_TRYH(tc_dev_alloc(h, &h->d_seg, V * (size_t)std::max(sumE, 1) * 4));
+    TC_TRYH(tc_dev_alloc(h, &h->d_seg_count, V * C));
     TC_TRYH(tc_dev_alloc(h, &h->d_act_cc, N * 2));
     TC_TRYH(tc_dev_alloc(h, &h->d_act_man, N));
     TC_TRYH(tc_dev_alloc(h, &h->d_h_reward, N));
@@ -351,8 +361,8 @@ int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, int3
     TC_TRYH(tc_dev_alloc(h, &h->d_h_trunc, N));
     TC_CUDAH(cudaMemset(h->d_sf, 0, N * TC_SF_N * sizeof(double)));
     TC_CUDAH(cudaMemset(h->d_si, 0xff, N * TC_SI_N * sizeof(int32_t)));
-    TC_CUDAH(cudaMemset(h->d_seg_count, 0, N * C * sizeof(int32_t)));
-    TC_CUDAH(cudaMemset(h->d_pose, 0, N * 12 * sizeof(double)));
+    TC_CUDAH(cudaMemset(h->d_seg_count, 0, V * C * sizeof(int32_t)));
+    TC_CUDAH(cudaMemset(h->d_pose, 0, V * 12 * sizeof(double)));
 
     // ---- kernel attributes / launch geometry
     h->proj_smem = tc_proj_smem_bytes(h->max_nodes);
@@ -452,20 +462,21 @@ int tc_set_camera_params(TcHandle *h, const double *dev_cam, const int32_t *dev_
 int tc_set_camera_params_host(TcHandle *h, const double *dev_cam, const int32_t *dev_thickness, const double *host_cam, void *stream) {
     if (!h || !dev_cam || !dev_thickness) return tc_fail(TC_ERR_INVALID, "tc_set_camera_params: null argument");
     TC_CUDA(cudaSetDevice(h->device));
-    TC_CUDA(cudaMemcpyAsync(h->d_cam, dev_cam, (size_t)h->n_envs * TC_CAM_N * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
-    TC_CUDA(cudaMemcpyAsync(h->d_thick, dev_thickness, (size_t)h->n_envs * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    TC_CUDA(cudaMemcpyAsync(h->d_cam, dev_cam, (size_t)h->n_views * TC_CAM_N * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    TC_CUDA(cudaMemcpyAsync(h->d_thick, dev_thickness, (size_t)h->n_views * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     h->cam_set = true;
     if (h->fused_all || h->envb_smem > 0 || h->cull_radius >= 0 || !h->cull_sets.empty()) {
         // the visible-set tables depend on how far the cameras see: from the caller's host copy of the rows, or read back (synchronises)
         std::vector<double> rows;
         if (!host_cam) {
-            rows.resize((size_t)h->n_envs * TC_CAM_N);
+            rows.resize((size_t)h->n_views * TC_CAM_N);
             TC_CUDA(cudaMemcpyAsync(rows.data(), h->d_cam, rows.size() * sizeof(double), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
             TC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
             host_cam = rows.data();
         }
+        // the largest reach over all views: tables built for a nearer camera would drop lines a farther one sees
         double radius = 0.0;
-        for (int i = 0; i < h->n_envs && radius >= 0; i++) {
+        for (int i = 0; i < h->n_views && radius >= 0; i++) {
             double r = tc_cull_radius_of(host_cam + (size_t)i * TC_CAM_N, h->H, h->W);
             radius = r < 0 ? -1.0 : std::max(radius, r);
         }
@@ -532,7 +543,7 @@ static TcRenderPath tc_render_path(const TcHandle *h, int obs_format, bool segme
 // arguments of the block-per-env kernels; plane_words: words of the stacked plane of the small-frame kernels, 0 for the others
 static TcRenderEnvArgs tc_render_env_args(const TcHandle *h, const uint8_t *mask, uint8_t *obs, int plane_words) {
     TcRenderEnvArgs ea;
-    ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = h->n_envs; ea.n_classes = h->C;
+    ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = h->n_views; ea.n_classes = h->C;
     ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = plane_words;
     ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = obs;
     memcpy(ea.colors, h->colors, sizeof(ea.colors));
@@ -543,10 +554,11 @@ static TcRenderEnvArgs tc_render_env_args(const TcHandle *h, const uint8_t *mask
     return ea;
 }
 
+// renders the handle's n_views views; mask (NULL = all) is per view
 static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int obs_format, int32_t *seg_count_out, int32_t *seg_out,
                             cudaStream_t st, cudaEvent_t after_project = nullptr) {
     using P = TcRenderPath;
-    const int N = h->n_envs, C = h->C;
+    const int N = h->n_views, C = h->C;
     long long *timeline = mask ? nullptr : h->timeline;
     const P path = tc_render_path(h, obs_format, seg_count_out || seg_out, timeline != nullptr);
     if (obs_format == TC_OBS_CLASSES_BITS || obs_format == TC_OBS_CLASSES_BF16) {
@@ -659,11 +671,13 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
     return TC_OK;
 }
 
+// mask: per env; in reset mode a rig's view mask (tc_view_mask) is written alongside
 static int tc_launch_track(TcHandle *h, int mode, const float *cc, const int32_t *man, const uint8_t *mask, const int32_t *spawn,
                            const TcOutputs *outs, cudaStream_t st, const double *cc64 = nullptr) {
     TcTrackArgs ta;
     memset(&ta, 0, sizeof(ta));
-    ta.blob = h->d_blob; ta.layout = h->layout; ta.n_envs = h->n_envs; ta.mode = mode; ta.wrapped = h->wrapped;
+    ta.blob = h->d_blob; ta.layout = h->layout; ta.n_envs = h->n_envs; ta.n_cams = h->n_cams; ta.mode = mode; ta.wrapped = h->wrapped;
+    ta.view_mask = mode == 1 && mask && h->n_cams > 1 ? h->d_view_mask : nullptr;
     ta.sf = h->d_sf; ta.si = h->d_si; ta.car = h->d_car; ta.cam = h->d_cam; ta.pose = h->d_pose;
     ta.act_cc = cc; ta.act_cc64 = cc64; ta.act_man = man; ta.mask = mask; ta.spawn_nodes = spawn;
     ta.near_x0 = h->near_h.x0; ta.near_y0 = h->near_h.y0; ta.near_inv_cell = h->near_h.inv_cell; ta.near_nx = h->near_h.nx; ta.near_ny = h->near_h.ny;
@@ -683,6 +697,10 @@ static int tc_launch_track(TcHandle *h, int mode, const float *cc, const int32_t
     TC_CUDA(cudaGetLastError());
     return TC_OK;
 }
+
+// the per-view mask the render kernels read for a per-env mask: the caller's own one camera per env, else the handle's
+// view mask, which the reset-mode tracking kernel or tc_pose_kernel writes in the same launch sequence
+static const uint8_t *tc_view_mask(const TcHandle *h, const uint8_t *mask) { return mask && h->n_cams > 1 ? h->d_view_mask : mask; }
 
 static int tc_launch_bev(TcHandle *h, const uint8_t *mask, cudaStream_t st) {
     TcBevArgs a;
@@ -737,7 +755,7 @@ int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_node
     cudaStream_t st = (cudaStream_t)stream;
     TC_TRY(tc_launch_track(h, 1, nullptr, nullptr, dev_mask, dev_spawn_nodes, outs, st));
     if (outs && (outs->obs || outs->seg_count || outs->seg_i32))
-        TC_TRY(tc_launch_render(h, dev_mask, outs->obs, h->obs_format, outs->seg_count, outs->seg_i32, st));
+        TC_TRY(tc_launch_render(h, tc_view_mask(h, dev_mask), outs->obs, h->obs_format, outs->seg_count, outs->seg_i32, st));
     if (h->bev_out) TC_TRY(tc_launch_bev(h, dev_mask, st));
     return TC_OK;
 }
@@ -777,12 +795,15 @@ static int tc_step_impl(TcHandle *h, const float *dev_car_control, const double 
     return TC_OK;
 }
 
-// recompute the camera poses from the current state (after tc_set_state / camera parameter changes)
-__global__ void tc_pose_kernel(int n, const double *sf, const double *cam, double *pose) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+// recompute the camera poses from the current state (after tc_set_state / camera parameter changes): a thread per view
+// v = env * n_cams + m; view_mask (optional) receives mask[env] for the render kernels
+__global__ void tc_pose_kernel(int n_views, int n_cams, const double *sf, const double *cam, double *pose, const uint8_t *mask, uint8_t *view_mask) {
+    int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= n_views) return;
+    const int i = v / n_cams;
+    if (view_mask) view_mask[v] = mask[i];
     const double *s = sf + (size_t)i * TC_SF_N;
-    tc_camera_pose(cam + (size_t)i * TC_CAM_N + TC_CAM_E, s[TC_SF_X], s[TC_SF_Y], cos(s[TC_SF_ROT]), sin(s[TC_SF_ROT]), pose + (size_t)i * 12);
+    tc_camera_pose(cam + (size_t)v * TC_CAM_N + TC_CAM_E, s[TC_SF_X], s[TC_SF_Y], cos(s[TC_SF_ROT]), sin(s[TC_SF_ROT]), pose + (size_t)v * 12);
 }
 
 int tc_render(TcHandle *h, const uint8_t *dev_mask, uint8_t *dev_obs, int32_t obs_format, int32_t *dev_seg_count, int32_t *dev_seg_i32,
@@ -792,10 +813,12 @@ int tc_render(TcHandle *h, const uint8_t *dev_mask, uint8_t *dev_obs, int32_t ob
     if (obs_format < TC_OBS_CLASSES || obs_format > TC_OBS_CLASSES_BF16) return tc_fail(TC_ERR_INVALID, "tc_render: bad obs_format");
     TC_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
-    tc_pose_kernel<<<(h->n_envs + 127) / 128, 128, 0, st>>>(h->n_envs, h->d_sf, h->d_cam, h->d_pose);
+    const uint8_t *view_mask = tc_view_mask(h, dev_mask);
+    tc_pose_kernel<<<(h->n_views + 127) / 128, 128, 0, st>>>(h->n_views, h->n_cams, h->d_sf, h->d_cam, h->d_pose, dev_mask,
+                                                               view_mask != dev_mask ? h->d_view_mask : nullptr);
     h->launches++;
     TC_CUDA(cudaGetLastError());
-    return tc_launch_render(h, dev_mask, dev_obs, obs_format, dev_seg_count, dev_seg_i32, st);
+    return tc_launch_render(h, view_mask, dev_obs, obs_format, dev_seg_count, dev_seg_i32, st);
 }
 
 int tc_get_state(TcHandle *h, double *dev_sf, int32_t *dev_si, void *stream) {
@@ -880,10 +903,10 @@ int tc_noise_blobs(TcHandle *h, uint8_t *dev_obs, uint64_t seed, uint32_t step, 
     if (n_blobs < 0 || max_radius < 1 || max_radius > 1023) return tc_fail(TC_ERR_INVALID, "tc_noise_blobs: max_radius must be in 1..1023, n_blobs >= 0");
     TC_CUDA(cudaSetDevice(h->device));
     TcNoiseArgs na;
-    na.n_envs = h->n_envs; na.n_classes = h->C; na.H = h->H; na.W = h->W; na.n_blobs = n_blobs; na.max_radius = max_radius;
+    na.n_envs = h->n_envs; na.n_cams = h->n_cams; na.n_classes = h->C; na.H = h->H; na.W = h->W; na.n_blobs = n_blobs; na.max_radius = max_radius;
     na.seed_lo = (uint32_t)seed; na.seed_hi = (uint32_t)(seed >> 32); na.step = step; na.env_offset = (uint32_t)env_index_offset;
     na.mask = dev_mask; na.obs = dev_obs;
-    tc_noise_blobs_kernel<<<h->n_envs, 256, 0, (cudaStream_t)stream>>>(na);
+    tc_noise_blobs_kernel<<<h->n_views, 256, 0, (cudaStream_t)stream>>>(na);
     h->launches++;
     TC_CUDA(cudaGetLastError());
     return TC_OK;

@@ -44,10 +44,11 @@ static void ht_attach_near(const HtMap *m, TcTrackTables &t, bool use) {
     t.near_off = m->near.off.data(); t.near_edge = m->near.edge.data();
 }
 
-// mirrors tc_track_kernel for n envs (mode 0 step / 1 reset)
-HT_API void ht_track(const HtMap *m, int n, int mode, int wrapped, double *sf, int32_t *si, const double *car, const double *cam,
-                     double *pose, const float *act_cc, const int32_t *act_man, const uint8_t *mask, const int32_t *spawn,
-                     double *info_f64, int32_t *nearest, uint8_t *terminated, uint8_t *truncated) {
+// mirrors tc_track_kernel for n envs (mode 0 step / 1 reset) with n_cams cameras each: cam / pose are per view
+// v = env * n_cams + m; view_mask (optional, reset with a mask) receives mask[env] for each view, as the kernels write it
+HT_API void ht_track_rig(const HtMap *m, int n, int n_cams, int mode, int wrapped, double *sf, int32_t *si, const double *car, const double *cam,
+                         double *pose, const float *act_cc, const int32_t *act_man, const uint8_t *mask, const int32_t *spawn,
+                         double *info_f64, int32_t *nearest, uint8_t *terminated, uint8_t *truncated, uint8_t *view_mask) {
     TcTrackTables t = tc_track_tables(m->pk.blob.data(), m->pk.L);
     ht_attach_near(m, t, true);
     TcLanes g = {0, 1};
@@ -57,6 +58,7 @@ HT_API void ht_track(const HtMap *m, int n, int mode, int wrapped, double *sf, i
         TcCarState s;
         bool trunc = false;
         if (mode == 1) {
+            if (view_mask && mask) for (int k = 0; k < n_cams; k++) view_mask[(size_t)env * n_cams + k] = mask[env];
             if (mask && !mask[env]) continue;
             tc_load_state(sf + (size_t)env * TC_SF_N, si + (size_t)env * TC_SI_N, s);
             if (!tc_car_reset(t, cp, s, spawn[env])) continue;
@@ -69,13 +71,22 @@ HT_API void ht_track(const HtMap *m, int n, int mode, int wrapped, double *sf, i
         int near[TC_MAX_CLASSES];
         TcInfo info = tc_get_info(g, t, cp, s, wrapped != 0, dist, near);
         tc_store_state(sf + (size_t)env * TC_SF_N, si + (size_t)env * TC_SI_N, s);
-        tc_camera_pose(cam + (size_t)env * TC_CAM_N + TC_CAM_E, s.x, s.y, cos(s.rot), sin(s.rot), pose + (size_t)env * 12);
+        const double c = cos(s.rot), sn = sin(s.rot);
+        for (int k = 0; k < n_cams; k++) {
+            const size_t v = (size_t)env * n_cams + k;
+            tc_camera_pose(cam + v * TC_CAM_N + TC_CAM_E, s.x, s.y, c, sn, pose + v * 12);
+        }
         double *r = info_f64 + (size_t)env * (4 + C);
         r[0] = info.cte; r[1] = info.heading; r[2] = info.velocity;
         if (mode == 0) r[3] = info.reward;
         for (int c = 0; c < C; c++) { r[4 + c] = dist[c]; nearest[(size_t)env * C + c] = near[c]; }
         if (mode == 0) { terminated[env] = info.terminated; truncated[env] = trunc; }
     }
+}
+HT_API void ht_track(const HtMap *m, int n, int mode, int wrapped, double *sf, int32_t *si, const double *car, const double *cam,
+                     double *pose, const float *act_cc, const int32_t *act_man, const uint8_t *mask, const int32_t *spawn,
+                     double *info_f64, int32_t *nearest, uint8_t *terminated, uint8_t *truncated) {
+    ht_track_rig(m, n, 1, mode, wrapped, sf, si, car, cam, pose, act_cc, act_man, mask, spawn, info_f64, nearest, terminated, truncated, nullptr);
 }
 
 // mirrors tc_project_kernel for one (env, class)

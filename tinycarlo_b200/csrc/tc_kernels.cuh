@@ -63,17 +63,19 @@ struct TcTrackArgs {
     const unsigned char *blob; // packed map tables (global)
     TcBlobLayout layout;
     int n_envs;
+    int n_cams;   // M cameras per env: view v = env * M + m
     int mode;     // 0 = step, 1 = reset
     int wrapped;
     double *sf;
     int32_t *si;
     const double *car;   // [N, TC_CP_N]
-    const double *cam;   // [N, TC_CAM_N]
-    double *pose;        // [N, 12] out
+    const double *cam;   // [N*M, TC_CAM_N]
+    double *pose;        // [N*M, 12] out
     const float *act_cc; // [N,2]
     const double *act_cc64; // [N,2] optional float64 actions (single-env drop-in: Python-float actions keep full precision)
     const int32_t *act_man;
     const uint8_t *mask;        // reset: envs to reset (NULL = all)
+    uint8_t *view_mask;         // reset, optional [N*M] out: mask[env] for each of the env's views (the render kernels index masks by view)
     const int32_t *spawn_nodes; // reset
     // next-step autoreset (gymnasium AutoresetMode.NEXT_STEP): an env whose previous step ended is reset by this step
     uint8_t *done;              // [N] in/out, NULL = autoreset off
@@ -99,8 +101,14 @@ __device__ __forceinline__ void tc_track_store(const TcTrackArgs &a, const TcTra
     if (a.mode == 0 && a.done) a.done[env] = (info.terminated || truncated) ? 1 : 0;
     if (a.mode == 0 && a.was_reset) a.was_reset[env] = auto_reset ? 1 : 0;
     tc_store_state(sf, si, s);
-    // pose for the camera pass: front-axle update already evaluated cos/sin(rot); recomputing keeps the code simple
-    tc_camera_pose(a.cam + (size_t)env * TC_CAM_N + TC_CAM_E, s.x, s.y, cos(s.rot), sin(s.rot), a.pose + (size_t)env * 12);
+    // poses of the env's M views for the camera pass: front-axle update already evaluated cos/sin(rot); recomputing keeps the code simple
+    {
+        const double c = cos(s.rot), sn = sin(s.rot);
+        for (int m = 0; m < a.n_cams; m++) {
+            const size_t v = (size_t)env * a.n_cams + m;
+            tc_camera_pose(a.cam + v * TC_CAM_N + TC_CAM_E, s.x, s.y, c, sn, a.pose + v * 12);
+        }
+    }
     const TcOutputs &o = a.out;
     if (o.cte) o.cte[env] = (float)info.cte;
     if (o.heading_error) o.heading_error[env] = (float)info.heading;
@@ -131,6 +139,12 @@ __device__ __forceinline__ void tc_track_store(const TcTrackArgs &a, const TcTra
         if (o.terminated) o.terminated[env] = info.terminated ? 1 : 0;
         if (o.truncated) o.truncated[env] = truncated ? 1 : 0;
     }
+}
+
+// Reset mode with a camera rig: the caller's mask value of the env for each of its views (a.view_mask is set only together with
+// a.mask). Written before the reset can return early, so that a selected env whose reset fails is rendered at its old pose.
+__device__ __forceinline__ void tc_store_view_mask(const TcTrackArgs &a, int env) {
+    for (int m = 0; m < a.n_cams; m++) a.view_mask[(size_t)env * a.n_cams + m] = a.mask[env];
 }
 
 // G lanes per env (a power of two <= 32): the scalar part of a step is computed redundantly by the G lanes, the scans are spread
@@ -175,6 +189,7 @@ __global__ void __launch_bounds__(TC_TRACK_THREADS, 3) tc_track_kernel(const TcT
     }
     if (auto_reset) {
     } else if (a.mode == 1) {
+        if (a.view_mask && g.lane == 0) tc_store_view_mask(a, env);
         if (a.mask && !a.mask[env]) return;
         tc_load_state(sf, si, s);
         int node = -1;
@@ -247,6 +262,7 @@ __global__ void __launch_bounds__(TC_TRACK1_THREADS) tc_track_thread_kernel(cons
     }
     if (auto_reset) {
     } else if (a.mode == 1) {
+        if (a.view_mask && in_range) tc_store_view_mask(a, env);
         if (a.mask && !a.mask[env]) live = false;
         else {
             int node = -1;
@@ -1801,25 +1817,26 @@ __host__ __device__ inline void tc_philox4x32_10(uint32_t c0, uint32_t c1, uint3
 }
 
 struct TcNoiseArgs {
-    int n_envs, n_classes, H, W;
+    int n_envs, n_cams, n_classes, H, W;
     int n_blobs, max_radius;
     uint32_t seed_lo, seed_hi, step, env_offset;
-    const uint8_t *mask; // optional
-    uint8_t *obs;        // [N,C,H,W] u8
+    const uint8_t *mask; // optional, per env
+    uint8_t *obs;        // [N*M,C,H,W] u8
 };
 
+// a block per view v = env * M + m
 __global__ void __launch_bounds__(256) tc_noise_blobs_kernel(const TcNoiseArgs a) {
     __shared__ int hw[1024]; // half width of the filled midpoint circle per |row offset| (radius < 1024)
     __shared__ int bx, by, brad, bcopy, bsrc;
-    const int env = blockIdx.x, tid = threadIdx.x;
+    const int env = blockIdx.x / a.n_cams, cam = blockIdx.x % a.n_cams, tid = threadIdx.x;
     if (a.mask && !a.mask[env]) return;
     const size_t plane = (size_t)a.H * a.W;
-    uint8_t *base = a.obs + (size_t)env * a.n_classes * plane;
+    uint8_t *base = a.obs + (size_t)blockIdx.x * a.n_classes * plane;
     for (int c = 0; c < a.n_classes; c++)
         for (int k = 0; k < a.n_blobs; k++) {
             if (tid == 0) {
                 uint32_t r[4];
-                tc_philox4x32_10((uint32_t)env + a.env_offset, a.step, (uint32_t)(c * a.n_blobs + k), 0u, a.seed_lo, a.seed_hi, r);
+                tc_philox4x32_10((uint32_t)env + a.env_offset, a.step, (uint32_t)(c * a.n_blobs + k), (uint32_t)cam, a.seed_lo, a.seed_hi, r);
                 bx = (int)(r[0] % (uint32_t)a.W);
                 by = (int)(r[1] % (uint32_t)a.H);
                 brad = a.max_radius > 1 ? 1 + (int)(r[2] % (uint32_t)(a.max_radius - 1)) : 1;   // randint(1, max_radius)

@@ -71,11 +71,13 @@ class _CarFacade:
 
 
 class _CameraFacade:
-    """tinycarlo.camera.Camera's mutable parameters; update_params() re-stages E and K (camera.py:48-50)."""
+    """tinycarlo.camera.Camera's mutable parameters; update_params() re-stages E and K (camera.py:48-50). With a camera rig
+    (the config's `cameras` list) there is one facade per camera, `index` m."""
 
-    def __init__(self, env: "TinyCarloEnv"):
+    def __init__(self, env: "TinyCarloEnv", index: int = 0):
         self._env = env
-        cc = env._vec.cam_cfg
+        self.index = index
+        cc = env._vec.cam_cfgs[index]
         self.resolution = list(cc["resolution"])
         self.position = list(cc["position"])
         self.orientation = list(cc["orientation"])
@@ -83,26 +85,32 @@ class _CameraFacade:
         self.max_range = cc["max_range"]
         self.line_thickness = cc["line_thickness"]
 
+    def _view(self, t):
+        """this camera's frame of env 0 in a tensor of the vec env's layout"""
+        return t[0] if self._env._vec.rig is None else t[0, self.index]
+
     def update_params(self):
-        self._env._vec.set_camera_params(position=np.asarray(self.position, np.float64), orientation=np.asarray(self.orientation, np.float64),
-                                         fov=float(self.fov), max_range=float(self.max_range), line_thickness=int(self.line_thickness))
+        v = self._env._vec
+        v.set_camera_params(position=np.asarray(self.position, np.float64), orientation=np.asarray(self.orientation, np.float64),
+                            fov=float(self.fov), max_range=float(self.max_range), line_thickness=int(self.line_thickness),
+                            camera=None if v.rig is None else self.index)
 
     @property
     def E(self):
-        return self._env._vec._cam_rows[0, :12].reshape(3, 4).copy()
+        return self._env._vec._cam_rows[self.index, :12].reshape(3, 4).copy()
 
     @property
     def K(self):
-        r = self._env._vec._cam_rows[0]
+        r = self._env._vec._cam_rows[self.index]
         return np.array([[r[12], 0, r[14]], [0, r[13], r[15]], [0, 0, 1]])
 
     def get_last_frame_rgb(self):
-        return self._env._vec.render_rgb()[0].cpu().numpy()
+        return self._view(self._env._vec.render_rgb()).cpu().numpy()
 
     def get_last_frame_classes(self):
         if self._env.observation_space_format == "rgb":
             return None
-        return self._env._vec.obs[0].cpu().numpy().copy()
+        return self._view(self._env._vec.obs).cpu().numpy().copy()
 
 
 class TinyCarloEnv(gc.Env):
@@ -116,7 +124,9 @@ class TinyCarloEnv(gc.Env):
         self.observation_space_format: str = v.observation_space_format
         self.map = v.map
         self.car = _CarFacade(self)
-        self.camera = _CameraFacade(self)
+        # camera rig: one facade per camera; `camera` is camera 0, the reference's one camera
+        self.cameras = [_CameraFacade(self, m) for m in range(v.n_cameras)]
+        self.camera = self.cameras[0]
         self._wrapped = False
         self._overview = None
         self._windows = None
@@ -202,7 +212,8 @@ class TinyCarloEnv(gc.Env):
         return self._overview.render([float(sf[0]), float(sf[1])], float(sf[2]), float(sf[3]), self.car.wheelbase, self.car.track_width, path)
 
     def render(self) -> Optional[np.ndarray]:
-        """env.py:149-174: rgb_array -> the RGB camera frame (whatever the observation format); human -> two OpenCV windows"""
+        """env.py:149-174: rgb_array -> the RGB camera frame (whatever the observation format; camera 0 of a rig); human -> two
+        OpenCV windows"""
         if self.render_mode == "rgb_array":
             return self.camera.get_last_frame_rgb()
         if self.render_mode == "human":

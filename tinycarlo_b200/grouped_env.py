@@ -93,8 +93,9 @@ class TinyCarloGroupedVecEnv:
         outs = self._fan_out(lambda e, sl: e.reset_done())
         return [o[0] for o in outs], self._cat_info([o[1] for o in outs])
 
-    def set_camera_params(self, env_ids=None, **kw):
-        """per-env camera parameters by GLOBAL env index (arrays cover all envs when env_ids is None)"""
+    def set_camera_params(self, env_ids=None, camera=None, **kw):
+        """per-env camera parameters by GLOBAL env index (arrays cover all envs when env_ids is None); camera: the rig's
+        camera index or indices, as TinyCarloVecEnv.set_camera_params (the config's `cameras` list applies to every group)"""
         import numpy as np
         ids = np.arange(self.num_envs) if env_ids is None else np.asarray(env_ids).reshape(-1)
         for e, (a, b) in zip(self.envs, zip(self.offsets[:-1], self.offsets[1:])):
@@ -107,7 +108,7 @@ class TinyCarloGroupedVecEnv:
                     continue
                 v = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
                 sub[k] = v[sel] if v.ndim >= 1 and len(v) == len(ids) else v
-            e.set_camera_params(env_ids=ids[sel] - a, **sub)
+            e.set_camera_params(env_ids=ids[sel] - a, camera=camera, **sub)
 
     def set_car_params(self, **kw):
         import numpy as np

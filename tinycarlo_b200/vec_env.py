@@ -17,8 +17,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .camera_params import camera_row
-from .config import LINE_THICKNESS_MAX, bev_params, camera_params, car_param_row, load_config, resolve_map_path, sim_params
+from .camera_params import camera_row, view_rows
+from .config import LINE_THICKNESS_MAX, bev_params, camera_params, camera_rig, car_param_row, load_config, resolve_map_path, sim_params
 from .maptables import MapTables
 from .spawn import spawn_stream_states
 
@@ -48,6 +48,11 @@ class TinyCarloVecEnv:
         self.map = MapTables(resolve_map_path(self.config["map"], self.config_path), self.config["map"]["pixel_per_meter"],
                              self.config["map"].get("spawn_points", None))
         self.cam_cfg = camera_params(self.config["camera"])
+        # camera rig (the config's optional `cameras` list, tc_create_rig): M cameras per car, view v = env * M + m, and
+        # observations with an M axis [N, M, ...]; None: the reference's one camera, no extra axis
+        self.rig = camera_rig(self.config)
+        self.cam_cfgs = self.rig or [self.cam_cfg]
+        self.n_cameras = len(self.cam_cfgs)
         self.num_envs = int(num_envs)
         self.device = torch.device(device if not isinstance(device, int) else f"cuda:{device}")
         if self.device.index is None:
@@ -69,6 +74,8 @@ class TinyCarloVecEnv:
         # "classes_bf16": bfloat16 [N,C,H,W] with 0.0 / 1.0
         self.obs_shape = {_lib.TC_OBS_CLASSES: (Cn, self.H, self.W), _lib.TC_OBS_RGB: (self.H, self.W, 3),
                           _lib.TC_OBS_CLASSES_BITS: (Cn, (self.H * self.W + 31) // 32), _lib.TC_OBS_CLASSES_BF16: (Cn, self.H, self.W)}[fmt]
+        self._rig_axis = () if self.rig is None else (self.n_cameras,)
+        self.obs_shape = self._rig_axis + self.obs_shape
         self.obs_dtype = {_lib.TC_OBS_CLASSES_BITS: torch.int32, _lib.TC_OBS_CLASSES_BF16: torch.bfloat16}.get(fmt, torch.uint8)
 
         # ---- library handle (map tables go to the device once)
@@ -81,7 +88,7 @@ class TinyCarloVecEnv:
         sim = _lib.TcSimDesc(self.H, self.W, fmt)
         self._L = _lib.lib()
         h = C.c_void_p()
-        _lib.check(self._L.tc_create(C.byref(desc), C.byref(sim), N, self.device.index, C.byref(h)), "tc_create")
+        _lib.check(self._L.tc_create_rig(C.byref(desc), C.byref(sim), N, self.n_cameras, self.device.index, C.byref(h)), "tc_create_rig")
         self._h = h
 
         # ---- outputs (allocated once; step()/reset() return views)
@@ -96,9 +103,10 @@ class TinyCarloVecEnv:
                         "terminated": torch.zeros(N, dtype=torch.uint8, device=dev),
                         "truncated": torch.zeros(N, dtype=torch.uint8, device=dev),
                         "info_f64": torch.zeros((N, 4 + Cn), dtype=torch.float64, device=dev)}
-            if debug_segments:
-                self.out["seg_count"] = torch.zeros((N, Cn), dtype=torch.int32, device=dev)
-                self.out["seg_i32"] = torch.zeros((N, max(int(m.ll_edge_off[-1]), 1), 4), dtype=torch.int32, device=dev)
+            if debug_segments:   # per view
+                V = N * self.n_cameras
+                self.out["seg_count"] = torch.zeros((V, Cn), dtype=torch.int32, device=dev)
+                self.out["seg_i32"] = torch.zeros((V, max(int(m.ll_edge_off[-1]), 1), 4), dtype=torch.int32, device=dev)
             # bird's-eye view (config section `bev`, tc_set_bev): [N,P,H,W] u8 or [N,P,H*W/32] int32, rewritten by every
             # step() / reset() whatever no_observation says; None without the section
             self.bev_cfg = bev_params(self.config, Cn)
@@ -119,9 +127,7 @@ class TinyCarloVecEnv:
 
         # ---- parameters
         self._car_rows = np.tile(np.array(car_param_row(self.config["car"], self.T), np.float64), (N, 1))
-        cc = self.cam_cfg
-        self._cam_rows = np.tile(camera_row(cc["position"], cc["orientation"], cc["fov"], cc["resolution"], cc["max_range"]), (N, 1))
-        self._thickness = np.full(N, int(cc["line_thickness"]), np.int32)
+        self._cam_rows, self._thickness = view_rows(self.cam_cfgs, N)   # one per view, env-major: [N*M, 20], [N*M]
         self._check_car_rows(self._car_rows)
         self._upload_params()
 
@@ -236,46 +242,70 @@ class TinyCarloVecEnv:
             raise ValueError(f"camera.line_thickness must be integers in 1..{LINE_THICKNESS_MAX}, got {v!r}")
         return np.broadcast_to(a, shape).astype(np.int32)
 
-    def set_camera_params(self, position=None, orientation=None, fov=None, max_range=None, line_thickness=None, env_ids=None):
+    def _cameras(self, camera) -> np.ndarray:
+        """the camera indices set_camera_params acts on: None is the one camera of an env without a rig; a rig's caller names
+        them, since neither all cameras (a rear camera would turn forward) nor camera 0 alone is a safe guess"""
+        if camera is None:
+            if self.rig is not None:
+                raise ValueError("set_camera_params: this env has a camera rig; choose the cameras with camera=index or a list of indices")
+            return np.zeros(1, np.int64)
+        cams = np.asarray(camera).reshape(-1)
+        if cams.size == 0 or not np.issubdtype(cams.dtype, np.integer) or ((cams < 0) | (cams >= self.n_cameras)).any():
+            raise ValueError(f"camera must be an index or a list of indices in 0..{self.n_cameras - 1}, got {camera!r}")
+        return cams
+
+    def set_camera_params(self, position=None, orientation=None, fov=None, max_range=None, line_thickness=None, env_ids=None, camera=None):
         """Per-env camera parameters (camera.py:48-50 update_params, vectorised). Arrays are [n,3] / [n] for the envs in
-        env_ids (default: all), or a single value broadcast. E and K are rebuilt on the host with the reference's calls."""
+        env_ids (default: all), or a single value broadcast. E and K are rebuilt on the host with the reference's calls.
+        camera: with a rig, the camera index or list of indices the values apply to (each selected camera gets the same
+        per-env values; required); without a rig, None (or 0) is the one camera."""
         ids = np.arange(self.num_envs) if env_ids is None else np.asarray(env_ids).reshape(-1)
-        n = len(ids)
+        cams = self._cameras(camera)
+        n, M = len(ids), self.n_cameras
         thickness = None if line_thickness is None else self._thickness_rows(line_thickness, (n,))
-        if not hasattr(self, "_cam_src"):
-            cc = self.cam_cfg
-            self._cam_src = {"position": np.tile(np.asarray(cc["position"], np.float64), (self.num_envs, 1)),
-                             "orientation": np.tile(np.asarray(cc["orientation"], np.float64), (self.num_envs, 1)),
-                             "fov": np.full(self.num_envs, float(cc["fov"])), "max_range": np.full(self.num_envs, float(cc["max_range"]))}
+        if not hasattr(self, "_cam_src"):   # per view
+            cfgs, N = self.cam_cfgs, self.num_envs
+            self._cam_src = {"position": np.tile(np.array([c["position"] for c in cfgs], np.float64), (N, 1)),
+                             "orientation": np.tile(np.array([c["orientation"] for c in cfgs], np.float64), (N, 1)),
+                             "fov": np.tile(np.array([float(c["fov"]) for c in cfgs]), N),
+                             "max_range": np.tile(np.array([float(c["max_range"]) for c in cfgs]), N)}
 
         def bc(v, shape):
             v = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v, np.float64)
             return np.broadcast_to(v, shape)
-        if position is not None:
-            self._cam_src["position"][ids] = bc(position, (n, 3))
-        if orientation is not None:
-            self._cam_src["orientation"][ids] = bc(orientation, (n, 3))
-        if fov is not None:
-            self._cam_src["fov"][ids] = bc(fov, (n,))
-        if max_range is not None:
-            self._cam_src["max_range"][ids] = bc(max_range, (n,))
-        if thickness is not None:
-            self._thickness[ids] = thickness
-        res = [self.H, self.W]
         s = self._cam_src
+        for m in cams:
+            views = ids * M + m
+            if position is not None:
+                s["position"][views] = bc(position, (n, 3))
+            if orientation is not None:
+                s["orientation"][views] = bc(orientation, (n, 3))
+            if fov is not None:
+                s["fov"][views] = bc(fov, (n,))
+            if max_range is not None:
+                s["max_range"][views] = bc(max_range, (n,))
+            if thickness is not None:
+                self._thickness[views] = thickness
+        res = [self.H, self.W]
         cache = {}
-        for i in ids:
-            key = (tuple(s["position"][i]), tuple(s["orientation"][i]), float(s["fov"][i]), float(s["max_range"][i]))
+        for v in (ids[:, None] * M + cams[None, :]).reshape(-1):
+            key = (tuple(s["position"][v]), tuple(s["orientation"][v]), float(s["fov"][v]), float(s["max_range"][v]))
             row = cache.get(key)
             if row is None:
-                row = cache[key] = camera_row(s["position"][i], s["orientation"][i], s["fov"][i], res, s["max_range"][i])
-            self._cam_rows[i] = row
+                row = cache[key] = camera_row(s["position"][v], s["orientation"][v], s["fov"][v], res, s["max_range"][v])
+            self._cam_rows[v] = row
         self._upload_params()
 
     def set_camera_rows(self, cam_rows: np.ndarray, line_thickness=None):
-        """Raw per-env camera rows [N,20] (E 3x4 row-major, fx, fy, cx, cy, max_range, pad) — include/tinycarlo_b200.h TC_CAM_*."""
-        thickness = None if line_thickness is None else self._thickness_rows(line_thickness, (self.num_envs,))
-        self._cam_rows[:] = np.asarray(cam_rows, np.float64).reshape(self.num_envs, _lib.TC_CAM_N)
+        """Raw camera rows, one per view (E 3x4 row-major, fx, fy, cx, cy, max_range, pad) — include/tinycarlo_b200.h TC_CAM_*:
+        [N,20], or with a rig [N,M,20] or [N*M,20] (view v = env * M + m). line_thickness: a value, or one per view ([N*M] or
+        [N,M])."""
+        V = self.num_envs * self.n_cameras
+        thickness = None
+        if line_thickness is not None:
+            th = line_thickness.detach().cpu().numpy() if isinstance(line_thickness, torch.Tensor) else np.asarray(line_thickness)
+            thickness = self._thickness_rows(th.reshape(-1) if th.ndim == 2 else th, (V,))
+        self._cam_rows[:] = np.asarray(cam_rows, np.float64).reshape(V, _lib.TC_CAM_N)
         if thickness is not None:
             self._thickness[:] = thickness
         self._upload_params()
@@ -424,10 +454,11 @@ class TinyCarloVecEnv:
                            "tc_step_host_obs")
 
     def render_rgb(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """RGB camera frames [N,H,W,3] at the current poses (renderer.py:36-44), independent of the obs format."""
+        """RGB camera frames [N,H,W,3] ([N,M,H,W,3] with a rig) at the current poses (renderer.py:36-44), independent of the
+        obs format."""
         with torch.cuda.device(self.device):
             if out is None:
-                out = torch.empty((self.num_envs, self.H, self.W, 3), dtype=torch.uint8, device=self.device)
+                out = torch.empty((self.num_envs,) + self._rig_axis + (self.H, self.W, 3), dtype=torch.uint8, device=self.device)
             _lib.check(self._L.tc_render(self._h, None, _ptr(out), _lib.TC_OBS_RGB, None, None, self._stream()), "tc_render")
         return out
 
@@ -454,7 +485,7 @@ class TinyCarloVecEnv:
         return self.bev
 
     def render_obs(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Re-render self.obs at the current poses (after load_state_dict / set_camera_params)."""
+        """Re-render self.obs (all views) at the current poses (after load_state_dict / set_camera_params); mask is per env."""
         with torch.cuda.device(self.device):
             m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
             _lib.check(self._L.tc_render(self._h, _ptr(m), _ptr(self.obs), self._fmt, _ptr(self.out.get("seg_count")),

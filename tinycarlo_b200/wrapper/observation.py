@@ -3,6 +3,7 @@ erase a class mask or OR in the pixels of a random class — as a device kernel 
 for the single-env drop-in. Same constructor arguments as the reference plus `seed`: the reference draws from numpy's
 unseeded global RNG, so there is no stream to reproduce; here the noise of (env, step, class, blob) is a pure function of
 the seed through Philox4x32-10 (contract in include/tinycarlo_b200.h), reproducible and independent of the GPU sharding.
+With a camera rig every view is noised: camera m draws with counter word 3 = m, so camera 0 gets the rig-less noise.
 Like the reference, constructing it sets `unwrapped.wrapped = True` and it only acts on the "classes" format."""
 import ctypes as C
 
