@@ -174,6 +174,33 @@ def test_headline_kernel_keeps_its_register_budget():
     assert m and int(m.group(1)) <= 64, "block-per-env kernel missing or over its register budget"
 
 
+# (kernel, mangled name, registers at most, stack bytes at most) on sm_100a. The registers decide the blocks per SM, and the
+# packed kernel's envs per block and chunk count are chosen from its occupancy at run time (tc_install_cull); a spill is a
+# local-memory access that queues behind the observation stores. 76 and 80 registers both allocate 20480 per 256-thread block.
+_RESOURCE_BUDGETS = (
+    [(f"tc_render_env_kernel<256,{f}>", f"_Z20tc_render_env_kernelILi256ELi{f}EEv15TcRenderEnvArgs", 64, 0) for f in range(4)]
+    + [(f"tc_render_envs_kernel<256,{f},{e}>", f"_Z21tc_render_envs_kernelILi256ELi{f}ELi{e}EEv15TcRenderEnvArgs", {2: 76, 4: 80}[e], 0)
+       for f in range(4) for e in (2, 4)]
+    + [("tc_prims_kernel<256,2>", "_Z15tc_prims_kernelILi256ELi2EEv15TcRenderEnvArgs10TcPrimsOut", 76, 0),
+       ("tc_draw_class_kernel<256,2>", "_Z20tc_draw_class_kernelILi256ELi2EEv10TcDrawArgs", 44, 0),
+       ("tc_render_env_banded_kernel<1>", "_Z27tc_render_env_banded_kernelILi1EEv15TcRenderEnvArgs", 64, 8),
+       ("tc_render_env_banded_kernel<2>", "_Z27tc_render_env_banded_kernelILi2EEv15TcRenderEnvArgs", 64, 0)])
+
+
+@pytest.mark.parametrize("name,mangled,max_reg,max_stack", _RESOURCE_BUDGETS, ids=[b[0] for b in _RESOURCE_BUDGETS])
+def test_block_per_env_kernels_keep_their_register_budget(name, mangled, max_reg, max_stack):
+    """Every instance of the block-per-env render kernels and the per-class draw kernel of the two-kernel path stays within
+    its registers and stack (DESIGN.md section 4). Checked on the built library (no GPU needed)."""
+    import shutil
+    import subprocess
+    if shutil.which("cuobjdump") is None or not os.path.exists(_lib.LIB_PATH):
+        pytest.skip("cuobjdump or the built library is not available")
+    out = subprocess.run(["cuobjdump", "-res-usage", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    m = re.search(rf"Function {mangled}:\s*\n\s*REG:(\d+) STACK:(\d+)", out)
+    assert m, f"{name} not found in the library"
+    assert int(m.group(1)) <= max_reg and int(m.group(2)) <= max_stack, f"{name}: {m.group(0)}"
+
+
 @pytest.mark.parametrize("config", [3, 1, 4, 5])
 def test_bench_reference_arm_prints_the_contract_line(config):
     """bench.py --impl reference (the CPU arm: the unmodified reference from baseline/_ref, one process per host core, plus

@@ -44,8 +44,11 @@ struct TcCullSet {
     unsigned char *d_blob = nullptr;
     TcCullGrid grid{};
     int np = 0, max_bytes = 0, cells = 0, max_nodes = 0;
-    size_t env_smem = 0, envb_smem = 0, envs_smem = 0;
-    int pack = 0, chunks = 1, blocks = 0;
+    size_t env_smem = 0;     // tc_render_env_kernel (small frames)
+    size_t envb_smem = 0;    // tc_render_env_banded_kernel (large frames, RGB / 1 bit per pixel); 0: not available
+    size_t envs_smem = 0;
+    int pack = 0, chunks = 1;   // pack > 0: tc_render_envs_kernel with that many envs per block
+    int blocks = 0;             // resident blocks per SM of the packed kernel as chosen (diagnostics)
     double radius = -1.0, mean_nodes = 0.0;
 };
 
@@ -94,25 +97,15 @@ struct TcHandle {
     TcNear near_h;                 // geometry (the tables themselves live on the device)
     int32_t *d_near_off = nullptr;
     uint16_t *d_near_edge = nullptr;
-    TcCellBlob *d_cell_desc = nullptr;
-    unsigned char *d_cell_blob = nullptr;
-    TcCullGrid cull_grid{};
     std::vector<TcCullSet> cull_sets;   // every set built so far (freed by tc_destroy)
-    double cull_key = -2.0;             // the active one
+    int cull_active = 0;                // cull_sets[cull_active] is the active one (tc_cull_set); tc_create installs the first
     int cull_builds = 0, cull_hits = 0;
     double cull_build_ms_last = 0.0, cull_build_ms_total = 0.0;
-    int env_np = 0, env_max_bytes = 0, env_words = 0;
-    size_t env_smem = 0;     // tc_render_env_kernel (small frames)
+    int env_words = 0;
     // two-kernel path of large bit-packed frames (tc_prims_kernel + tc_draw_class_kernel): buffers allocated at first use
     TcPrimsOut prims{};
-    int env_blocks = 0;      // resident blocks per SM of the packed kernel as chosen (diagnostics)
-    int env_pack = 0, env_chunks = 1;   // > 0: tc_render_envs_kernel with that many envs per block
-    size_t envs_smem = 0;
-    size_t envb_smem = 0;    // tc_render_env_banded_kernel (large frames, RGB / 1 bit per pixel); 0: not available
     int envb_rows = 0, envb_bands = 0, envb_words = 0;
-    double cull_radius = -1.0, cull_mean_nodes = 0.0;
     bool cull_built_once = false;
-    int cull_cells = 0, cull_max_nodes = 0;
     uint8_t *ar_done = nullptr; // autoreset flags: caller-owned device buffer
     uint8_t *ar_was_reset = nullptr; // optional: which envs the last step reset (caller-owned)
     uint64_t *rng = nullptr;    // spawn streams: caller-owned device buffers
@@ -166,20 +159,15 @@ static TcMapDesc tc_host_map(const TcHandle *h) {
     m.ll_nodes = h->m_nodes.data(); m.ll_edges = h->m_edges.data();
     return m;
 }
+// the active visible-set tables and the launch geometry derived from them
+static const TcCullSet &tc_cull_set(const TcHandle *h) { return h->cull_sets[h->cull_active]; }
 // makes the visible-set tables for camera reach `radius` (< 0: culling off) the active ones: from the handle's cache, or built
 // on the host (tc_cull.h, ~50-150 ms for Knuffingen) and copied to the device. Never frees tables a running kernel may read.
-static void tc_activate_cull(TcHandle *h, const TcCullSet &c) {
-    h->d_cell_desc = c.d_desc; h->d_cell_blob = c.d_blob;
-    h->cull_grid = c.grid; h->env_np = c.np; h->env_max_bytes = c.max_bytes; h->env_smem = c.env_smem; h->envb_smem = c.envb_smem;
-    h->cull_radius = c.radius; h->cull_mean_nodes = c.mean_nodes; h->cull_cells = c.cells; h->cull_max_nodes = c.max_nodes;
-    h->env_pack = c.pack; h->env_chunks = c.chunks; h->envs_smem = c.envs_smem; h->env_blocks = c.blocks;
-    h->cull_key = c.key;
-}
 static int tc_install_cull(TcHandle *h, double radius) {
     if (const char *ce = getenv("TC_CULL")) if (atoi(ce) == 0) radius = -1.0;
-    for (const TcCullSet &c : h->cull_sets)
-        if (c.key == radius) {
-            tc_activate_cull(h, c);
+    for (size_t i = 0; i < h->cull_sets.size(); i++)
+        if (h->cull_sets[i].key == radius) {
+            h->cull_active = (int)i;
             h->cull_hits++;
             return TC_OK;
         }
@@ -227,7 +215,7 @@ static int tc_install_cull(TcHandle *h, double radius) {
     c.grid = cull.grid; c.np = (int)np; c.max_bytes = cull.max_bytes; c.env_smem = smem; c.envb_smem = smem_b;
     c.radius = cull.radius; c.mean_nodes = cull.mean_nodes; c.cells = (int)cull.desc.size(); c.max_nodes = cull.max_nodes;
     h->cull_sets.back() = c;
-    tc_activate_cull(h, c);
+    h->cull_active = (int)h->cull_sets.size() - 1;
     h->cull_builds++;
     h->cull_build_ms_last = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     h->cull_build_ms_total += h->cull_build_ms_last;
@@ -465,28 +453,27 @@ int tc_set_camera_params_host(TcHandle *h, const double *dev_cam, const int32_t 
     TC_CUDA(cudaMemcpyAsync(h->d_cam, dev_cam, (size_t)h->n_views * TC_CAM_N * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     TC_CUDA(cudaMemcpyAsync(h->d_thick, dev_thickness, (size_t)h->n_views * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     h->cam_set = true;
-    if (h->fused_all || h->envb_smem > 0 || h->cull_radius >= 0 || !h->cull_sets.empty()) {
-        // the visible-set tables depend on how far the cameras see: from the caller's host copy of the rows, or read back (synchronises)
-        std::vector<double> rows;
-        if (!host_cam) {
-            rows.resize((size_t)h->n_views * TC_CAM_N);
-            TC_CUDA(cudaMemcpyAsync(rows.data(), h->d_cam, rows.size() * sizeof(double), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-            TC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-            host_cam = rows.data();
-        }
-        // the largest reach over all views: tables built for a nearer camera would drop lines a farther one sees
-        double radius = 0.0;
-        for (int i = 0; i < h->n_views && radius >= 0; i++) {
-            double r = tc_cull_radius_of(host_cam + (size_t)i * TC_CAM_N, h->H, h->W);
-            radius = r < 0 ? -1.0 : std::max(radius, r);
-        }
-        // keep the active tables while they cover the cameras and are not more than twice too wide
-        const bool keep = radius >= 0 && h->cull_radius >= radius && h->cull_radius <= 2.0 * radius;
-        if (radius != h->cull_radius && !keep) {
-            const bool first = !h->cull_built_once;
-            TC_TRY(tc_install_cull(h, radius < 0 || first ? radius : tc_cull_ladder(radius)));
-            h->cull_built_once = true;
-        }
+    // the visible-set tables depend on how far the cameras see: from the caller's host copy of the rows, or read back (synchronises)
+    std::vector<double> rows;
+    if (!host_cam) {
+        rows.resize((size_t)h->n_views * TC_CAM_N);
+        TC_CUDA(cudaMemcpyAsync(rows.data(), h->d_cam, rows.size() * sizeof(double), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+        TC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+        host_cam = rows.data();
+    }
+    // the largest reach over all views: tables built for a nearer camera would drop lines a farther one sees
+    double radius = 0.0;
+    for (int i = 0; i < h->n_views && radius >= 0; i++) {
+        double r = tc_cull_radius_of(host_cam + (size_t)i * TC_CAM_N, h->H, h->W);
+        radius = r < 0 ? -1.0 : std::max(radius, r);
+    }
+    // keep the active tables while they cover the cameras and are not more than twice too wide
+    const double active = tc_cull_set(h).radius;
+    const bool keep = radius >= 0 && active >= radius && active <= 2.0 * radius;
+    if (radius != active && !keep) {
+        const bool first = !h->cull_built_once;
+        TC_TRY(tc_install_cull(h, radius < 0 || first ? radius : tc_cull_ladder(radius)));
+        h->cull_built_once = true;
     }
     return TC_OK;
 }
@@ -533,23 +520,25 @@ static TcRenderPath tc_render_path(const TcHandle *h, int obs_format, bool segme
     using P = TcRenderPath;
     const bool bits = obs_format == TC_OBS_CLASSES_BITS;
     if (segments) return P::UNFUSED;
-    if (h->fused_all) return h->env_pack > 0 && !timeline ? P::ENVS : P::ENV;
-    if (h->envb_smem > 0 && bits && (h->H * h->W) % 128 == 0 && (size_t)h->plane_words_full * 4 <= 64 * 1024) return P::PRIMS;
-    if (h->envb_smem > 0 && (bits || obs_format == TC_OBS_RGB)) return P::BANDED;
+    const TcCullSet &cs = tc_cull_set(h);
+    if (h->fused_all) return cs.pack > 0 && !timeline ? P::ENVS : P::ENV;
+    if (cs.envb_smem > 0 && bits && (h->H * h->W) % 128 == 0 && (size_t)h->plane_words_full * 4 <= 64 * 1024) return P::PRIMS;
+    if (cs.envb_smem > 0 && (bits || obs_format == TC_OBS_RGB)) return P::BANDED;
     if (h->fused_ok && obs_format != TC_OBS_RGB) return P::CLASSES;
     return P::UNFUSED;
 }
 
 // arguments of the block-per-env kernels; plane_words: words of the stacked plane of the small-frame kernels, 0 for the others
 static TcRenderEnvArgs tc_render_env_args(const TcHandle *h, const uint8_t *mask, uint8_t *obs, int plane_words) {
+    const TcCullSet &cs = tc_cull_set(h);
     TcRenderEnvArgs ea;
-    ea.cell_desc = h->d_cell_desc; ea.cell_blob = h->d_cell_blob; ea.grid = h->cull_grid; ea.n_envs = h->n_views; ea.n_classes = h->C;
-    ea.np = h->env_np; ea.max_bytes = h->env_max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = plane_words;
+    ea.cell_desc = cs.d_desc; ea.cell_blob = cs.d_blob; ea.grid = cs.grid; ea.n_envs = h->n_views; ea.n_classes = h->C;
+    ea.np = cs.np; ea.max_bytes = cs.max_bytes; ea.H = h->H; ea.W = h->W; ea.plane_words = plane_words;
     ea.pose = h->d_pose; ea.cam = h->d_cam; ea.thickness = h->d_thick; ea.mask = mask; ea.obs = obs;
     memcpy(ea.colors, h->colors, sizeof(ea.colors));
     ea.timeline = nullptr;
     ea.rows_per_band = h->envb_rows; ea.n_bands = h->envb_bands; ea.band_words = h->envb_words;
-    ea.region_bytes = (int)tc_envs_region_bytes((size_t)h->env_np, h->env_max_bytes, plane_words);
+    ea.region_bytes = (int)tc_envs_region_bytes((size_t)cs.np, cs.max_bytes, plane_words);
     ea.prim_chunks = 1;
     return ea;
 }
@@ -559,6 +548,7 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
                             cudaStream_t st, cudaEvent_t after_project = nullptr) {
     using P = TcRenderPath;
     const int N = h->n_views, C = h->C;
+    const TcCullSet &cs = tc_cull_set(h);
     long long *timeline = mask ? nullptr : h->timeline;
     const P path = tc_render_path(h, obs_format, seg_count_out || seg_out, timeline != nullptr);
     if (obs_format == TC_OBS_CLASSES_BITS || obs_format == TC_OBS_CLASSES_BF16) {
@@ -578,9 +568,9 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
     switch (launch) {
     case P::ENVS: {
         TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, h->env_words);
-        ea.prim_chunks = h->env_chunks;
-        const int E = h->env_pack, grid = (N + E - 1) / E;
-        const size_t sm = h->envs_smem;
+        ea.prim_chunks = cs.chunks;
+        const int E = cs.pack, grid = (N + E - 1) / E;
+        const size_t sm = cs.envs_smem;
 #define TC_LAUNCH_ENVS(F)                                                                             \
     do {                                                                                              \
         if (E == 4) tc_render_envs_kernel<256, F, 4><<<grid, 256, sm, st>>>(ea);                      \
@@ -596,7 +586,7 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
     case P::ENV: {
         TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, h->env_words);
         ea.timeline = timeline;
-        const size_t sm = h->env_smem;
+        const size_t sm = cs.env_smem;
         if (obs_format == TC_OBS_RGB) tc_render_env_kernel<256, TC_FMT_RGB><<<N, 256, sm, st>>>(ea);
         else if (obs_format == TC_OBS_CLASSES_BITS) tc_render_env_kernel<256, TC_FMT_BITS><<<N, 256, sm, st>>>(ea);
         else if (obs_format == TC_OBS_CLASSES_BF16) tc_render_env_kernel<256, TC_FMT_BF16><<<N, 256, sm, st>>>(ea);
@@ -607,7 +597,7 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
         // large frames, 1 bit per pixel: geometry + set-up once per env (primitives to L2), then a block per (env, class) draws and stores;
         // envs with more segments than the primitive buffer holds are flagged and rendered by the banded kernel
         TcRenderEnvArgs ea = tc_render_env_args(h, mask, nullptr, 0);
-        const size_t sm1 = tc_envs_smem_bytes(2, (size_t)h->env_np, h->env_max_bytes, 0, 1);
+        const size_t sm1 = tc_envs_smem_bytes(2, (size_t)cs.np, cs.max_bytes, 0, 1);
         tc_prims_kernel<256, 2><<<(N + 1) / 2, 256, sm1, st>>>(ea, h->prims);
         h->launches++;
         TC_CUDA(cudaGetLastError());
@@ -617,14 +607,14 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
         h->launches++;
         TC_CUDA(cudaGetLastError());
         ea.mask = h->prims.overflow; ea.obs = obs;   // (the flag is only set for envs the caller's mask selected)
-        tc_render_env_banded_kernel<TC_FMT_BITS><<<std::min(N, 2 * h->n_sms), 256, h->envb_smem, st>>>(ea);   // few blocks scan the (sparse) flags
+        tc_render_env_banded_kernel<TC_FMT_BITS><<<std::min(N, 2 * h->n_sms), 256, cs.envb_smem, st>>>(ea);   // few blocks scan the (sparse) flags
         break;
     }
     case P::BANDED: {
         // large frames whose stores are not the bound: a block per env, bands walked inside the block
         const TcRenderEnvArgs ea = tc_render_env_args(h, mask, obs, 0);
-        if (obs_format == TC_OBS_RGB) tc_render_env_banded_kernel<TC_FMT_RGB><<<N, 256, h->envb_smem, st>>>(ea);
-        else tc_render_env_banded_kernel<TC_FMT_BITS><<<N, 256, h->envb_smem, st>>>(ea);
+        if (obs_format == TC_OBS_RGB) tc_render_env_banded_kernel<TC_FMT_RGB><<<N, 256, cs.envb_smem, st>>>(ea);
+        else tc_render_env_banded_kernel<TC_FMT_BITS><<<N, 256, cs.envb_smem, st>>>(ea);
         break;
     }
     case P::CLASSES: {
@@ -879,7 +869,8 @@ int tc_debug_set_timeline(TcHandle *h, long long *dev_timeline) {
 
 int tc_debug_cull_info(TcHandle *h, double *out4) {
     if (!h || !out4) return tc_fail(TC_ERR_INVALID, "tc_debug_cull_info: null argument");
-    out4[0] = (h->fused_all || h->envb_smem > 0) ? h->cull_radius : -2.0; out4[1] = h->cull_cells; out4[2] = h->cull_mean_nodes; out4[3] = h->cull_max_nodes;
+    const TcCullSet &cs = tc_cull_set(h);
+    out4[0] = (h->fused_all || cs.envb_smem > 0) ? cs.radius : -2.0; out4[1] = cs.cells; out4[2] = cs.mean_nodes; out4[3] = cs.max_nodes;
     return TC_OK;
 }
 
@@ -891,9 +882,10 @@ int tc_debug_cull_stats(TcHandle *h, double *out4) {
 
 int tc_debug_render_info(TcHandle *h, int32_t *out8) {
     if (!h || !out8) return tc_fail(TC_ERR_INVALID, "tc_debug_render_info: null argument");
-    out8[0] = h->fused_all; out8[1] = h->fused_all ? h->env_pack : 0; out8[2] = h->env_chunks;
-    out8[3] = (int32_t)(h->fused_all ? (h->env_pack ? h->envs_smem : h->env_smem) : h->render_smem);
-    out8[4] = h->track_per_thread + 16 * h->env_blocks + 1024 * h->track_group; out8[5] = (int32_t)h->envb_smem; out8[6] = h->env_np; out8[7] = h->env_max_bytes;
+    const TcCullSet &cs = tc_cull_set(h);
+    out8[0] = h->fused_all; out8[1] = h->fused_all ? cs.pack : 0; out8[2] = cs.chunks;
+    out8[3] = (int32_t)(h->fused_all ? (cs.pack ? cs.envs_smem : cs.env_smem) : h->render_smem);
+    out8[4] = h->track_per_thread + 16 * cs.blocks + 1024 * h->track_group; out8[5] = (int32_t)cs.envb_smem; out8[6] = cs.np; out8[7] = cs.max_bytes;
     return TC_OK;
 }
 

@@ -791,6 +791,28 @@ __host__ __device__ inline size_t tc_render_smem_bytes(int max_nodes, int max_ed
            (size_t)TC_SETUP_CHUNK * TC_MAX_PRIMS_PER_SEG * sizeof(TcPrim) + (size_t)((max_edges + 15) & ~15);
 }
 
+// per-block phase clocks for tools/timeline.py (tc_render_classes_kernel, tc_render_env_kernel): compiled in only with
+// -DTC_TIMELINE (the seven 64-bit counters cost registers and spills in the production build). TC_TL runs a statement on
+// thread 0 when a timeline is asked for; TC_TL_RECORD writes the block's record [smid, t0, t1, t2, t3, t_end, segments,
+// zeroing, set-up, draw] into row blockIdx.x.
+#ifdef TC_TIMELINE
+#define TC_TL(stmt) do { if (a.timeline && tid == 0) { stmt; } } while (0)
+#define TC_TL_DECL long long tl0 = 0, tl1 = 0, tl2 = 0, tl3 = 0, tl_setup = 0, tl_draw = 0, tl_z = 0, tc0 = 0
+#define TC_TL_RECORD(t1, cnt) TC_TL(tc_timeline_record(a.timeline, tl0, t1, tl2, tl3, cnt, tl_z, tl_setup, tl_draw))
+__device__ __forceinline__ void tc_timeline_record(long long *timeline, long long tl0, long long tl1, long long tl2, long long tl3, int cnt,
+                                                   long long tl_z, long long tl_setup, long long tl_draw) {
+    unsigned smid;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+    long long *r = timeline + (size_t)blockIdx.x * 10;
+    r[0] = smid; r[1] = tl0; r[2] = tl1; r[3] = tl2; r[4] = tl3; r[5] = clock64();
+    r[6] = cnt; r[7] = tl_z ? tl_z - tl2 : 0; r[8] = tl_setup; r[9] = tl_draw;
+}
+#else
+#define TC_TL(stmt) do { } while (0)
+#define TC_TL_DECL do { } while (0)
+#define TC_TL_RECORD(t1, cnt) do { } while (0)
+#endif
+
 // NT = 256 threads per block, 4 blocks/SM: the stores dominate
 template <int NT, int FMT>
 __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const TcRenderArgs a) {
@@ -801,14 +823,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
     const int env = blockIdx.x / a.n_classes, c = blockIdx.x % a.n_classes;
     if (a.mask && !a.mask[env]) return;
     const int tid = threadIdx.x;
-// per-block phase clocks for tools/timeline.py: compiled in only with -DTC_TIMELINE (the seven 64-bit counters cost
-// registers and spills in the production build)
-#ifdef TC_TIMELINE
-#define TC_TL(stmt) do { if (a.timeline && tid == 0) { stmt; } } while (0)
-    long long tl0 = 0, tl1 = 0, tl2 = 0, tl3 = 0, tl_setup = 0, tl_draw = 0, tl_z = 0, tc0 = 0;
-#else
-#define TC_TL(stmt) do { } while (0)
-#endif
+    TC_TL_DECL;
     TC_TL(tl0 = clock64());
     const TcClassBlob cb = a.cblob_desc[c];
     unsigned char *tab_smem = smem_raw + tc_render_scratch_bytes(a.max_nodes);
@@ -918,16 +933,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
     } else if (FMT == TC_FMT_BF16)
         tc_store_bf16<NT>((uint16_t *)a.obs + blockIdx.x * hw, (uint32_t)hw, plane, cnt > 0);
     else tc_store_plane<NT>(a.obs + blockIdx.x * hw, hw, plane, cnt > 0);
-#ifdef TC_TIMELINE
-    if (a.timeline && tid == 0) {
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        long long *r = a.timeline + (size_t)blockIdx.x * 10;
-        r[0] = smid; r[1] = tl0; r[2] = tl1; r[3] = tl2; r[4] = tl3; r[5] = clock64();
-        r[6] = cnt; r[7] = tl_z ? tl_z - tl2 : 0; r[8] = tl_setup; r[9] = tl_draw;
-    }
-#endif
-#undef TC_TL
+    TC_TL_RECORD(tl1, cnt);
 }
 
 // ------------------------------------------------------------------------------------------------ fused, block per env
@@ -1059,9 +1065,191 @@ __device__ __forceinline__ void tc_env_camera_pass(unsigned char *smem_raw, size
     __syncthreads();   // projected coordinates, flags and tables are dead: plane and primitive slots take their place
 }
 
+// The other phases of the block-per-env kernels, each written once. Where the kernels differ, a template flag or a
+// compile-time constant argument selects the difference, so each kernel compiles to what its own copy did.
+
+// Stages view `env` in a block of its own (tc_render_env_kernel, tc_render_env_banded_kernel): thread 0 finds the camera's
+// ground cell, whose tables come in with one TMA bulk copy on `bar` (initialised here when init_bar: the banded kernel
+// initialises it once for all the views it walks), resets the segment count and publishes the cell's descriptor; warp 1 loads
+// the pose and the intrinsics, and in RGB warp 2 the class colours. Ends with a block barrier.
+template <bool RGB>
+__device__ __forceinline__ void tc_stage_env(const TcRenderEnvArgs &a, int env, unsigned char *tab_smem, uint64_t *bar, bool init_bar, int *seg_cnt,
+                                             TcCellBlob *s_desc, double *s_pose, double *s_cam, uint32_t *s_color24) {
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        // which part of the map can this camera see: its ground cell selects the tables (one TMA bulk copy)
+        const TcCellBlob d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
+        *seg_cnt = 0;
+        if (init_bar) {
+            tc_mbar_init(bar, 1);
+            tc_fence_mbar_init();
+        }
+        if (d.bytes > 0) {
+            tc_mbar_expect_tx(bar, (uint32_t)d.bytes);
+            tc_bulk_g2s(tab_smem, a.cell_blob + d.offset, (uint32_t)d.bytes, bar);
+        }
+        *s_desc = d;
+    }
+    if (RGB && tid >= 64 && tid < 64 + TC_MAX_CLASSES) s_color24[tid - 64] = tc_color24_of(a.colors, tid - 64);
+    if (tid >= 32 && tid < 44) s_pose[tid - 32] = a.pose[(size_t)env * 12 + tid - 32];
+    else if (tid >= 44 && tid < 44 + (TC_CAM_MAX_RANGE - TC_CAM_FX + 1)) s_cam[TC_CAM_FX + tid - 44] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + tid - 44];
+    __syncthreads();      // barrier init, descriptor, pose and intrinsics visible to all threads
+}
+
+// Stages the E view slots of a packed block (tc_render_envs_kernel, tc_prims_kernel; views blockIdx.x * E + e, each with its
+// region of a.region_bytes) and runs their camera passes side by side: thread -> (slot j, index of its NT/E threads). A slot past
+// the last view or masked out is inactive: the empty cell, thickness 1. `bar` takes one arrival per slot, with its tables' bytes.
+template <int NT, int E, bool RGB>
+__device__ __forceinline__ void tc_stage_envs(const TcRenderEnvArgs &a, unsigned char *smem_raw, uint64_t *bar, int *seg_cnt, int *s_thick, int *s_active,
+                                              TcCellBlob *s_desc, double (*s_pose)[12], double (*s_cam)[TC_CAM_N], uint32_t *s_color24) {
+    constexpr int TPE = NT / E;
+    if (threadIdx.x == 0) {
+        tc_mbar_init(bar, E);
+        tc_fence_mbar_init();
+    }
+    __syncwarp();
+    if (threadIdx.x < E) {
+        // which part of the map can this env's camera see: its ground cell selects the tables (one TMA bulk copy per env)
+        const int e = threadIdx.x, env = blockIdx.x * E + e;
+        const bool act = env < a.n_envs && !(a.mask && !a.mask[env]);
+        TcCellBlob d;
+        if (act) d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
+        else { d.n_nodes = 0; d.n_edges = 0; d.bytes = 0; d.offset = 0; }
+        s_active[e] = act; seg_cnt[e] = 0; s_thick[e] = act ? a.thickness[env] : 1;
+        s_desc[e] = d;
+        // one arrival per env slot, with its bytes
+        if (d.bytes > 0) {
+            tc_mbar_expect_tx(bar, (uint32_t)d.bytes);
+            tc_bulk_g2s(smem_raw + (size_t)e * a.region_bytes + tc_env_off_tables((size_t)a.np), a.cell_blob + d.offset, (uint32_t)d.bytes, bar);
+        } else tc_mbar_arrive(bar);
+    }
+    if (RGB && threadIdx.x >= 64 && threadIdx.x < 64 + TC_MAX_CLASSES) s_color24[threadIdx.x - 64] = tc_color24_of(a.colors, threadIdx.x - 64);
+    if (threadIdx.x >= 32 && threadIdx.x < 32 + E * 17) {
+        const int k = threadIdx.x - 32, e = k / 17, i = k % 17, env = blockIdx.x * E + e;
+        if (env < a.n_envs) {
+            if (i < 12) s_pose[e][i] = a.pose[(size_t)env * 12 + i];
+            else s_cam[e][TC_CAM_FX + i - 12] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + i - 12];
+        }
+    }
+    __syncthreads();
+    // ---- camera pass (camera.py:52-110) of the E envs side by side
+    const int j = threadIdx.x / TPE;
+    unsigned char *region = smem_raw + (size_t)j * a.region_bytes;
+    tc_env_camera_pass<TPE, true>(region, (size_t)a.np, region + tc_env_off_tables((size_t)a.np), s_desc[j], bar, s_pose[j], s_cam[j], a.H, a.W,
+                                  &seg_cnt[j], (int)threadIdx.x - j * TPE);
+}
+
+// thread 0: where each slot's segments start in the block's concatenated list, and (s_pref[E]) how many there are
+template <int E>
+__device__ __forceinline__ void tc_seg_prefix(const int *seg_cnt, int *s_pref) {
+    if (threadIdx.x == 0) {
+        int acc = 0;
+        for (int e = 0; e < E; e++) { s_pref[e] = acc; acc += seg_cnt[e]; }
+        s_pref[E] = acc;
+    }
+}
+
+// marks the primitive slots of a set-up round's nseg segments empty (the set-up fills only the slots a segment needs)
+template <int NT>
+__device__ __forceinline__ void tc_clear_prim_slots(int32_t *pw, int nseg) {
+    for (int i = threadIdx.x; i < nseg * TC_MAX_PRIMS_PER_SEG; i += NT)
+        pw[(i / TC_MAX_PRIMS_PER_SEG) * TC_ENV_SEG_WORDS + (i % TC_MAX_PRIMS_PER_SEG) * 8] = TC_PRIM_NONE;
+}
+
+// Gathers segments base .. base + nseg - 1 of a packed block's concatenated list for one set-up round: thread i copies segment i
+// of the round next to its tag (env slot << 8 | class), and with WITH_GPOS its position in its env's class-sorted list (the
+// class's offset s_clsoff plus the segment's rank within its class, rank[e] in slot e's region). Thread 0 resets the task queue.
+template <int E, bool WITH_GPOS>
+__device__ __forceinline__ void tc_gather_round(const TcRenderEnvArgs &a, const unsigned char *smem_raw, int base, int nseg, const int *s_pref,
+                                                const TcCellBlob *s_desc, int4 *s_seg, uint16_t *s_tag, int *s_gpos,
+                                                const int (*s_clsoff)[TC_MAX_CLASSES], int *s_task, int *s_nseg, int *s_ntask) {
+    if ((int)threadIdx.x < nseg) {   // segment tid of the round: find its env slot, copy it next to its tag
+        const int sidx = base + threadIdx.x;
+        int e = 0;
+#pragma unroll
+        for (int k = 1; k < E; k++) e += sidx >= s_pref[k];
+        const int i = sidx - s_pref[e];
+        const unsigned char *region = smem_raw + (size_t)e * a.region_bytes;
+        const int4 *segs = (const int4 *)region;
+        const uint8_t cls = ((const uint8_t *)(segs + s_desc[e].n_edges))[i];
+        s_seg[threadIdx.x] = segs[i];
+        s_tag[threadIdx.x] = (uint16_t)((e << 8) | cls);
+        if (WITH_GPOS) s_gpos[threadIdx.x] = s_clsoff[e][cls] + ((const uint16_t *)(region + (size_t)a.np * 24))[i];
+    }
+    if (threadIdx.x == 0) {
+        *s_task = 0; *s_nseg = nseg;
+        *s_ntask = ((nseg + TC_ENV_CHUNK - 1) / TC_ENV_CHUNK) * TC_N_ROLES;
+    }
+}
+
+// Set-up of a packed block's round: (role, chunk) tasks from a queue, lane = segment of the chunk; spans (role 0) are handed out
+// first. Each segment's primitives go to its TC_ENV_SEG_WORDS words at pw.
+// (Tried in round 2 and rejected: draw tasks in the same queue, each waiting only for the set-up task that fills its slot, so
+// that the short roles' primitives are drawn while the spans are still being set up - no barrier between the phases, but
+// 9-10 % slower on every small-frame configuration: the ticket order serialises what the barrier let all warps share.)
+__device__ __forceinline__ void tc_setup_queue(const TcRenderEnvArgs &a, int *s_task, const int *s_ntask, const int *s_nseg, const int4 *s_seg,
+                                               const uint16_t *s_tag, const int *s_thick, int32_t *pw) {
+    while (true) {
+        int k = 0;
+        if ((threadIdx.x & 31) == 0) k = atomicAdd(s_task, 1);
+        k = __shfl_sync(0xffffffffu, k, 0);
+        if (k >= *s_ntask) break;
+        const int nchunks = *s_ntask / TC_N_ROLES;
+        const int role = k / nchunks, sl = (k - role * nchunks) * TC_ENV_CHUNK + (threadIdx.x & 31);
+        if (sl < *s_nseg) {
+            const int4 s4 = s_seg[sl];
+            tc_polyline_setup<true>(a.W, a.H, s4.x, s4.y, s4.z, s4.w, s_thick[s_tag[sl] >> 8], role, (TcPrim *)(pw + sl * TC_ENV_SEG_WORDS));
+        }
+    }
+}
+
+// Draws the primitive slots at pw of `nchunks` chunks of 32 segments (nseg of them filled), one thread per primitive: a warp
+// takes one slot (= one kind of primitive) of the 32 segments of a chunk. Round 0: every lane draws its own primitive if it is
+// short; further rounds: the whole warp draws the long ones (more than TC_SMALL_PRIM_ITEMS items), one after the other - one
+// instance of the drawing code serves both. plane_of(sl) is the plane that segment sl of the round draws into.
+template <int NT, typename PlaneOf>
+__device__ __forceinline__ void tc_draw_prims_by_thread(const int32_t *pw, int nchunks, int nseg, PlaneOf plane_of) {
+    const int lane = threadIdx.x & 31;
+    for (int p = threadIdx.x; p < nchunks * TC_MAX_PRIMS_PER_SEG * 32; p += NT) {   // uniform trip count within a warp
+        const int c = p / (TC_MAX_PRIMS_PER_SEG * 32), slot = (p - c * (TC_MAX_PRIMS_PER_SEG * 32)) >> 5;
+        const int sl0 = c * TC_ENV_CHUNK;
+        const TcPrim *q = (const TcPrim *)(pw + (sl0 + lane) * TC_ENV_SEG_WORDS + slot * 8);
+        int items = 0;
+        if (sl0 + lane < nseg && q->kind != TC_PRIM_NONE) items = tc_prim_items(*q);
+        unsigned big = __ballot_sync(0xffffffffu, items > TC_SMALL_PRIM_ITEMS);
+        bool own = true;
+        while (own || big) {
+            int src = lane;
+            bool active = items > 0 && items <= TC_SMALL_PRIM_ITEMS;
+            TcLanes gg = {0, 1};
+            if (!own) {
+                src = __ffs(big) - 1;
+                big &= big - 1;
+                active = true;
+                gg.lane = lane; gg.n = 32;
+            }
+            own = false;
+            if (active) tc_prim_draw(gg, plane_of(sl0 + src), *(const TcPrim *)(pw + (sl0 + src) * TC_ENV_SEG_WORDS + slot * 8));
+        }
+    }
+}
+
+// Stores view env's stacked C*H-row plane in the output format; any == false: the view has no segments, the frame is zeros.
+template <int NT, int FMT>
+__device__ __forceinline__ void tc_store_env_frame(const TcRenderEnvArgs &a, int env, const uint32_t *plane, const uint32_t *s_color24, bool any) {
+    if (FMT == TC_FMT_RGB)
+        tc_store_rgb<NT>(a.obs + (size_t)env * a.H * a.W * 3, (uint32_t)(a.H * a.W), plane, (uint32_t)(a.H * a.W), a.n_classes, s_color24, any);
+    else if (FMT == TC_FMT_BITS) {
+        // planes are whole words here (the host only selects this format for H*W % 32 == 0)
+        const int words = (int)(((size_t)a.H * a.W + 31) / 32) * a.n_classes;
+        tc_store_bits<NT>((uint32_t *)a.obs + (size_t)env * words, words, plane, any);
+    } else if (FMT == TC_FMT_BF16)
+        tc_store_bf16<NT>((uint16_t *)a.obs + (size_t)env * a.n_classes * a.H * a.W, (uint32_t)(a.n_classes * a.H * a.W), plane, any);
+    else tc_store_plane_sparse<NT>(a.obs + (size_t)env * a.n_classes * a.H * a.W, (size_t)a.n_classes * a.H * a.W, plane, any);
+}
+
 template <int NT, int FMT>
 __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_env_kernel(const TcRenderEnvArgs a) {
-    constexpr bool RGB = FMT == TC_FMT_RGB;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int seg_cnt;
     __shared__ __align__(8) uint64_t bar;
@@ -1071,34 +1259,11 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_env_kernel(const TcRe
     const int env = blockIdx.x;
     if (a.mask && !a.mask[env]) return;
     const int tid = threadIdx.x;
-#ifdef TC_TIMELINE
-#define TC_TL(stmt) do { if (a.timeline && tid == 0) { stmt; } } while (0)
-    long long tl0 = 0, tl1 = 0, tl2 = 0, tl3 = 0, tl_setup = 0, tl_draw = 0, tl_z = 0, tc0 = 0;
-#else
-#define TC_TL(stmt) do { } while (0)
-#endif
+    TC_TL_DECL;
     TC_TL(tl0 = clock64());
     const size_t np = (size_t)a.np;
     unsigned char *tab_smem = smem_raw + tc_env_off_tables(np);
-    if (tid == 0) {
-        // which part of the map can this camera see: its ground cell selects the tables (one TMA bulk copy)
-        const TcCellBlob d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
-        seg_cnt = 0;
-        tc_mbar_init(&bar, 1);
-        tc_fence_mbar_init();
-        if (d.bytes > 0) {
-            tc_mbar_expect_tx(&bar, (uint32_t)d.bytes);
-            tc_bulk_g2s(tab_smem, a.cell_blob + d.offset, (uint32_t)d.bytes, &bar);
-        }
-        s_desc = d;
-    }
-    if (RGB && tid >= 64 && tid < 64 + TC_MAX_CLASSES) {
-        const int cc = tid - 64;
-        s_color24[cc] = tc_color24_of(a.colors, cc);
-    }
-    if (tid >= 32 && tid < 44) s_pose[tid - 32] = a.pose[(size_t)env * 12 + tid - 32];
-    else if (tid >= 44 && tid < 44 + (TC_CAM_MAX_RANGE - TC_CAM_FX + 1)) s_cam[TC_CAM_FX + tid - 44] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + tid - 44];
-    __syncthreads();      // barrier init, descriptor, pose and intrinsics visible to all threads
+    tc_stage_env<FMT == TC_FMT_RGB>(a, env, tab_smem, &bar, true, &seg_cnt, &s_desc, s_pose, s_cam, s_color24);
     const int n = s_desc.n_nodes, m = s_desc.n_edges;
     int4 *segs = (int4 *)smem_raw;                                   // phase 2 views
     uint32_t *plane = (uint32_t *)(smem_raw + tc_env_off_plane(np));
@@ -1108,7 +1273,6 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_env_kernel(const TcRe
     }
     const int cnt = seg_cnt;
     TC_TL(tl2 = clock64());
-    const int n_planes = a.n_classes;
     if (cnt > 0) {
         const uint8_t *seg_cls = (const uint8_t *)(segs + m);
         // the plane is zeroed by the warps that have no role in the first set-up round (when the block has more warps than roles)
@@ -1120,12 +1284,10 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_env_kernel(const TcRe
         TC_TL(tl_z = clock64());
         const int t = a.thickness[env];
         const int warp = tid >> 5, lane = tid & 31;
-        const TcLanes g = {lane, 32}, g1 = {0, 1};
         for (int base = 0; base < cnt; base += TC_ENV_CHUNK) {
             const int nseg = min(TC_ENV_CHUNK, cnt - base);
             TC_TL(tc0 = clock64());
-            for (int i = tid; i < nseg * TC_MAX_PRIMS_PER_SEG; i += NT)
-                pw[(i / TC_MAX_PRIMS_PER_SEG) * TC_ENV_SEG_WORDS + (i % TC_MAX_PRIMS_PER_SEG) * 8] = TC_PRIM_NONE;
+            tc_clear_prim_slots<NT>(pw, nseg);
             __syncthreads();
             if (ZERO_IN_SETUP && base == 0 && warp >= TC_N_ROLES) {
                 for (int i = tid - TC_N_ROLES * 32; i < a.plane_words; i += NT - TC_N_ROLES * 32) plane[i] = 0;
@@ -1136,58 +1298,21 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_env_kernel(const TcRe
             }
             __syncthreads();
             TC_TL(long long x = clock64(); tl_setup += x - tc0; tc0 = x);
-            // one thread per primitive; a warp takes one slot (= one kind of primitive) of the 32 segments
-            for (int p = tid; p < TC_MAX_PRIMS_PER_SEG * 32; p += NT) {   // uniform trip count within a warp
-                const int slot = p >> 5;
-                const TcPrim *q = (const TcPrim *)(pw + lane * TC_ENV_SEG_WORDS + slot * 8);
-                int items = 0;
-                if (lane < nseg && q->kind != TC_PRIM_NONE) items = tc_prim_items(*q);
-                // round 0: every lane draws its own primitive if it is short; further rounds: the whole warp draws the long
-                // ones, one after the other (one instance of the drawing code serves both)
-                unsigned big = __ballot_sync(0xffffffffu, items > TC_SMALL_PRIM_ITEMS);
-                bool own = true;
-                while (own || big) {
-                    int src = lane;
-                    bool active = items > 0 && items <= TC_SMALL_PRIM_ITEMS;
-                    TcLanes gg = g1;
-                    if (!own) {
-                        src = __ffs(big) - 1;
-                        big &= big - 1;
-                        active = true;
-                        gg = g;
-                    }
-                    own = false;
-                    if (active) {
-                        TcPlane pl = {plane, a.H, a.W, 0, a.H, -(int)seg_cls[base + src] * a.H};
-                        tc_prim_draw(gg, pl, *(const TcPrim *)(pw + src * TC_ENV_SEG_WORDS + slot * 8));
-                    }
-                }
-            }
+            tc_draw_prims_by_thread<NT>(pw, 1, nseg, [&](int sl) {
+                const TcPlane pl = {plane, a.H, a.W, 0, a.H, -(int)seg_cls[base + sl] * a.H};
+                return pl;
+            });
             __syncthreads();
             TC_TL(tl_draw += clock64() - tc0);
         }
     }
     TC_TL(tl3 = clock64());
-    if (FMT == TC_FMT_RGB)
-        tc_store_rgb<NT>(a.obs + (size_t)env * a.H * a.W * 3, (uint32_t)(a.H * a.W), plane, (uint32_t)(a.H * a.W), a.n_classes, s_color24, cnt > 0);
-    else if (FMT == TC_FMT_BITS) {
-        // planes are whole words here (the host only selects this format for H*W % 32 == 0)
-        const int words = (int)(((size_t)a.H * a.W + 31) / 32) * n_planes;
-        tc_store_bits<NT>((uint32_t *)a.obs + (size_t)env * words, words, plane, cnt > 0);
-    } else if (FMT == TC_FMT_BF16)
-        tc_store_bf16<NT>((uint16_t *)a.obs + (size_t)env * n_planes * a.H * a.W, (uint32_t)(n_planes * a.H * a.W), plane, cnt > 0);
-    else tc_store_plane_sparse<NT>(a.obs + (size_t)env * n_planes * a.H * a.W, (size_t)n_planes * a.H * a.W, plane, cnt > 0);
-#ifdef TC_TIMELINE
-    if (a.timeline && tid == 0) {
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        long long *r = a.timeline + (size_t)blockIdx.x * 10;
-        r[0] = smid; r[1] = tl0; r[2] = tl1 ? tl1 : tl0; r[3] = tl2; r[4] = tl3; r[5] = clock64();
-        r[6] = cnt; r[7] = tl_z ? tl_z - tl2 : 0; r[8] = tl_setup; r[9] = tl_draw;
-    }
-#endif
-#undef TC_TL
+    tc_store_env_frame<NT, FMT>(a, env, plane, s_color24, cnt > 0);
+    TC_TL_RECORD(tl1 ? tl1 : tl0, cnt);   // (the tables' arrival is waited for inside the camera pass: no t1 of its own)
 }
+#undef TC_TL
+#undef TC_TL_DECL
+#undef TC_TL_RECORD
 
 // ------------------------------------------------------------------------------------------------ fused, E envs per block
 // tc_render_env_kernel leaves most of its lanes idle: a Knuffingen frame has ~120 nodes for 256 threads, ~12 segments for
@@ -1220,7 +1345,6 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_render_envs_ker
     // Register discipline: the set-up code needs all 64 registers, and a spilled value is a local-memory access that queues
     // behind the observation stores of the co-resident blocks (thousands of cycles each). So nothing is kept in registers across
     // the phases that can be re-read from the kernel parameters (constant bank) or from shared memory.
-    constexpr int TPE = NT / E;                       // threads of the camera pass per env
     constexpr int CAP = TC_ENVS_CHUNKS * TC_ENV_CHUNK; // most segments per set-up round (a.prim_chunks <= TC_ENVS_CHUNKS chunks of 32)
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int seg_cnt[E], s_pref[E + 1], s_thick[E], s_active[E];
@@ -1231,49 +1355,10 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_render_envs_ker
     __shared__ int4 s_seg[CAP];        // the round's segments ...
     __shared__ uint16_t s_tag[CAP];    // ... and for each its env slot << 8 | class
     __shared__ int s_task, s_nseg, s_ntask;
-#define TC_REGION(e) (smem_raw + (size_t)(e) * a.region_bytes)
-#define TC_PLANE(e) ((uint32_t *)(TC_REGION(e) + (size_t)a.np * 24))
+#define TC_PLANE(e) ((uint32_t *)(smem_raw + (size_t)(e) * a.region_bytes + (size_t)a.np * 24))
 #define TC_PW ((int32_t *)(smem_raw + (size_t)E * a.region_bytes))
-    if (threadIdx.x == 0) {
-        tc_mbar_init(&bar, E);
-        tc_fence_mbar_init();
-    }
-    __syncwarp();
-    if (threadIdx.x < E) {
-        // which part of the map can this env's camera see: its ground cell selects the tables (one TMA bulk copy per env)
-        const int e = threadIdx.x, env = blockIdx.x * E + e;
-        const bool act = env < a.n_envs && !(a.mask && !a.mask[env]);
-        TcCellBlob d;
-        if (act) d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
-        else { d.n_nodes = 0; d.n_edges = 0; d.bytes = 0; d.offset = 0; }
-        s_active[e] = act; seg_cnt[e] = 0; s_thick[e] = act ? a.thickness[env] : 1;
-        s_desc[e] = d;
-        // one arrival per env slot, with its bytes
-        if (d.bytes > 0) {
-            tc_mbar_expect_tx(&bar, (uint32_t)d.bytes);
-            tc_bulk_g2s(TC_REGION(e) + tc_env_off_tables((size_t)a.np), a.cell_blob + d.offset, (uint32_t)d.bytes, &bar);
-        } else tc_mbar_arrive(&bar);
-    }
-    if (FMT == TC_FMT_RGB && threadIdx.x >= 64 && threadIdx.x < 64 + TC_MAX_CLASSES) s_color24[threadIdx.x - 64] = tc_color24_of(a.colors, threadIdx.x - 64);
-    if (threadIdx.x >= 32 && threadIdx.x < 32 + E * 17) {
-        const int k = threadIdx.x - 32, e = k / 17, i = k % 17, env = blockIdx.x * E + e;
-        if (env < a.n_envs) {
-            if (i < 12) s_pose[e][i] = a.pose[(size_t)env * 12 + i];
-            else s_cam[e][TC_CAM_FX + i - 12] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + i - 12];
-        }
-    }
-    __syncthreads();
-    // ---- camera pass (camera.py:52-110) of the E envs side by side: thread -> (env slot j, index of its TPE threads)
-    {
-        const int j = threadIdx.x / TPE;
-        tc_env_camera_pass<TPE, true>(TC_REGION(j), (size_t)a.np, TC_REGION(j) + tc_env_off_tables((size_t)a.np), s_desc[j], &bar, s_pose[j], s_cam[j], a.H, a.W,
-                                &seg_cnt[j], (int)threadIdx.x - j * TPE);
-    }
-    if (threadIdx.x == 0) {
-        int acc = 0;
-        for (int e = 0; e < E; e++) { s_pref[e] = acc; acc += seg_cnt[e]; }
-        s_pref[E] = acc;
-    }
+    tc_stage_envs<NT, E, FMT == TC_FMT_RGB>(a, smem_raw, &bar, seg_cnt, s_thick, s_active, s_desc, s_pose, s_cam, s_color24);
+    tc_seg_prefix<E>(seg_cnt, s_pref);
     // zero the planes of the envs that have segments (the others are stored as zeros without a plane)
     for (int e = 0; e < E; e++)
         if (seg_cnt[e] > 0) {
@@ -1284,88 +1369,21 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_render_envs_ker
     for (int base = 0; base < s_pref[E]; base += a.prim_chunks * TC_ENV_CHUNK) {
         {
             const int nseg = min(a.prim_chunks * TC_ENV_CHUNK, s_pref[E] - base);
-            int32_t *pw = TC_PW;
-            for (int i = threadIdx.x; i < nseg * TC_MAX_PRIMS_PER_SEG; i += NT)
-                pw[(i / TC_MAX_PRIMS_PER_SEG) * TC_ENV_SEG_WORDS + (i % TC_MAX_PRIMS_PER_SEG) * 8] = TC_PRIM_NONE;
-            if ((int)threadIdx.x < nseg) {   // segment tid of the round: find its env slot, copy it next to its tag
-                const int sidx = base + threadIdx.x;
-                int e = 0;
-#pragma unroll
-                for (int k = 1; k < E; k++) e += sidx >= s_pref[k];
-                const int i = sidx - s_pref[e];
-                const int4 *segs = (const int4 *)TC_REGION(e);
-                s_seg[threadIdx.x] = segs[i];
-                s_tag[threadIdx.x] = (uint16_t)((e << 8) | ((const uint8_t *)(segs + s_desc[e].n_edges))[i]);
-            }
-            if (threadIdx.x == 0) {
-                s_task = 0; s_nseg = nseg;
-                s_ntask = ((nseg + TC_ENV_CHUNK - 1) / TC_ENV_CHUNK) * TC_N_ROLES;
-            }
+            tc_clear_prim_slots<NT>(TC_PW, nseg);
+            tc_gather_round<E, false>(a, smem_raw, base, nseg, s_pref, s_desc, s_seg, s_tag, nullptr, nullptr, &s_task, &s_nseg, &s_ntask);
         }
         __syncthreads();
-        // set-up: (role, chunk) tasks from a queue, lane = segment of the chunk; spans (role 0) are handed out first.
-        // (Tried in round 2 and rejected: draw tasks in the same queue, each waiting only for the set-up task that fills its slot, so
-        // that the short roles' primitives are drawn while the spans are still being set up - no barrier between the phases, but
-        // 9-10 % slower on every small-frame configuration: the ticket order serialises what the barrier let all warps share.)
-        while (true) {
-            int k = 0;
-            if ((threadIdx.x & 31) == 0) k = atomicAdd(&s_task, 1);
-            k = __shfl_sync(0xffffffffu, k, 0);
-            if (k >= s_ntask) break;
-            const int nchunks = s_ntask / TC_N_ROLES;
-            const int role = k / nchunks, sl = (k - role * nchunks) * TC_ENV_CHUNK + (threadIdx.x & 31);
-            if (sl < s_nseg) {
-                const int4 s4 = s_seg[sl];
-                tc_polyline_setup<true>(a.W, a.H, s4.x, s4.y, s4.z, s4.w, s_thick[s_tag[sl] >> 8], role, (TcPrim *)(TC_PW + sl * TC_ENV_SEG_WORDS));
-            }
-        }
+        tc_setup_queue(a, &s_task, &s_ntask, &s_nseg, s_seg, s_tag, s_thick, TC_PW);
         __syncthreads();
-        // draw: one thread per primitive; a warp takes one slot (= one kind of primitive) of the 32 segments of a chunk
-        for (int p = threadIdx.x; p < (s_ntask / TC_N_ROLES) * TC_MAX_PRIMS_PER_SEG * 32; p += NT) {   // uniform trip count within a warp
-            const int lane = threadIdx.x & 31;
-            const int c = p / (TC_MAX_PRIMS_PER_SEG * 32), slot = (p - c * (TC_MAX_PRIMS_PER_SEG * 32)) >> 5;
-            const int sl0 = c * TC_ENV_CHUNK;
-            const int32_t *pw = TC_PW;
-            const TcPrim *q = (const TcPrim *)(pw + (sl0 + lane) * TC_ENV_SEG_WORDS + slot * 8);
-            int items = 0;
-            if (sl0 + lane < s_nseg && q->kind != TC_PRIM_NONE) items = tc_prim_items(*q);
-            unsigned big = __ballot_sync(0xffffffffu, items > TC_SMALL_PRIM_ITEMS);
-            bool own = true;
-            while (own || big) {
-                int src = lane;
-                bool active = items > 0 && items <= TC_SMALL_PRIM_ITEMS;
-                TcLanes gg = {0, 1};
-                if (!own) {
-                    src = __ffs(big) - 1;
-                    big &= big - 1;
-                    active = true;
-                    gg.lane = lane; gg.n = 32;
-                }
-                own = false;
-                if (active) {
-                    const int tag = s_tag[sl0 + src];
-                    TcPlane pl = {TC_PLANE(tag >> 8), a.H, a.W, 0, a.H, -(tag & 0xff) * a.H};
-                    tc_prim_draw(gg, pl, *(const TcPrim *)(pw + (sl0 + src) * TC_ENV_SEG_WORDS + slot * 8));
-                }
-            }
-        }
+        tc_draw_prims_by_thread<NT>(TC_PW, s_ntask / TC_N_ROLES, s_nseg, [&](int sl) {
+            const int tag = s_tag[sl];
+            const TcPlane pl = {TC_PLANE(tag >> 8), a.H, a.W, 0, a.H, -(tag & 0xff) * a.H};
+            return pl;
+        });
         __syncthreads();
     }
-    for (int e = 0; e < E; e++) {
-        if (!s_active[e]) continue;
-        const int env = blockIdx.x * E + e;
-        const uint32_t *plane = TC_PLANE(e);
-        const bool any = seg_cnt[e] > 0;
-        if (FMT == TC_FMT_RGB)
-            tc_store_rgb<NT>(a.obs + (size_t)env * a.H * a.W * 3, (uint32_t)(a.H * a.W), plane, (uint32_t)(a.H * a.W), a.n_classes, s_color24, any);
-        else if (FMT == TC_FMT_BITS) {
-            const int words = (int)(((size_t)a.H * a.W + 31) / 32) * a.n_classes;
-            tc_store_bits<NT>((uint32_t *)a.obs + (size_t)env * words, words, plane, any);
-        } else if (FMT == TC_FMT_BF16)
-            tc_store_bf16<NT>((uint16_t *)a.obs + (size_t)env * a.n_classes * a.H * a.W, (uint32_t)(a.n_classes * a.H * a.W), plane, any);
-        else tc_store_plane_sparse<NT>(a.obs + (size_t)env * a.n_classes * a.H * a.W, (size_t)a.n_classes * a.H * a.W, plane, any);
-    }
-#undef TC_REGION
+    for (int e = 0; e < E; e++)
+        if (s_active[e]) tc_store_env_frame<NT, FMT>(a, blockIdx.x * E + e, TC_PLANE(e), s_color24, seg_cnt[e] > 0);
 #undef TC_PLANE
 #undef TC_PW
 }
@@ -1390,7 +1408,6 @@ struct TcPrimsOut {
 
 template <int NT, int E>
 __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_prims_kernel(const TcRenderEnvArgs a, const TcPrimsOut o) {
-    constexpr int TPE = NT / E;
     constexpr int CAP = TC_ENVS_CHUNKS * TC_ENV_CHUNK;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int seg_cnt[E], s_pref[E + 1], s_thick[E], s_active[E];
@@ -1405,38 +1422,8 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_prims_kernel(co
 #define TC_REGION(e) (smem_raw + (size_t)(e) * a.region_bytes)
 #define TC_PW ((int32_t *)(smem_raw + (size_t)E * a.region_bytes))
 #define TC_RANK(e) ((uint16_t *)(TC_REGION(e) + (size_t)a.np * 24))   /* rank of a segment within its class: over the dead camera-pass scratch */
-    if (threadIdx.x == 0) {
-        tc_mbar_init(&bar, E);
-        tc_fence_mbar_init();
-    }
     if (threadIdx.x < E * TC_MAX_CLASSES) (&s_clscnt[0][0])[threadIdx.x] = 0;
-    __syncwarp();
-    if (threadIdx.x < E) {
-        const int e = threadIdx.x, env = blockIdx.x * E + e;
-        const bool act = env < a.n_envs && !(a.mask && !a.mask[env]);
-        TcCellBlob d;
-        if (act) d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
-        else { d.n_nodes = 0; d.n_edges = 0; d.bytes = 0; d.offset = 0; }
-        s_active[e] = act; seg_cnt[e] = 0; s_thick[e] = act ? a.thickness[env] : 1;
-        s_desc[e] = d;
-        if (d.bytes > 0) {
-            tc_mbar_expect_tx(&bar, (uint32_t)d.bytes);
-            tc_bulk_g2s(TC_REGION(e) + tc_env_off_tables((size_t)a.np), a.cell_blob + d.offset, (uint32_t)d.bytes, &bar);
-        } else tc_mbar_arrive(&bar);
-    }
-    if (threadIdx.x >= 32 && threadIdx.x < 32 + E * 17) {
-        const int k = threadIdx.x - 32, e = k / 17, i = k % 17, env = blockIdx.x * E + e;
-        if (env < a.n_envs) {
-            if (i < 12) s_pose[e][i] = a.pose[(size_t)env * 12 + i];
-            else s_cam[e][TC_CAM_FX + i - 12] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + i - 12];
-        }
-    }
-    __syncthreads();
-    {
-        const int j = threadIdx.x / TPE;
-        tc_env_camera_pass<TPE, true>(TC_REGION(j), (size_t)a.np, TC_REGION(j) + tc_env_off_tables((size_t)a.np), s_desc[j], &bar, s_pose[j], s_cam[j], a.H, a.W,
-                                &seg_cnt[j], (int)threadIdx.x - j * TPE);
-    }
+    tc_stage_envs<NT, E, false>(a, smem_raw, &bar, seg_cnt, s_thick, s_active, s_desc, s_pose, s_cam, nullptr);
     if (threadIdx.x < E) {
         const int e = threadIdx.x, env = blockIdx.x * E + e;
         if (env < a.n_envs) {
@@ -1453,11 +1440,7 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_prims_kernel(co
         const uint8_t *cls = (const uint8_t *)((const int4 *)TC_REGION(e) + s_desc[e].n_edges);
         for (int i = threadIdx.x; i < seg_cnt[e]; i += NT) TC_RANK(e)[i] = (uint16_t)atomicAdd(&s_clscnt[e][cls[i]], 1);
     }
-    if (threadIdx.x == 0) {
-        int acc = 0;
-        for (int e = 0; e < E; e++) { s_pref[e] = acc; acc += seg_cnt[e]; }
-        s_pref[E] = acc;
-    }
+    tc_seg_prefix<E>(seg_cnt, s_pref);
     __syncthreads();
     if (threadIdx.x < E * a.n_classes) {
         const int e = threadIdx.x / a.n_classes, c = threadIdx.x - e * a.n_classes, env = blockIdx.x * E + e;
@@ -1470,39 +1453,11 @@ __global__ void __launch_bounds__(NT, TC_ENVS_MIN_BLOCKS(NT)) tc_prims_kernel(co
     for (int base = 0; base < s_pref[E]; base += a.prim_chunks * TC_ENV_CHUNK) {
         {
             const int nseg = min(a.prim_chunks * TC_ENV_CHUNK, s_pref[E] - base);
-            int32_t *pw = TC_PW;
-            for (int i = threadIdx.x; i < nseg * TC_MAX_PRIMS_PER_SEG; i += NT)
-                pw[(i / TC_MAX_PRIMS_PER_SEG) * TC_ENV_SEG_WORDS + (i % TC_MAX_PRIMS_PER_SEG) * 8] = TC_PRIM_NONE;
-            if ((int)threadIdx.x < nseg) {
-                const int sidx = base + threadIdx.x;
-                int e = 0;
-#pragma unroll
-                for (int k = 1; k < E; k++) e += sidx >= s_pref[k];
-                const int i = sidx - s_pref[e];
-                const int4 *segs = (const int4 *)TC_REGION(e);
-                const uint8_t cls = ((const uint8_t *)(segs + s_desc[e].n_edges))[i];
-                s_seg[threadIdx.x] = segs[i];
-                s_tag[threadIdx.x] = (uint16_t)((e << 8) | cls);
-                s_gpos[threadIdx.x] = s_clsoff[e][cls] + TC_RANK(e)[i];
-            }
-            if (threadIdx.x == 0) {
-                s_task = 0; s_nseg = nseg;
-                s_ntask = ((nseg + TC_ENV_CHUNK - 1) / TC_ENV_CHUNK) * TC_N_ROLES;
-            }
+            tc_clear_prim_slots<NT>(TC_PW, nseg);
+            tc_gather_round<E, true>(a, smem_raw, base, nseg, s_pref, s_desc, s_seg, s_tag, s_gpos, s_clsoff, &s_task, &s_nseg, &s_ntask);
         }
         __syncthreads();
-        while (true) {
-            int k = 0;
-            if ((threadIdx.x & 31) == 0) k = atomicAdd(&s_task, 1);
-            k = __shfl_sync(0xffffffffu, k, 0);
-            if (k >= s_ntask) break;
-            const int nchunks = s_ntask / TC_N_ROLES;
-            const int role = k / nchunks, sl = (k - role * nchunks) * TC_ENV_CHUNK + (threadIdx.x & 31);
-            if (sl < s_nseg) {
-                const int4 s4 = s_seg[sl];
-                tc_polyline_setup<true>(a.W, a.H, s4.x, s4.y, s4.z, s4.w, s_thick[s_tag[sl] >> 8], role, (TcPrim *)(TC_PW + sl * TC_ENV_SEG_WORDS));
-            }
-        }
+        tc_setup_queue(a, &s_task, &s_ntask, &s_nseg, s_seg, s_tag, s_thick, TC_PW);
         __syncthreads();
         // the round's primitives to global memory: consecutive threads write consecutive words of a segment's 12 slots
         for (int i = threadIdx.x; i < s_nseg * TC_PRIMS_SEG_WORDS; i += NT) {
@@ -1630,19 +1585,7 @@ __global__ void __launch_bounds__(256, TC_ENVB_MIN_BLOCKS) tc_render_env_banded_
     for (int env = blockIdx.x; env < a.n_envs; env += gridDim.x) {
     if (a.mask && !a.mask[env]) continue;
     __syncthreads();   // the previous env's shared state is dead (and the barrier initialised)
-    if (tid == 0) {
-        const TcCellBlob d = a.cell_desc[tc_cull_cell(a.grid, a.pose + (size_t)env * 12)];
-        seg_cnt = 0;
-        if (d.bytes > 0) {
-            tc_mbar_expect_tx(&bar, (uint32_t)d.bytes);
-            tc_bulk_g2s(tab_smem, a.cell_blob + d.offset, (uint32_t)d.bytes, &bar);
-        }
-        s_desc = d;
-    }
-    if (FMT == TC_FMT_RGB && tid >= 64 && tid < 64 + TC_MAX_CLASSES) s_color24[tid - 64] = tc_color24_of(a.colors, tid - 64);
-    if (tid >= 32 && tid < 44) s_pose[tid - 32] = a.pose[(size_t)env * 12 + tid - 32];
-    else if (tid >= 44 && tid < 44 + (TC_CAM_MAX_RANGE - TC_CAM_FX + 1)) s_cam[TC_CAM_FX + tid - 44] = a.cam[(size_t)env * TC_CAM_N + TC_CAM_FX + tid - 44];
-    __syncthreads();
+    tc_stage_env<FMT == TC_FMT_RGB>(a, env, tab_smem, &bar, false, &seg_cnt, &s_desc, s_pose, s_cam, s_color24);
     const int n = s_desc.n_nodes, m = s_desc.n_edges;
     int4 *segs = (int4 *)smem_raw;
     uint32_t *planes = (uint32_t *)(smem_raw + np * 24);
@@ -1659,8 +1602,7 @@ __global__ void __launch_bounds__(256, TC_ENVB_MIN_BLOCKS) tc_render_env_banded_
     // ---- rasteriser: set-up once (or, for more than TC_RGBE_MAX_SEGS segments, per band in rounds), bands in turn
     auto setup = [&](int first, int cnt) {
         if (tid == 0) band_mask = 0;
-        for (int i = tid; i < cnt * TC_MAX_PRIMS_PER_SEG; i += NT)
-            pw[(i / TC_MAX_PRIMS_PER_SEG) * TC_ENV_SEG_WORDS + (i % TC_MAX_PRIMS_PER_SEG) * 8] = TC_PRIM_NONE;
+        tc_clear_prim_slots<NT>(pw, cnt);
         __syncthreads();
         for (int sub = 0; sub < cnt; sub += 32) {
             const int sl = sub + lane;
