@@ -31,7 +31,10 @@ struct TcLanes {
 };
 
 // lexicographic (value, index) minimum over the group; every lane receives the result. Ties -> lowest index
-// (layer.py:44 `d.index(min(d))`).
+// (layer.py:44 `d.index(min(d))`). A NaN value ties with another NaN: a car whose position is NaN (a NaN action) has NaN
+// distances to every edge, and the sequential scan keeps its first candidate. Without the tie each lane would keep its own
+// first candidate, and the result would depend on the lane that stores it (lane 0 of a group, or the lane that asked a
+// whole warp to scan for it in the thread-per-env kernel).
 TC_HD void tc_group_argmin(const TcLanes &g, double &d, int &idx) {
 #if defined(__CUDA_ARCH__)
     // groups are aligned power-of-two slices of a warp (32: warp-per-env tracking; 8: four envs per warp; 1: thread-per-env, where
@@ -43,7 +46,7 @@ TC_HD void tc_group_argmin(const TcLanes &g, double &d, int &idx) {
     for (int off = g.n >> 1; off > 0; off >>= 1) {
         double od = __shfl_xor_sync(mask, d, off);
         int oi = __shfl_xor_sync(mask, idx, off);
-        if (oi >= 0 && (idx < 0 || od < d || (od == d && oi < idx))) {
+        if (oi >= 0 && (idx < 0 || od < d || ((od == d || (od != od && d != d)) && oi < idx))) {
             d = od;
             idx = oi;
         }
