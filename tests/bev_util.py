@@ -41,16 +41,20 @@ def oracle_bev(tables, sf_row, si_row, H, W, pixel_per_meter, car_pixel, thickne
     return out
 
 
-def oracle_bev_ulp(tables, sf_row, si_row, got, **kw):
-    """Compares a device BEV frame with the oracle. -> 0: identical with libm's cos / sin, 1: identical once cos or sin is moved
-    by one ulp (the documented device-versus-glibc difference), -1: anything else."""
-    if np.array_equal(got, oracle_bev(tables, sf_row, si_row, **kw)):
+def oracle_bev_ulp(tables, sf_row, si_row, got, bits=False, **kw):
+    """Compares a device BEV frame with the oracle (bits: `got` is the classes_bits frame, compared with pack_bits of the
+    oracle's). -> 0: identical with libm's cos / sin, 1: identical once cos or sin is moved by one ulp (the documented
+    device-versus-glibc difference), -1: anything else."""
+    def same(cs=None):
+        want = oracle_bev(tables, sf_row, si_row, cs=cs, **kw)
+        return np.array_equal(got, pack_bits(want) if bits else want)
+    if same():
         return 0
     rot = float(sf_row[2])
     c, s = math.cos(rot), math.sin(rot)
     for cc in (np.nextafter(c, -np.inf), c, np.nextafter(c, np.inf)):
         for ss in (np.nextafter(s, -np.inf), s, np.nextafter(s, np.inf)):
-            if (cc, ss) != (c, s) and np.array_equal(got, oracle_bev(tables, sf_row, si_row, cs=(float(cc), float(ss)), **kw)):
+            if (cc, ss) != (c, s) and same((float(cc), float(ss))):
                 return 1
     return -1
 

@@ -11,6 +11,7 @@ the known ones; only the laneline layers are regrouped:
        every node to two classes (1494 nodes instead of 827), and the whole-graph tables of that union outgrow what the
        small-frame block-per-env kernels accept (tc_create's fused_all rule); the runs keep the union near Knuffingen's size,
        so 16 classes reach those kernels too, with class joints every 16 edges.
+  K15  K16 without its empty class: 15 classes, so that 15 classes + the bird's-eye view's route plane make 16 planes.
 Tests only; the product never imports this."""
 import copy
 import json
@@ -99,7 +100,13 @@ def k16(run=1):
     return d
 
 
-MAPS = {"K1": k1, "K2": k2, "K16": k16, "K16R": lambda: k16(run=16)}
+def k15():
+    d = k16()
+    d["lanelines"].pop(f"c{K16_EMPTY:02d}")
+    return d
+
+
+MAPS = {"K1": k1, "K2": k2, "K15": k15, "K16": k16, "K16R": lambda: k16(run=16)}
 
 
 def write(data, directory, name):
