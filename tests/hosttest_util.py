@@ -46,6 +46,9 @@ def ht():
         L.ht_project_culled.argtypes = [vp, vp, i, i, i, vp, vp, vp, vp, vp]
         L.ht_nearest.argtypes = [vp, i, vp, i, i, vp, vp, vp]
         L.ht_polyline.argtypes = [vp, i, i, C.c_int32, C.c_int32, C.c_int32, C.c_int32, i, i, i, i]
+        L.ht_philox.argtypes = [i, vp, vp, vp]
+        L.ht_circle.argtypes = [vp, i, i, i, i, i]
+        L.ht_noise_blobs.argtypes = [vp, i, i, i, i, i, C.c_uint64, C.c_uint32, i, i, C.c_int32, vp]
         _ht = L
     return _ht
 
@@ -120,6 +123,30 @@ class HostCore:
         self._track(0, cc, man, None, None)
         if render:
             self.render()
+
+
+def philox(ctr, key):
+    """Philox4x32-10 of counters ctr [n,4] under keys key [n,2] (uint32) -> [n,4]"""
+    ctr, key = np.ascontiguousarray(ctr, np.uint32), np.ascontiguousarray(key, np.uint32)
+    out = np.zeros((len(ctr), 4), np.uint32)
+    ht().ht_philox(len(ctr), P(ctr), P(key), P(out))
+    return out
+
+
+def circle(H, W, centre, radius):
+    img = np.zeros((H, W), np.uint8)
+    ht().ht_circle(P(img), H, W, int(centre[0]), int(centre[1]), int(radius))
+    return img
+
+
+def noise_blobs(obs, seed, step, n_blobs, max_radius, env_index_offset=0, mask=None):
+    """ht_noise_blobs on obs u8 [N, M, C, H, W] (a copy), mask per env -> the noised copy"""
+    out = np.array(obs, np.uint8, order="C")
+    N, M, Cn, H, W = out.shape
+    m = None if mask is None else np.ascontiguousarray(mask, np.uint8)
+    ht().ht_noise_blobs(P(out), N, M, Cn, H, W, int(seed) & (2**64 - 1), int(step) & 0xFFFFFFFF, int(n_blobs), int(max_radius),
+                        int(env_index_offset), P(m))
+    return out
 
 
 def polyline(H, W, p0, p1, t, y_lo=0, y_hi=0, nlanes=1):

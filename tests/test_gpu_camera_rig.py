@@ -13,6 +13,7 @@ import pytest
 import torch
 
 from hosttest_util import ht
+from noise_util import reference_noise
 from pair_util import make_config, oracle_env
 from rig_util import REAR, oracle_view_segments, oracle_views
 from test_gpu_map_shapes import LAUNCHES, decode, render_path
@@ -342,34 +343,6 @@ def test_set_camera_params_per_camera():
     assert np.array_equal(env._cam_rows, rows0) and (env._thickness == 2).all()
 
 
-def philox4x32_10(c, k):
-    c = [int(x) & 0xFFFFFFFF for x in c]
-    k = [int(x) & 0xFFFFFFFF for x in k]
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c[0], 0xCD9E8D57 * c[2]
-        c = [((p1 >> 32) ^ c[1] ^ k[0]) & 0xFFFFFFFF, p1 & 0xFFFFFFFF, ((p0 >> 32) ^ c[3] ^ k[1]) & 0xFFFFFFFF, p0 & 0xFFFFFFFF]
-        k = [(k[0] + 0x9E3779B9) & 0xFFFFFFFF, (k[1] + 0xBB67AE85) & 0xFFFFFFFF]
-    return c
-
-
-def noise_view(obs, env_global, camera, seed, step, n_blobs, max_radius):
-    """observation.py:14-27 with the draws of the tc_noise_blobs contract: counter (env, step, c * n_blobs + blob, camera)"""
-    Cn = obs.shape[0]
-    for c in range(Cn):
-        for k in range(n_blobs):
-            r = philox4x32_10([env_global, step, c * n_blobs + k, camera], [seed & 0xFFFFFFFF, seed >> 32])
-            x, y = r[0] % obs.shape[2], r[1] % obs.shape[1]
-            radius = 1 + r[2] % (max_radius - 1) if max_radius > 1 else 1
-            if (r[3] & 0xFFFF) < 19661:
-                mask = np.zeros(obs[c].shape, dtype=np.uint8)
-                cv2.circle(mask, (x, y), radius, 255, -1)
-                mask = cv2.bitwise_and(obs[(r[3] >> 16) % Cn], mask, mask=mask)
-                obs[c] = cv2.bitwise_or(obs[c], mask)
-            else:
-                cv2.circle(obs[c], (x, y), radius, 0, -1)
-    return obs
-
-
 def test_noise_wrapper_on_rig_views():
     """camera 0's views get the rig-less noise; views of camera m > 0 the noise of counter word 3 = m"""
     from tinycarlo_b200 import TinyCarloVecEnv
@@ -391,7 +364,7 @@ def test_noise_wrapper_on_rig_views():
         changed = 0
         for i in range(n):
             for m in range(1, M):
-                want = noise_view(c[i, m].copy(), off + i, m, seed, t, n_blobs, max_radius)
+                want = reference_noise(c[i, m].copy(), off + i, m, seed, t, n_blobs, max_radius)
                 assert np.array_equal(got[i, m], want), (t, i, m)
                 changed += int((want != c[i, m]).any())
         assert changed > 0

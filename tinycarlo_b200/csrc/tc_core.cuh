@@ -542,6 +542,51 @@ TC_HD int tc_spawn_draw(const TcTrackTables &t, uint64_t *st, const int32_t *cho
     return -1;
 }
 
+// ------------------------------------------------------------------------------------------------ blob noise
+// NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) draws from the unseeded global numpy RNG; tc_noise_blobs
+// draws every blob from Philox4x32-10 instead (contract in include/tinycarlo_b200.h), so the noise is a pure function of
+// (seed, global env index, step, class, blob, camera), reproducible and independent of the sharding.
+TC_HD void tc_philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t *out) {
+    for (int r = 0; r < 10; r++) {
+        uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
+        uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1, n3 = (uint32_t)p0;
+        c0 = n0; c1 = n1; c2 = n2; c3 = n3;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
+
+struct TcBlobDraw {
+    int x, y, radius, copy, src;
+};
+// blob `blob` of class c in camera `cam` of the env with global index env_global (counter word 2 wraps mod 2^32)
+TC_HD TcBlobDraw tc_noise_draw(uint32_t seed_lo, uint32_t seed_hi, uint32_t env_global, uint32_t step, int c, int blob, int cam, int n_blobs,
+                               int max_radius, int H, int W, int C) {
+    uint32_t r[4];
+    tc_philox4x32_10(env_global, step, (uint32_t)c * (uint32_t)n_blobs + (uint32_t)blob, (uint32_t)cam, seed_lo, seed_hi, r);
+    TcBlobDraw d;
+    d.x = (int)(r[0] % (uint32_t)W);
+    d.y = (int)(r[1] % (uint32_t)H);
+    d.radius = max_radius > 1 ? 1 + (int)(r[2] % (uint32_t)(max_radius - 1)) : 1;   // randint(1, max_radius)
+    d.copy = (r[3] & 0xffffu) < 19661u;                                              // p = 0.3
+    d.src = (int)((r[3] >> 16) % (uint32_t)C);
+    return d;
+}
+
+// cv2.circle(img, centre, radius, colour, -1) is the filled midpoint circle: hw[|dy|] (dy = -radius..radius) = the half
+// width of the disc's row dy, -1 for a row it does not reach. hw holds radius + 1 entries.
+TC_HD void tc_circle_halfwidths(int radius, int *hw) {
+    for (int i = 0; i <= radius; i++) hw[i] = -1;
+    int err = 0, dx = radius, dy = 0, plus = 1, minus = (radius << 1) - 1;
+    while (dx >= dy) {
+        hw[dy] = hw[dy] > dx ? hw[dy] : dx;
+        hw[dx] = hw[dx] > dy ? hw[dx] : dy;
+        dy++; err += plus; plus += 2;
+        int m = (err <= 0) - 1;
+        err -= minus & m; dx += m; minus -= m & 2;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ camera.py
 // numpy matmul == OpenBLAS dgemm on these shapes: c_ij = fma(a_i3,b_3j, fma(a_i2,b_2j, fma(a_i1,b_1j, a_i0*b_0j)))
 TC_HD void tc_mm_chain(const double *A, int ar, int ac, const double *B, int bc, double *C) {

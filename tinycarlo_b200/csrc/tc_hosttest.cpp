@@ -2,7 +2,8 @@
 //
 // NOT part of the product: nothing under tinycarlo_b200/*.py loads this library. It exists so that the
 // node-parallel clip passes, the closed-form rasteriser and the tracking logic that the CUDA kernels run can be
-// checked against the oracle in a container without a GPU (tests/test_core_host.py). The glue below mirrors the
+// checked against the oracle in a container without a GPU (tests/test_core_host.py), and the blob noise against cv2
+// (tests/test_noise_host.py). The glue below mirrors the
 // kernels in tc_kernels.cuh step by step (same pass order, same ping-pong flags), sequentially.
 #include <cstdlib>
 #include <cstring>
@@ -226,6 +227,55 @@ HT_API void ht_spawn_draws(const HtMap *m, int n, uint64_t *rng_state, const int
 HT_API void ht_pcg_bounded(int n, uint64_t *rng_state, uint32_t high_excl, int k, uint32_t *out) {
     for (int env = 0; env < n; env++)
         for (int j = 0; j < k; j++) out[(size_t)env * k + j] = tc_pcg_bounded(rng_state + (size_t)env * TC_RNG_N, high_excl);
+}
+
+// n Philox4x32-10 blocks: counters ctr [n,4], keys key [n,2] -> out [n,4]
+HT_API void ht_philox(int n, const uint32_t *ctr, const uint32_t *key, uint32_t *out) {
+    for (int i = 0; i < n; i++)
+        tc_philox4x32_10(ctr[4 * i], ctr[4 * i + 1], ctr[4 * i + 2], ctr[4 * i + 3], key[2 * i], key[2 * i + 1], out + 4 * i);
+}
+
+// the fill phase of tc_noise_blobs_kernel with its 256 threads replayed as one: inside the disc hw of radius rad at (x, y),
+// clipped to [H,W], dst |= sp (copy) or dst = 0
+static void ht_blob_fill(uint8_t *dst, const uint8_t *sp, int H, int W, int x, int y, int rad, bool copy, const int *hw) {
+    const int side = 2 * rad + 1;
+    for (int i = 0; i < side * side; i++) {
+        int ry = i / side - rad, rx = i % side - rad;
+        int h = hw[ry < 0 ? -ry : ry];
+        if (h < 0 || rx < -h || rx > h) continue;
+        int px = x + rx, py = y + ry;
+        if ((unsigned)px >= (unsigned)W || (unsigned)py >= (unsigned)H) continue;
+        size_t o = (size_t)py * W + px;
+        if (copy) dst[o] |= sp[o];
+        else dst[o] = 0;
+    }
+}
+
+// cv2.circle(img, (x, y), radius, 255, -1) on a zero img [H,W] through tc_circle_halfwidths and the kernel's fill (radius < 1024)
+HT_API void ht_circle(uint8_t *img, int H, int W, int x, int y, int radius) {
+    int hw[1024];
+    tc_circle_halfwidths(radius, hw);
+    std::vector<uint8_t> ones((size_t)H * W, 255);
+    ht_blob_fill(img, ones.data(), H, W, x, y, radius, true, hw);
+}
+
+// mirrors tc_noise_blobs_kernel over obs [n*n_cams, C, H, W] u8 in place (mask: optional, per env)
+HT_API void ht_noise_blobs(uint8_t *obs, int n, int n_cams, int C, int H, int W, uint64_t seed, uint32_t step, int n_blobs, int max_radius,
+                           int32_t env_index_offset, const uint8_t *mask) {
+    int hw[1024];
+    const size_t plane = (size_t)H * W;
+    for (int v = 0; v < n * n_cams; v++) {
+        const int env = v / n_cams, cam = v % n_cams;
+        if (mask && !mask[env]) continue;
+        uint8_t *base = obs + (size_t)v * C * plane;
+        for (int c = 0; c < C; c++)
+            for (int k = 0; k < n_blobs; k++) {
+                const TcBlobDraw d = tc_noise_draw((uint32_t)seed, (uint32_t)(seed >> 32), (uint32_t)env + (uint32_t)env_index_offset, step, c, k, cam,
+                                                   n_blobs, max_radius, H, W, C);
+                tc_circle_halfwidths(d.radius, hw);
+                if (!(d.copy && d.src == c)) ht_blob_fill(base + (size_t)c * plane, base + (size_t)d.src * plane, H, W, d.x, d.y, d.radius, d.copy != 0, hw);
+            }
+    }
 }
 
 // ---- visible-set tables (tc_cull.h): the camera pass of tc_render_env_kernel on the sub-graph of the camera's ground cell

@@ -1745,19 +1745,8 @@ __global__ void __launch_bounds__(TC_BEV_THREADS) tc_bev_kernel(const TcBevArgs 
 // ------------------------------------------------------------------------------------------------ blob noise
 // NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) on the device: per class, n_blobs filled circles that
 // either erase the class mask or OR in the pixels of a randomly chosen class, applied in the reference's order (classes
-// ascending, blobs in sequence, in place: a blob sees what earlier blobs did). The reference draws from the unseeded global
-// numpy RNG; here every draw is a pure function of (seed, global env index, step, class, blob) through Philox4x32-10, so
-// runs are reproducible and independent of the sharding. cv2.circle(..., -1) is the midpoint circle of tc_circle_filled.
-__host__ __device__ inline void tc_philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t *out) {
-    for (int r = 0; r < 10; r++) {
-        uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
-        uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1, n3 = (uint32_t)p0;
-        c0 = n0; c1 = n1; c2 = n2; c3 = n3;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-
+// ascending, blobs in sequence, in place: a blob sees what earlier blobs did). The draws (tc_noise_draw) and the disc
+// (tc_circle_halfwidths) are tc_core.cuh's, shared with the host test build's mirror ht_noise_blobs.
 struct TcNoiseArgs {
     int n_envs, n_cams, n_classes, H, W;
     int n_blobs, max_radius;
@@ -1777,22 +1766,10 @@ __global__ void __launch_bounds__(256) tc_noise_blobs_kernel(const TcNoiseArgs a
     for (int c = 0; c < a.n_classes; c++)
         for (int k = 0; k < a.n_blobs; k++) {
             if (tid == 0) {
-                uint32_t r[4];
-                tc_philox4x32_10((uint32_t)env + a.env_offset, a.step, (uint32_t)(c * a.n_blobs + k), (uint32_t)cam, a.seed_lo, a.seed_hi, r);
-                bx = (int)(r[0] % (uint32_t)a.W);
-                by = (int)(r[1] % (uint32_t)a.H);
-                brad = a.max_radius > 1 ? 1 + (int)(r[2] % (uint32_t)(a.max_radius - 1)) : 1;   // randint(1, max_radius)
-                bcopy = (r[3] & 0xffffu) < 19661u;                                               // p = 0.3
-                bsrc = (int)((r[3] >> 16) % (uint32_t)a.n_classes);
-                for (int i = 0; i <= brad; i++) hw[i] = -1;
-                int err = 0, dx = brad, dy = 0, plus = 1, minus = (brad << 1) - 1;
-                while (dx >= dy) {
-                    hw[dy] = max(hw[dy], dx);
-                    hw[dx] = max(hw[dx], dy);
-                    dy++; err += plus; plus += 2;
-                    int m = (err <= 0) - 1;
-                    err -= minus & m; dx += m; minus -= m & 2;
-                }
+                const TcBlobDraw d = tc_noise_draw(a.seed_lo, a.seed_hi, (uint32_t)env + a.env_offset, a.step, c, k, cam, a.n_blobs, a.max_radius,
+                                                   a.H, a.W, a.n_classes);
+                bx = d.x; by = d.y; brad = d.radius; bcopy = d.copy; bsrc = d.src;
+                tc_circle_halfwidths(d.radius, hw);
             }
             __syncthreads();
             const int x = bx, y = by, rad = brad, src = bsrc;

@@ -3,13 +3,16 @@ erase a class mask or OR in the pixels of a random class — as a device kernel 
 for the single-env drop-in. Same constructor arguments as the reference plus `seed`: the reference draws from numpy's
 unseeded global RNG, so there is no stream to reproduce; here the noise of (env, step, class, blob) is a pure function of
 the seed through Philox4x32-10 (contract in include/tinycarlo_b200.h), reproducible and independent of the GPU sharding.
-With a camera rig every view is noised: camera m draws with counter word 3 = m, so camera 0 gets the rig-less noise.
-Like the reference, constructing it sets `unwrapped.wrapped = True` and it only acts on the "classes" format."""
+With a camera rig every view is noised: camera m draws with counter word 3 = m, so camera 0 gets the rig-less noise. On a
+TinyCarloGroupedVecEnv each group's observation is noised with its own handle and env_index_offset, so the noise of an env
+depends on its global index only. Like the reference, constructing it sets `unwrapped.wrapped = True` and it only acts
+on the "classes" format."""
 import ctypes as C
 
 import torch
 
 from .. import _lib
+from ..grouped_env import TinyCarloGroupedVecEnv
 from ..gym_compat import Wrapper
 from .reward import _VecWrapper, _make
 
@@ -30,8 +33,10 @@ class _NoiseVec(_VecWrapper):
     def step(self, action):
         observation, reward, terminated, truncated, info = self.env.step(action)
         u = self.unwrapped
-        if u.observation_space_format == "classes" and not u.no_observation:
-            _apply(u, observation, self.seed, self.steps, self.n_blobs, self.max_radius)   # in place, like the reference
+        # a grouped env returns one observation tensor per group, each owned by that group's env
+        for e, obs in zip(u.envs, observation) if isinstance(u, TinyCarloGroupedVecEnv) else [(u, observation)]:
+            if e.observation_space_format == "classes" and not e.no_observation:
+                _apply(e, obs, self.seed, self.steps, self.n_blobs, self.max_radius)   # in place, like the reference
         self.steps += 1
         return observation, reward, terminated, truncated, info
 
