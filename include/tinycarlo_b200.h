@@ -127,8 +127,8 @@ TC_API int tc_create(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_env
  *                              renders for that camera row and that car state
  *   obs                        N*M frames in the handle's format, all of one resolution: u8 [N,M,C,H,W], RGB [N,M,H,W,3],
  *                              bits [N,M,C,ceil(H*W/32)], bf16 [N,M,C,H,W]
- *   masks                      of tc_reset, tc_render and tc_render_bev stay per env [N]: an env's mask selects all its views
- *   per-env outputs            state, TcOutputs except seg_*, flags, spawn draws and the BEV stay per env [N]
+ *   masks                      of tc_reset, tc_render, tc_render_bev and tc_render_lidar stay per env [N]: an env's mask selects all its views
+ *   per-env outputs            state, TcOutputs except seg_*, flags, spawn draws, the BEV and the range scan stay per env [N]
  *   per-view outputs           seg_count [N*M, C], seg_i32 [N*M, sumE, 4], the tc_debug_set_timeline buffer [N*M*C][10]
  *   tc_noise_blobs             obs [N*M, C, H, W]; Philox counter (env_index_offset + i, step, c * n_blobs + blob, m)
  *   tc_step_host_obs           obs_bytes covers all views
@@ -234,6 +234,43 @@ typedef struct {
 TC_API int tc_set_bev(TcHandle *h, const TcBevDesc *desc, uint8_t *dev_bev);
 /* Re-renders the BEV of the envs with dev_mask[i] != 0 (NULL = all) at the current state (after tc_set_state). */
 TC_API int tc_render_bev(TcHandle *h, const uint8_t *dev_mask, void *stream);
+
+/* Lidar-style range scan: R rays around every car, and per laneline class the distance along each ray to the first edge of
+ * that class. For env i with state x = sf[TC_SF_X], y = sf[TC_SF_Y], θ = sf[TC_SF_ROT] (rear axle, map metres, image-like
+ * y down), evaluated in float64, in exactly this order, with no FMA (the library is built with -fmad=false, the host build
+ * with -ffp-contract=off):
+ *
+ *   c = cos θ, s = sin θ                                   # device libm, like tc_bev_kernel
+ *   ox = x + (f*c - r*s);  oy = y + (f*s + r*c)            # origin: (f, r) = (forward, right) metres in the car frame
+ *   phi_j = (fov * ((j + 0.5) / R) - fov / 2) * (pi / 180) # host, j = 0..R-1: ray 0 leftmost, ascending to the right
+ *   a_j = cos(phi_j), b_j = sin(phi_j)                     # host glibc, uploaded by tc_set_lidar
+ *   dx = a_j*c - b_j*s;  dy = a_j*s + b_j*c                # the car's right is (-s, c), as in the BEV contract
+ *   for every edge (A, B) of class p:
+ *       ex = bx - ax; ey = by - ay; wx = ax - ox; wy = ay - oy
+ *       den = dx*ey - dy*ex
+ *       if den != 0:  t = (wx*ey - wy*ex) / den;  u = (wx*dy - wy*dx) / den
+ *                     hit iff t >= 0 and u >= 0 and u <= 1
+ *   out[i, p, j] = (float) min(max_range, min over hits of t)   # no hit: max_range; a zero distance is stored as +0.0
+ *
+ * Consequences: parallel and collinear edges (den == 0) and zero-length edges never hit. A non-finite state gives max_range
+ * on every ray, because every comparison is false. min is exact and order-free, so the kernel may visit edges in any order
+ * (unlike the BEV, whose draw order is fixed). "Right" means what it means in the BEV contract: (f, r) = (0, 1) is one metre
+ * to the car's right, and with fov < 360 ray 0 looks left of the heading and ray R-1 right of it. */
+typedef struct {
+    int32_t rays;                          /* R, 1..1024 */
+    double fov;                            /* degrees, (0, 360] */
+    double max_range;                      /* metres, finite, > 0 */
+    double origin_forward, origin_right;   /* metres from the rear axle, finite */
+} TcLidarDesc;
+/* Registers the scan description and a caller-owned device buffer float [N, C, R], which must stay alive (like the BEV's).
+ * Computes a_j, b_j on the host and uploads them to a handle-owned buffer (a set-up call: it synchronises). From then on
+ * tc_step / tc_step_f64 launch the scan right after the BEV (post-step, post-autoreset state), tc_reset scans the masked
+ * envs, and tc_render_lidar re-scans. The scan is per env: a camera rig changes nothing about it. dev_lidar NULL switches
+ * the scan off. A bad description fails with TC_ERR_INVALID; it is checked before the handle. */
+TC_API int tc_set_lidar(TcHandle *h, const TcLidarDesc *desc, float *dev_lidar);
+/* Re-scans the envs with dev_mask[i] != 0 (NULL = all) at the current state (after tc_set_state). TC_ERR_STATE without a
+ * scan set. */
+TC_API int tc_render_lidar(TcHandle *h, const uint8_t *dev_mask, void *stream);
 
 /* Number of kernel launches issued through this handle since creation (bench.py reports it). */
 TC_API int64_t tc_launch_count(const TcHandle *h);

@@ -161,6 +161,40 @@ def bev_params(config: Dict[str, Any], n_classes: int) -> Optional[Dict[str, Any
             "route": route, "format": fmt, "planes": planes}
 
 
+LIDAR_MAX_RAYS = 1024             # TC_LIDAR_RPT * TC_LIDAR_THREADS: rays of one scan
+
+
+def lidar_params(config: Dict[str, Any], n_classes: int) -> Optional[Dict[str, Any]]:
+    """The optional `lidar` section (an extension: a range scan of R rays around every car, per laneline class the distance
+    to the first edge along each ray, include/tinycarlo_b200.h tc_set_lidar) with its defaults, or None when the config has
+    none. Raises ValueError for a bad section."""
+    lidar = config.get("lidar")
+    if lidar is None:
+        return None
+    if not isinstance(lidar, dict):
+        raise ValueError("lidar must be a mapping")
+    unknown = sorted(set(lidar) - {"rays", "fov", "max_range", "origin"})
+    if unknown:
+        raise ValueError(f"lidar: unknown keys {unknown} (allowed: rays, fov, max_range, origin)")
+
+    def finite(v):
+        return isinstance(v, numbers.Real) and not isinstance(v, bool) and math.isfinite(v)
+    rays = lidar.get("rays", 64)
+    if not (isinstance(rays, numbers.Integral) and not isinstance(rays, bool) and 1 <= rays <= LIDAR_MAX_RAYS):
+        raise ValueError(f"lidar.rays must be an integer in 1..{LIDAR_MAX_RAYS}, got {rays!r}")
+    fov = lidar.get("fov", 360)
+    if not (finite(fov) and 0 < fov <= 360):
+        raise ValueError(f"lidar.fov must be a number of degrees in (0, 360], got {fov!r}")
+    max_range = lidar.get("max_range", 0.5)
+    if not (finite(max_range) and max_range > 0):
+        raise ValueError(f"lidar.max_range must be a finite number > 0 (metres), got {max_range!r}")
+    origin = lidar.get("origin", [0.0, 0.0])
+    if not (isinstance(origin, (list, tuple)) and len(origin) == 2 and all(finite(v) for v in origin)):
+        raise ValueError(f"lidar.origin must be [forward, right] with finite numbers (metres), got {origin!r}")
+    return {"rays": int(rays), "fov": float(fov), "max_range": float(max_range), "origin": [float(origin[0]), float(origin[1])],
+            "classes": int(n_classes)}
+
+
 # ------------------------------------------------------------------------------------------------ shipped configurations
 # The car / camera sections of examples/config_knuffingen.yaml and config_simple_layout.yaml, and the spawn points they
 # list, as dict configs over the maps bundled in tinycarlo_b200/maps/ (benchmarks, tools and tests build theirs from these).

@@ -115,6 +115,9 @@ struct TcHandle {
     TcBevDesc bev{};            // bird's-eye view (tc_set_bev): off while bev_out is NULL
     uint8_t *bev_out = nullptr; // caller-owned
     int bev_planes = 0, bev_plane_words = 0;
+    TcLidarDesc lidar{};          // range scan (tc_set_lidar): off while lidar_out is NULL
+    float *lidar_out = nullptr;   // caller-owned [N,C,R]
+    double *d_lidar_ab = nullptr; // handle-owned [1024][2]: (cos phi_j, sin phi_j)
     // optional per-kernel CUDA-event timing (tc_profile_begin/end)
     bool profiling = false;
     int prof_cap = 0, prof_used = 0; // step slots
@@ -737,6 +740,54 @@ int tc_render_bev(TcHandle *h, const uint8_t *dev_mask, void *stream) {
     return tc_launch_bev(h, dev_mask, (cudaStream_t)stream);
 }
 
+static int tc_launch_lidar(TcHandle *h, const uint8_t *mask, cudaStream_t st) {
+    TcLidarArgs a;
+    a.blob = h->d_blob; a.layout = h->layout; a.sf = h->d_sf; a.ab = h->d_lidar_ab;
+    a.g.rays = h->lidar.rays; a.g.fov = h->lidar.fov; a.g.max_range = h->lidar.max_range;
+    a.g.fwd = h->lidar.origin_forward; a.g.right = h->lidar.origin_right;
+    a.n_envs = h->n_envs; a.mask = mask; a.out = h->lidar_out;
+    const int threads = std::min(TC_LIDAR_THREADS, (h->lidar.rays + 31) / 32 * 32);
+    tc_lidar_kernel<<<h->n_envs, threads, 0, st>>>(a);
+    h->launches++;
+    TC_CUDA(cudaGetLastError());
+    return TC_OK;
+}
+
+int tc_set_lidar(TcHandle *h, const TcLidarDesc *desc, float *dev_lidar) {
+    if (dev_lidar) {   // the description first, so that it can be checked without a device
+        if (!desc) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: null description");
+        const TcLidarDesc &d = *desc;
+        if (d.rays < 1 || d.rays > TC_LIDAR_RPT * TC_LIDAR_THREADS) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: rays must be in 1..1024");
+        if (!(d.fov > 0 && d.fov <= 360)) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: fov must be in (0, 360] degrees");
+        if (!(std::isfinite(d.max_range) && d.max_range > 0)) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: max_range must be finite and > 0");
+        if (!std::isfinite(d.origin_forward) || !std::isfinite(d.origin_right)) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: origin must be finite");
+    }
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_set_lidar: null handle");
+    if (!dev_lidar) {
+        h->lidar_out = nullptr;
+        return TC_OK;
+    }
+    const TcLidarDesc &d = *desc;
+    std::vector<double> ab(2 * (size_t)d.rays);
+    for (int j = 0; j < d.rays; j++) {
+        const double phi = (d.fov * ((j + 0.5) / d.rays) - d.fov / 2) * (TC_PI / 180.0);
+        ab[2 * j] = cos(phi);
+        ab[2 * j + 1] = sin(phi);
+    }
+    TC_CUDA(cudaSetDevice(h->device));
+    if (!h->d_lidar_ab) TC_TRY(tc_dev_alloc(h, &h->d_lidar_ab, 2 * TC_LIDAR_RPT * TC_LIDAR_THREADS));
+    TC_CUDA(cudaMemcpy(h->d_lidar_ab, ab.data(), ab.size() * sizeof(double), cudaMemcpyHostToDevice));
+    h->lidar = d; h->lidar_out = dev_lidar;
+    return TC_OK;
+}
+
+int tc_render_lidar(TcHandle *h, const uint8_t *dev_mask, void *stream) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_render_lidar: null handle");
+    if (!h->lidar_out) return tc_fail(TC_ERR_STATE, "tc_render_lidar: no scan set (tc_set_lidar)");
+    TC_CUDA(cudaSetDevice(h->device));
+    return tc_launch_lidar(h, dev_mask, (cudaStream_t)stream);
+}
+
 int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_nodes, const TcOutputs *outs, void *stream) {
     if (!h) return tc_fail(TC_ERR_INVALID, "tc_reset: null handle");
     if (!dev_spawn_nodes && !h->rng) return tc_fail(TC_ERR_STATE, "tc_reset: no spawn nodes given and no spawn streams set (tc_set_spawn_rng)");
@@ -747,6 +798,7 @@ int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_node
     if (outs && (outs->obs || outs->seg_count || outs->seg_i32))
         TC_TRY(tc_launch_render(h, tc_view_mask(h, dev_mask), outs->obs, h->obs_format, outs->seg_count, outs->seg_i32, st));
     if (h->bev_out) TC_TRY(tc_launch_bev(h, dev_mask, st));
+    if (h->lidar_out) TC_TRY(tc_launch_lidar(h, dev_mask, st));
     return TC_OK;
 }
 
@@ -782,6 +834,7 @@ static int tc_step_impl(TcHandle *h, const float *dev_car_control, const double 
         h->prof_used++;
     }
     if (h->bev_out) TC_TRY(tc_launch_bev(h, nullptr, st));
+    if (h->lidar_out) TC_TRY(tc_launch_lidar(h, nullptr, st));
     return TC_OK;
 }
 

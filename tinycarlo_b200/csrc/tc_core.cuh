@@ -1157,3 +1157,88 @@ TC_HD bool tc_bev_segment(const TcTrackTables &tt, const TcBevGeom &g, double x,
     const int64_t m = g.thickness + 1, r = (int64_t)g.W - 1 + m, b = (int64_t)g.H - 1 + m;
     return !((p[0] < -m && p[2] < -m) || (p[1] < -m && p[3] < -m) || (p[0] > r && p[2] > r) || (p[1] > b && p[3] > b));
 }
+
+// ------------------------------------------------------------------------------------------------ range scan
+// The range-scan contract (include/tinycarlo_b200.h, tc_set_lidar), float64 in the contract's order (no FMA contraction).
+struct TcLidarGeom {
+    int rays;
+    double fov, max_range, fwd, right;
+};
+
+// origin O of the rays: (fwd, right) metres in the car frame
+TC_HD void tc_lidar_origin(const TcLidarGeom &g, double x, double y, double c, double s, double &ox, double &oy) {
+    ox = x + (g.fwd * c - g.right * s);
+    oy = y + (g.fwd * s + g.right * c);
+}
+// direction of ray j from the host's (a_j, b_j) = (cos phi_j, sin phi_j)
+TC_HD void tc_lidar_dir(double a, double b, double c, double s, double &dx, double &dy) {
+    dx = a * c - b * s;
+    dy = a * s + b * c;
+}
+
+// true when RN(n / den) is certainly < 0 (not -0.0, which counts as >= 0): opposite signs, |n| >= 2^-1000 and |den| <= 2^70 make
+// |n / den| >= 2^-1070, far above the 2^-1075 below which the quotient rounds to -0.0. NaN operands are never rejected here.
+TC_HD bool tc_lidar_negative(double n, double den) {
+    return (n < 0) != (den < 0) && fabs(n) >= 0x1p-1000 && fabs(den) <= 0x1p70;
+}
+// true when RN(un / den) is certainly > 1: same signs, |den| >= 2^-1000 (the product below is not subnormal) and
+// |un| > RN(|den| * (1 + 2^-20)) >= |den| * (1 + 2^-20) * (1 - 2^-53) > |den| * (1 + 2^-53): the quotient lies above the midpoint
+// between 1 and its successor, so it rounds above 1. A quotient that rounds to exactly 1.0 is never rejected.
+TC_HD bool tc_lidar_above_one(double un, double den) {
+    const double ad = fabs(den);
+    return (un < 0) == (den < 0) && ad >= 0x1p-1000 && fabs(un) > ad * (1.0 + 0x1p-20);
+}
+
+// one ray (dx, dy) against one staged edge (tc_lidar_stage: ex, ey, wx, wy, tn = wx*ey - wy*ex): true and t for a hit of the
+// contract. The division-free rejections above only drop pairs whose quotients provably fail the contract's tests, so the
+// result is the contract's bit for bit; u is divided before t, and t only for the pairs whose u passes.
+TC_HD bool tc_lidar_hit(double dx, double dy, double ex, double ey, double wx, double wy, double tn, double &t) {
+    const double den = dx * ey - dy * ex;
+    if (den == 0) return false;
+    const double un = wx * dy - wy * dx;
+    if (tc_lidar_negative(tn, den) || tc_lidar_negative(un, den) || tc_lidar_above_one(un, den)) return false;
+    const double u = un / den;
+    if (!(u >= 0 && u <= 1)) return false;
+    t = tn / den;
+    return t >= 0;
+}
+
+// Stages edge (A, B) for origin O and heading (c, s): st = {ex, ey, wx, wy, tn}. Returns false when no ray of the fan can hit
+// the edge with t <= max_range (the cull), true otherwise. Conservative, including rounding:
+//  - kept: every edge whose bounding box meets the square of half-size M = max_range * (1 + 2^-10) + 2^-50 * (|ox| + |oy|)
+//    around O. The rounding of ox +- M costs less than 2^-51 * (M + |ox| + |oy|), so the square tested contains the one of
+//    half-size max_range * (1 + 2^-11) whatever the origin's magnitude.
+//  - an edge outside that square needs, for a hit with t <= max_range, the computed intersection t*d (|d| = 1 within a few
+//    ulp) to be more than g = max_range * 2^-12 from the edge point A + u*e. Write z = (A + u*e - O) - t*d. The rounding of
+//    den, tn, un and of the two divisions bounds |cross(z, d)| by ~5 * 2^-53 * (|w| + |e|) and |cross(z, e)| by
+//    ~5 * 2^-53 * |e| * (|w| + max_range) (exact identities: cross(w, e) = t*den, cross(w, d) = u*den). With |z| >= g,
+//    the component of z along d is >= g / 2, so the sine of the angle between the edge and the ray is at most
+//    tol = 2^-34 * (2|w| + max_range + |e|) / max_range (16x that bound), and O lies within max_range + 2^-48 * (|w| +
+//    max_range) of the edge's line. Such an edge - far away, and parallel to a ray to within tol - is kept; every other
+//    edge outside the square is dropped. The 1-norms below bound the 2-norms from above.
+//  - zero-length edges (den == 0 for every ray) are dropped; non-finite or huge / tiny magnitudes are kept.
+TC_HD bool tc_lidar_stage(const TcLidarGeom &g, double ox, double oy, double c, double s, double ax, double ay, double bx, double by,
+                          double *st) {
+    const double ex = bx - ax, ey = by - ay, wx = ax - ox, wy = ay - oy;
+    const double tn = wx * ey - wy * ex;
+    st[0] = ex; st[1] = ey; st[2] = wx; st[3] = wy; st[4] = tn;
+    const double R = g.max_range, M = R * (1.0 + 0x1p-10) + 0x1p-50 * (fabs(ox) + fabs(oy));
+    const double x0 = ax < bx ? ax : bx, x1 = ax < bx ? bx : ax, y0 = ay < by ? ay : by, y1 = ay < by ? by : ay;
+    if (x0 <= ox + M && x1 >= ox - M && y0 <= oy + M && y1 >= oy - M) return true;
+    if (ex == 0 && ey == 0) return false;
+    const double w1 = fabs(wx) + fabs(wy), e1 = fabs(ex) + fabs(ey);
+    if (!(w1 <= 0x1p400 && e1 <= 0x1p400 && e1 >= 0x1p-400 && R >= 0x1p-400 && R <= 0x1p400)) return true;   // also NaN
+    if (fabs(tn) > (R * (1.0 + 0x1p-40) + 0x1p-48 * (w1 + R + e1)) * e1 * (1.0 + 0x1p-40)) return false;   // line too far from O
+    const double tol = 0x1p-34 * (2.0 * w1 + R + e1) / R;
+    if (tol >= 0.25) return true;
+    // angle of the edge in the car frame against the ray angles phi_j, lines taken modulo 180 degrees
+    const double psi = atan2(ey * c - ex * s, ex * c + ey * s) * (180.0 / TC_PI);
+    const double slack = (2.0 * tol + 0x1p-40) * (180.0 / TC_PI);
+    for (int k = -2; k <= 2; k++) {
+        const double a = psi + 180.0 * k;
+        double j = rint((a + g.fov / 2) / g.fov * g.rays - 0.5);
+        j = j < 0 ? 0 : (j > g.rays - 1 ? g.rays - 1 : j);
+        if (fabs(a - (g.fov * ((j + 0.5) / g.rays) - g.fov / 2)) <= slack) return true;
+    }
+    return false;
+}

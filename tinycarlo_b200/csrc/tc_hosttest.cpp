@@ -217,6 +217,49 @@ HT_API void ht_bev(const HtMap *m, int n, const double *sf, const int32_t *si, c
     }
 }
 
+// mirrors tc_lidar_kernel for n envs at state rows sf [n,TC_SF_N]: out_f64 [n,C,R] is the scan in float64, before the float32
+// cast (cos / sin of the heading and of the ray angles are the host libm's, as tc_set_lidar computes the latter)
+HT_API void ht_lidar(const HtMap *m, int n, const double *sf, const TcLidarDesc *d, double *out_f64) {
+    const TcTrackTables tt = tc_track_tables(m->pk.blob.data(), m->pk.L);
+    const TcLidarGeom g = {d->rays, d->fov, d->max_range, d->origin_forward, d->origin_right};
+    const int C = m->C, R = d->rays;
+    std::vector<double> a(R), b(R), best(R);
+    for (int j = 0; j < R; j++) {
+        const double phi = (d->fov * ((j + 0.5) / R) - d->fov / 2) * (TC_PI / 180.0);
+        a[j] = cos(phi);
+        b[j] = sin(phi);
+    }
+    for (int env = 0; env < n; env++) {
+        const double *s = sf + (size_t)env * TC_SF_N;
+        const double c = cos(s[TC_SF_ROT]), sn = sin(s[TC_SF_ROT]);
+        double ox, oy;
+        tc_lidar_origin(g, s[TC_SF_X], s[TC_SF_Y], c, sn, ox, oy);
+        for (int p = 0; p < C; p++) {
+            const double *nodes = tt.ll_nodes + 2 * tt.ll_node_off[p];
+            for (int j = 0; j < R; j++) best[j] = g.max_range;
+            for (int i = tt.ll_edge_off[p]; i < tt.ll_edge_off[p + 1]; i++) {
+                const int32_t n0 = tt.ll_edges[2 * i], n1 = tt.ll_edges[2 * i + 1];
+                double st[5];
+                if (!tc_lidar_stage(g, ox, oy, c, sn, nodes[2 * n0], nodes[2 * n0 + 1], nodes[2 * n1], nodes[2 * n1 + 1], st)) continue;
+                for (int j = 0; j < R; j++) {
+                    double dx, dy, t;
+                    tc_lidar_dir(a[j], b[j], c, sn, dx, dy);
+                    if (tc_lidar_hit(dx, dy, st[0], st[1], st[2], st[3], st[4], t) && t < best[j]) best[j] = t;
+                }
+            }
+            double *o = out_f64 + ((size_t)env * C + p) * R;
+            for (int j = 0; j < R; j++) o[j] = best[j] == 0 ? 0.0 : best[j];
+        }
+    }
+}
+
+// the cull of the scan (tc_lidar_stage) for one edge: 1 kept, 0 dropped
+HT_API int ht_lidar_keep(const TcLidarDesc *d, double ox, double oy, double c, double s, double ax, double ay, double bx, double by) {
+    const TcLidarGeom g = {d->rays, d->fov, d->max_range, d->origin_forward, d->origin_right};
+    double st[5];
+    return tc_lidar_stage(g, ox, oy, c, s, ax, ay, bx, by, st) ? 1 : 0;
+}
+
 // the reset paths' spawn draws (tc_spawn_draw): k consecutive draws of n env streams, states advanced in place
 HT_API void ht_spawn_draws(const HtMap *m, int n, uint64_t *rng_state, const int32_t *spawn_points, int n_spawn_points, int k, int32_t *out) {
     TcTrackTables t = tc_track_tables(m->pk.blob.data(), m->pk.L);

@@ -1742,6 +1742,84 @@ __global__ void __launch_bounds__(TC_BEV_THREADS) tc_bev_kernel(const TcBevArgs 
     else tc_store_plane_sparse<TC_BEV_THREADS>(a.out + (size_t)env * npx, npx, plane, drew != 0);
 }
 
+// ------------------------------------------------------------------------------------------------ range scan
+// tc_set_lidar's contract (include/tinycarlo_b200.h). A block per env, classes in turn: the block walks the class's edges
+// straight from the map tables, one edge per thread, stages the ones the conservative cull keeps (tc_lidar_stage) in a
+// shared-memory tile (order-free: the minimum does not depend on it), then every thread runs its rays (j = tid + k * blockDim,
+// at most TC_LIDAR_RPT of them) over the tile (tc_lidar_hit) and keeps a running minimum per ray. A class with more edges than
+// threads takes several tiles, so any map size works. After the class, out[env, p, j] is stored: consecutive threads write
+// consecutive floats. The block has as many threads as rays, rounded up to a warp, at most TC_LIDAR_THREADS.
+#define TC_LIDAR_THREADS 256
+#define TC_LIDAR_RPT 4             // rays per thread: TC_LIDAR_RPT * TC_LIDAR_THREADS = 1024 = the largest R tc_set_lidar accepts
+struct TcLidarArgs {
+    const unsigned char *blob;     // map tables (tc_track_tables)
+    TcBlobLayout layout;
+    const double *sf;              // [N,TC_SF_N]
+    const double *ab;              // [R][2]: (cos phi_j, sin phi_j) from the host
+    TcLidarGeom g;
+    int n_envs;
+    const uint8_t *mask;           // optional, per env
+    float *out;                    // [N,C,R]
+};
+
+__global__ void __launch_bounds__(TC_LIDAR_THREADS) tc_lidar_kernel(const TcLidarArgs a) {
+    __shared__ double tile[5][TC_LIDAR_THREADS];
+    __shared__ int n_tile;
+    const int env = blockIdx.x, tid = threadIdx.x, nt = blockDim.x, R = a.g.rays;
+    if (a.mask && !a.mask[env]) return;
+    const TcTrackTables tt = tc_track_tables(a.blob, a.layout);
+    const double *sf = a.sf + (size_t)env * TC_SF_N;
+    const double x = sf[TC_SF_X], y = sf[TC_SF_Y], c = cos(sf[TC_SF_ROT]), s = sin(sf[TC_SF_ROT]);
+    double ox, oy;
+    tc_lidar_origin(a.g, x, y, c, s, ox, oy);
+    double dx[TC_LIDAR_RPT], dy[TC_LIDAR_RPT];
+#pragma unroll
+    for (int k = 0; k < TC_LIDAR_RPT; k++) {
+        const int j = tid + k * nt;
+        dx[k] = dy[k] = 0;
+        if (j < R) tc_lidar_dir(a.ab[2 * j], a.ab[2 * j + 1], c, s, dx[k], dy[k]);
+    }
+    const int C = tt.n_classes;
+    for (int p = 0; p < C; p++) {
+        const double *nodes = tt.ll_nodes + 2 * tt.ll_node_off[p];
+        const int e0 = tt.ll_edge_off[p], e1 = tt.ll_edge_off[p + 1];
+        double best[TC_LIDAR_RPT];
+#pragma unroll
+        for (int k = 0; k < TC_LIDAR_RPT; k++) best[k] = a.g.max_range;
+        for (int base = e0; base < e1; base += nt) {   // uniform trip count: the barriers below are reached by every thread
+            if (tid == 0) n_tile = 0;
+            __syncthreads();
+            const int i = base + tid;
+            if (i < e1) {
+                const int32_t n0 = tt.ll_edges[2 * i], n1 = tt.ll_edges[2 * i + 1];
+                double st[5];
+                if (tc_lidar_stage(a.g, ox, oy, c, s, nodes[2 * n0], nodes[2 * n0 + 1], nodes[2 * n1], nodes[2 * n1 + 1], st)) {
+                    const int slot = atomicAdd(&n_tile, 1);
+#pragma unroll
+                    for (int q = 0; q < 5; q++) tile[q][slot] = st[q];
+                }
+            }
+            __syncthreads();
+            const int n = n_tile;
+            for (int e = 0; e < n; e++) {
+                const double ex = tile[0][e], ey = tile[1][e], wx = tile[2][e], wy = tile[3][e], tn = tile[4][e];
+#pragma unroll
+                for (int k = 0; k < TC_LIDAR_RPT; k++) {
+                    double t;
+                    if (tid + k * nt < R && tc_lidar_hit(dx[k], dy[k], ex, ey, wx, wy, tn, t) && t < best[k]) best[k] = t;
+                }
+            }
+            __syncthreads();   // the next tile reuses the slots
+        }
+        float *o = a.out + ((size_t)env * C + p) * R;
+#pragma unroll
+        for (int k = 0; k < TC_LIDAR_RPT; k++) {
+            const int j = tid + k * nt;
+            if (j < R) o[j] = best[k] == 0 ? 0.0f : (float)best[k];   // t = -0.0 is a hit at distance +0.0
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ blob noise
 // NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) on the device: per class, n_blobs filled circles that
 // either erase the class mask or OR in the pixels of a randomly chosen class, applied in the reference's order (classes

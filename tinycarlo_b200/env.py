@@ -176,6 +176,8 @@ class TinyCarloEnv(gc.Env):
                 "laneline_distances": dist, "local_path": local_path, "velocity": vel}
         if v.bev is not None:   # the config's `bev` section (an extension): this env's bird's-eye view
             info["bev"] = v.bev[0].cpu().numpy()
+        if v.lidar is not None:   # the config's `lidar` section (an extension): this env's range scan [C, R]
+            info["lidar"] = v.lidar[0].cpu().numpy()
         return info
 
     def reset(self, seed: Optional[int] = None, options: Optional[Any] = None) -> Tuple[np.ndarray, Dict[str, Any]]:

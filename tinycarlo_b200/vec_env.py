@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from .camera_params import camera_row, view_rows
-from .config import LINE_THICKNESS_MAX, bev_params, camera_params, camera_rig, car_param_row, load_config, resolve_map_path, sim_params
+from .config import LINE_THICKNESS_MAX, bev_params, camera_params, lidar_params, camera_rig, car_param_row, load_config, resolve_map_path, sim_params
 from .maptables import MapTables
 from .spawn import spawn_stream_states
 
@@ -120,6 +120,15 @@ class TinyCarloVecEnv:
                 bdesc = _lib.TcBevDesc(bh, bw, b["pixel_per_meter"], b["car_pixel"][0], b["car_pixel"][1], b["line_thickness"], int(b["route"]),
                                        _lib.TC_OBS_CLASSES_BITS if bits else _lib.TC_OBS_CLASSES)
                 _lib.check(self._L.tc_set_bev(self._h, C.byref(bdesc), _ptr(self.bev)), "tc_set_bev")
+            # range scan (config section `lidar`, tc_set_lidar): float32 [N,C,R] metres, rewritten by every step() / reset()
+            # whatever no_observation says; None without the section
+            self.lidar_cfg = lidar_params(self.config, Cn)
+            self.lidar = None
+            if self.lidar_cfg is not None:
+                li = self.lidar_cfg
+                self.lidar = torch.zeros((N, Cn, li["rays"]), dtype=torch.float32, device=dev)
+                ldesc = _lib.TcLidarDesc(li["rays"], li["fov"], li["max_range"], li["origin"][0], li["origin"][1])
+                _lib.check(self._L.tc_set_lidar(self._h, C.byref(ldesc), _ptr(self.lidar)), "tc_set_lidar")
             self._spawn_nodes = torch.full((N,), -1, dtype=torch.int32, device=dev)   # node of each env's latest reset
             self._mask_all = torch.ones(N, dtype=torch.uint8, device=dev)
         self._outs = self._make_outputs(with_obs=True)
@@ -325,6 +334,8 @@ class TinyCarloVecEnv:
                 "nearest_edge": o["nearest_edge"], "local_path_nodes": o["local_path_nodes"], "path_len": o["path_len"]}
         if self.bev is not None:
             info["bev"] = self.bev
+        if self.lidar is not None:
+            info["lidar"] = self.lidar
         return info
 
     def reset(self, seed: Optional[int] = None, mask: Optional[torch.Tensor] = None, spawn_nodes: Optional[torch.Tensor] = None):
@@ -484,6 +495,15 @@ class TinyCarloVecEnv:
             _lib.check(self._L.tc_render_bev(self._h, _ptr(m), self._stream()), "tc_render_bev")
         return self.bev
 
+    def render_lidar(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Re-scan self.lidar (the config's `lidar` section) at the current poses for the envs in `mask` (None = all)."""
+        if self.lidar is None:
+            raise ValueError("render_lidar: the config has no `lidar` section")
+        with torch.cuda.device(self.device):
+            m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            _lib.check(self._L.tc_render_lidar(self._h, _ptr(m), self._stream()), "tc_render_lidar")
+        return self.lidar
+
     def render_obs(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Re-render self.obs (all views) at the current poses (after load_state_dict / set_camera_params); mask is per env."""
         with torch.cuda.device(self.device):
@@ -524,6 +544,8 @@ class TinyCarloVecEnv:
         self.render_obs()
         if self.bev is not None:
             self.render_bev()
+        if self.lidar is not None:
+            self.render_lidar()
 
     def load_state_dict(self, state: Dict[str, torch.Tensor]):
         with torch.cuda.device(self.device):
