@@ -23,6 +23,8 @@
  *   tc_noise_blobs         NoiseObservationWrapper.observation (tinycarlo/wrapper/observation.py:14-27) with a counter-based RNG
  *   tc_step_host           the same step driven with HOST buffers (pinned or pageable): actions are copied in and the
  *                          scalar results copied out inside the call; used for the end-to-end measurement
+ *   tc_set_route           no counterpart (the reference has no task beyond lane keeping): a navigation goal per car with
+ *                          the route's next maneuver, distance and progress (TcRouteDesc)
  *
  * Conventions: every function returns 0 on success or a negative TcError; tc_last_error() gives the message of the
  * last failure on the calling thread. Pointers named dev_* are CUDA device pointers on the handle's device, host_*
@@ -271,6 +273,75 @@ TC_API int tc_set_lidar(TcHandle *h, const TcLidarDesc *desc, float *dev_lidar);
 /* Re-scans the envs with dev_mask[i] != 0 (NULL = all) at the current state (after tc_set_state). TC_ERR_STATE without a
  * scan set. */
 TC_API int tc_render_lidar(TcHandle *h, const uint8_t *dev_mask, void *stream);
+
+/* Navigation goals: a destination per car on the lanepath graph, with the route's next maneuver, the distance left and the
+ * progress along it, computed on the device after every step and reset.
+ *
+ * Edge transitions. A car that tracks lanepath edge e = (n0, n1) and holds maneuver m moves on to the edge that
+ * tc_find_local_path_given picks:
+ *
+ *   T(e, m) = next_edge[tc_pick_edge(t, n1, tc_clip_angle(lp_orient[e] + m*pi/2), next_edge, next_off[n1], next_off[n1+1], true)]
+ *
+ * for m in {0, 1, 3}; there is no transition when the pick returns -1 (tc_pick_edge filters self-loops from the orientation
+ * list but indexes the unfiltered list, and a node with one successor returns it unfiltered: both kept). Routes use no
+ * u-turns (m = 2) and assume forward driving.
+ *
+ * Route table. goals[0..G-1] are the candidate goal nodes. For candidate k, with L(e) = tc_dist of the edge's two nodes in
+ * float64:
+ *   D_k(e) = 0                                             if n1(e) == goals[k]
+ *   D_k(e) = min over m in {0, 1, 3} of L(T(e,m)) + D_k(T(e,m))   otherwise, each sum rounded once in float64
+ *   D_k(e) = +inf                                          when no transition leads to the goal
+ * cmd_k(e) is the smallest m attaining the minimum, -1 when D_k(e) is 0 or +inf. Dijkstra backwards from the goal computes
+ * this fixed point (the rounded sum is monotone and never below D). The table is a pure function of the map tables and the
+ * goal list: goal-major float64 D [G][Q] and int8 cmd [G][Q], built on the host by tc_set_route and uploaded once.
+ *
+ * Per env, at the post-step state: pe0 = si[TC_SI_PATH_EDGES], pn1 = si[TC_SI_PATH_NODES + 1], the front axle
+ * (fx, fy) = sf[TC_SF_FRONT_X], sf[TC_SF_FRONT_Y], and the goal index k (the env has a tracked edge when path_len > 0,
+ * 0 <= pe0 < Q and pn0, pn1 are valid nodes; it has a goal when 0 <= k < G):
+ *   command  = cmd_k(pe0)                                              (-1 without a tracked edge or goal)
+ *   distance = tc_dist(fx, fy, node pn1) + D_k(pe0) in float64, stored as float; +inf when D_k(pe0) is +inf, without a
+ *              tracked edge or without a goal (NaN when the front axle is NaN and a route exists)
+ *   reached  = pn1 == goals[k] && tc_dist(fx, fy, goal node) <= reach_radius   (a node on the opposite lane, or the spawn
+ *              node behind the car, does not count)
+ *   progress = prev_distance - distance when both are finite, else 0; prev_distance (float64 per env) then becomes distance
+ *
+ * Goal draws. The env's valid goals are the candidates k, in list order, with D_k(pe0) finite and not reached at the current
+ * pose. The draw is valid[j] with j = tc_pcg_bounded(len(valid)) (one bounded draw, no redraw loop) on the env's goal stream,
+ * a second PCG64 stream per env in the TC_RNG_* row layout: numpy's Generator(PCG64(SeedSequence(seed + env_index_offset +
+ * i).spawn(1)[0])). Without a valid goal or a tracked edge nothing is drawn and the goal is -1. Draws happen for every env
+ * tc_reset selects, for every env a step autoresets (the was-reset mask) and, with TC_ROUTE_RESAMPLE, right after a goal is
+ * reached. After a draw progress is 0 and prev_distance is the new goal's distance, except on the step a goal is reached:
+ * there progress is measured to the old goal and reached is 1, while goal, command and distance already refer to the new
+ * one. With TC_ROUTE_TERMINATE a reaching step ORs 1 into the step's terminated output and the autoreset done flag, whatever
+ * tc_set_wrapped says, and keeps the goal until the autoreset draws the next one. The default reward is untouched. */
+enum { TC_ROUTE_RESAMPLE = 0, TC_ROUTE_TERMINATE = 1 };
+typedef struct {
+    int32_t n_goals;          /* G, 1..4096 */
+    const int32_t *goals;     /* HOST [G]: lanepath node ids, each the end node of some lanepath edge */
+    double reach_radius;      /* metres, finite, >= 0 */
+    int32_t on_reach;         /* TC_ROUTE_RESAMPLE or TC_ROUTE_TERMINATE */
+} TcRouteDesc;
+/* Per-env device outputs of the navigation goals, rewritten for every env a step or an update touches. */
+typedef struct {
+    int32_t *goal;            /* [N] goal node (-1: none) */
+    float *goal_position;     /* [N,2] its lp_nodes coordinates (NaN: none) */
+    int32_t *command;         /* [N] maneuver that keeps the car on its route (0 straight, 1 right, 3 left; -1 none) */
+    float *distance;          /* [N] metres along the route */
+    float *progress;          /* [N] metres gained since the previous step */
+    uint8_t *reached;         /* [N] */
+} TcRouteOutputs;
+/* Registers the goals, builds the route table (a set-up call: it synchronises the device) and the caller-owned device buffers,
+ * which must stay alive: dev_goal_rng uint64 [N, TC_RNG_N] goal streams, dev_goal_index int32 [N] (index into goals, -1 none),
+ * dev_prev_distance float64 [N], and every pointer of *outs. From then on tc_step / tc_step_f64 launch tc_route_kernel after
+ * the range scan and tc_reset launches it for the masked envs. With autoreset on and no tc_set_reset_mask buffer the handle
+ * keeps a was-reset mask of its own. desc NULL switches the feature off. The description is checked before the handle
+ * (TC_ERR_INVALID): 1 <= G <= 4096, goals non-NULL, reach_radius finite and >= 0, on_reach 0 or 1; then every goal must be a
+ * node in range with a predecessor (otherwise it can never be pn1), and the table G * Q * 9 bytes at most 256 MiB. */
+TC_API int tc_set_route(TcHandle *h, const TcRouteDesc *desc, uint64_t *dev_goal_rng, int32_t *dev_goal_index,
+                        double *dev_prev_distance, const TcRouteOutputs *outs);
+/* For the envs with dev_mask[i] != 0 (NULL = all): draw = 1 draws new goals; draw = 0 recomputes the outputs at the current
+ * state and goal index with progress 0 (after tc_set_state, or after the caller wrote goal indices). TC_ERR_STATE without goals. */
+TC_API int tc_update_route(TcHandle *h, const uint8_t *dev_mask, int32_t draw, void *stream);
 
 /* Number of kernel launches issued through this handle since creation (bench.py reports it). */
 TC_API int64_t tc_launch_count(const TcHandle *h);

@@ -41,6 +41,17 @@ class TcLidarDesc(C.Structure):
                 ("origin_right", C.c_double)]
 
 
+class TcRouteDesc(C.Structure):
+    _fields_ = [("n_goals", C.c_int32), ("goals", C.c_void_p), ("reach_radius", C.c_double), ("on_reach", C.c_int32)]
+
+
+ROUTE_OUTPUT_FIELDS = ["goal", "goal_position", "command", "distance", "progress", "reached"]
+
+
+class TcRouteOutputs(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in ROUTE_OUTPUT_FIELDS]
+
+
 OUTPUT_FIELDS = ["obs", "cte", "heading_error", "velocity", "reward", "position", "orientation", "laneline_distances",
                  "nearest_edge", "local_path", "local_path_nodes", "path_len", "terminated", "truncated", "info_f64", "seg_count",
                  "seg_i32"]
@@ -136,6 +147,8 @@ def lib():
     L.tc_render_bev.argtypes = [vp, vp, vp]
     L.tc_set_lidar.argtypes = [vp, C.POINTER(TcLidarDesc), vp]
     L.tc_render_lidar.argtypes = [vp, vp, vp]
+    L.tc_set_route.argtypes = [vp, C.POINTER(TcRouteDesc), vp, vp, vp, C.POINTER(TcRouteOutputs)]
+    L.tc_update_route.argtypes = [vp, vp, i32, vp]
     L.tc_set_spawn_rng.argtypes = [vp, vp, vp, i32, vp]
     L.tc_debug_set_timeline.argtypes = [vp, vp]
     L.tc_debug_cull_info.argtypes = [vp, C.POINTER(C.c_double)]
@@ -155,7 +168,7 @@ def lib():
     L.tc_profile_begin.argtypes = [vp, i32]
     L.tc_profile_end.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32)]
     L.tc_debug_layer_query.argtypes = [vp, i32, C.c_double, C.c_double, C.c_double, i32, i32, vp, vp, vp]
-    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_set_lidar", "tc_render_lidar", "tc_create", "tc_create_rig", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
+    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_set_lidar", "tc_render_lidar", "tc_set_route", "tc_update_route", "tc_create", "tc_create_rig", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
                  "tc_render", "tc_get_state", "tc_set_state", "tc_step_host", "tc_debug_layer_query", "tc_profile_begin", "tc_profile_end"):
         getattr(L, name).restype = C.c_int
     if L.tc_abi_version() != 1:

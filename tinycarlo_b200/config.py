@@ -6,6 +6,8 @@ import numbers
 import os
 from typing import Any, Dict, List, Optional, Tuple, Union
 
+import numpy as np
+
 MAPS_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "maps")
 
 
@@ -193,6 +195,48 @@ def lidar_params(config: Dict[str, Any], n_classes: int) -> Optional[Dict[str, A
         raise ValueError(f"lidar.origin must be [forward, right] with finite numbers (metres), got {origin!r}")
     return {"rays": int(rays), "fov": float(fov), "max_range": float(max_range), "origin": [float(origin[0]), float(origin[1])],
             "classes": int(n_classes)}
+
+
+NAV_MAX_GOALS = 4096             # tc_set_route: goal candidates of one handle
+
+
+def navigation_params(config: Dict[str, Any], tables) -> Optional[Dict[str, Any]]:
+    """The optional `navigation` section (an extension: a goal node per car with the route's next maneuver, the distance left
+    and the progress along it, include/tinycarlo_b200.h tc_set_route) with its defaults, or None when the config has none.
+    tables: the map's MapTables. Keys: goals (lanepath node ids; default the map's spawn_points that have an incoming
+    lanepath edge, else every node with one), reach_radius (metres, default 0.05), on_reach ("resample", the default, or "terminate"). Raises ValueError
+    for a bad section."""
+    nav = config.get("navigation")
+    if nav is None:
+        return None
+    if not isinstance(nav, dict):
+        raise ValueError("navigation must be a mapping")
+    unknown = sorted(set(nav) - {"goals", "reach_radius", "on_reach"})
+    if unknown:
+        raise ValueError(f"navigation: unknown keys {unknown} (allowed: goals, reach_radius, on_reach)")
+    n_nodes = len(tables.lp_nodes)
+    has_pred = np.zeros(n_nodes, bool)
+    has_pred[tables.lp_edges[:, 1]] = True
+    goals = nav.get("goals")
+    if goals is None:
+        # the spawn points a car can arrive at (a spawn node without an incoming edge is only ever a start)
+        goals = [g for g in tables.spawn_points if has_pred[g]] if tables.spawn_points is not None else \
+            [int(v) for v in np.nonzero(has_pred)[0]]
+    if not (isinstance(goals, (list, tuple)) and 1 <= len(goals) <= NAV_MAX_GOALS
+            and all(isinstance(g, numbers.Integral) and not isinstance(g, bool) for g in goals)):
+        raise ValueError(f"navigation.goals must be a list of 1..{NAV_MAX_GOALS} lanepath node ids, got {goals!r}")
+    for g in goals:
+        if not 0 <= g < n_nodes:
+            raise ValueError(f"navigation.goals: node {g} is not a lanepath node (0..{n_nodes - 1})")
+        if not has_pred[g]:
+            raise ValueError(f"navigation.goals: node {g} has no incoming lanepath edge, so no car can reach it")
+    reach = nav.get("reach_radius", 0.05)
+    if not (isinstance(reach, numbers.Real) and not isinstance(reach, bool) and math.isfinite(reach) and reach >= 0):
+        raise ValueError(f"navigation.reach_radius must be a finite number >= 0 (metres), got {reach!r}")
+    on_reach = nav.get("on_reach", "resample")
+    if on_reach not in ("resample", "terminate"):
+        raise ValueError(f"navigation.on_reach must be 'resample' or 'terminate', got {on_reach!r}")
+    return {"goals": [int(g) for g in goals], "reach_radius": float(reach), "on_reach": on_reach}
 
 
 # ------------------------------------------------------------------------------------------------ shipped configurations

@@ -13,6 +13,7 @@
 #include "tc_kernels.cuh"
 #include "tc_cull.h"
 #include "tc_pack.h"
+#include "tc_route.h"
 
 // Kernel attributes are per function, not per handle: several handles with different shared-memory needs coexist
 // (TinyCarloGroupedVecEnv), so every kernel is simply allowed the device maximum (227 KB opt-in on sm_100).
@@ -118,6 +119,14 @@ struct TcHandle {
     TcLidarDesc lidar{};          // range scan (tc_set_lidar): off while lidar_out is NULL
     float *lidar_out = nullptr;   // caller-owned [N,C,R]
     double *d_lidar_ab = nullptr; // handle-owned [1024][2]: (cos phi_j, sin phi_j)
+    std::vector<unsigned char> blob_h; // host copy of the map tables (the route table's input)
+    bool route_on = false;           // navigation goals (tc_set_route)
+    TcRoute route{};                 // D, cmd, goals: handle-owned device copies (freed on the next tc_set_route / tc_destroy)
+    uint64_t *route_rng = nullptr;   // caller-owned goal streams, goal indices, prev_distance and outputs
+    int32_t *route_k = nullptr;
+    double *route_prev = nullptr;
+    TcRouteOutputs route_out{};
+    uint8_t *d_route_was_reset = nullptr; // [N]: the was-reset mask when autoreset runs without tc_set_reset_mask
     // optional per-kernel CUDA-event timing (tc_profile_begin/end)
     bool profiling = false;
     int prof_cap = 0, prof_used = 0; // step slots
@@ -240,6 +249,7 @@ int tc_destroy(TcHandle *h) {
     for (void *p : h->allocs) cudaFree(p);
     for (TcCullSet &c : h->cull_sets) { cudaFree(c.d_desc); cudaFree(c.d_blob); }
     for (cudaEvent_t e : h->prof_ev) cudaEventDestroy(e);
+    cudaFree((void *)h->route.D); cudaFree((void *)h->route.cmd); cudaFree((void *)h->route.goals);
     delete h;
     return TC_OK;
 }
@@ -279,6 +289,7 @@ int tc_create_rig(const TcMapDesc *map, const TcSimDesc *sim, int32_t num_envs, 
     h->m_edges.assign(map->ll_edges, map->ll_edges + 2 * (size_t)sumE);
     h->max_nodes = pk.max_nodes;
     h->layout = pk.L;
+    h->blob_h = pk.blob;
     const TcBlobLayout &L = h->layout;
     h->track_smem = (size_t)L.total_bytes;
     if (h->track_smem > 200 * 1024) { tc_destroy(h); return tc_fail(TC_ERR_INVALID, "tc_create: map tables exceed the shared-memory staging budget (200 KB)"); }
@@ -664,6 +675,12 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
     return TC_OK;
 }
 
+// the was-reset mask a step writes: the caller's (tc_set_reset_mask), else the handle's own when the route kernel needs one
+static uint8_t *tc_was_reset(const TcHandle *h) {
+    if (!h->ar_done) return nullptr;
+    return h->ar_was_reset ? h->ar_was_reset : (h->route_on ? h->d_route_was_reset : nullptr);
+}
+
 // mask: per env; in reset mode a rig's view mask (tc_view_mask) is written alongside
 static int tc_launch_track(TcHandle *h, int mode, const float *cc, const int32_t *man, const uint8_t *mask, const int32_t *spawn,
                            const TcOutputs *outs, cudaStream_t st, const double *cc64 = nullptr) {
@@ -675,7 +692,7 @@ static int tc_launch_track(TcHandle *h, int mode, const float *cc, const int32_t
     ta.act_cc = cc; ta.act_cc64 = cc64; ta.act_man = man; ta.mask = mask; ta.spawn_nodes = spawn;
     ta.near_x0 = h->near_h.x0; ta.near_y0 = h->near_h.y0; ta.near_inv_cell = h->near_h.inv_cell; ta.near_nx = h->near_h.nx; ta.near_ny = h->near_h.ny;
     ta.near_off = h->d_near_off; ta.near_edge = h->d_near_edge;
-    ta.done = h->ar_done; ta.was_reset = h->ar_done ? h->ar_was_reset : nullptr; ta.rng = h->rng; ta.spawn_points = h->spawn_points; ta.n_spawn_points = h->n_spawn_points; ta.last_spawn = h->last_spawn;
+    ta.done = h->ar_done; ta.was_reset = tc_was_reset(h); ta.rng = h->rng; ta.spawn_points = h->spawn_points; ta.n_spawn_points = h->n_spawn_points; ta.last_spawn = h->last_spawn;
     if (outs) ta.out = *outs;
     if (h->track_per_thread) {
         tc_track_thread_kernel<<<(h->n_envs + TC_TRACK1_THREADS - 1) / TC_TRACK1_THREADS, TC_TRACK1_THREADS, h->track_smem, st>>>(ta);
@@ -788,6 +805,79 @@ int tc_render_lidar(TcHandle *h, const uint8_t *dev_mask, void *stream) {
     return tc_launch_lidar(h, dev_mask, (cudaStream_t)stream);
 }
 
+// mode as in tc_route_update: 0 after a step (terminated: the step's output), 1 draw, 2 recompute
+static int tc_launch_route(TcHandle *h, int mode, const uint8_t *mask, uint8_t *terminated, cudaStream_t st) {
+    TcRouteArgs a;
+    a.blob = h->d_blob; a.layout = h->layout; a.sf = h->d_sf; a.si = h->d_si; a.r = h->route;
+    a.rng = h->route_rng; a.goal_index = h->route_k; a.prev = h->route_prev; a.out = h->route_out;
+    a.n_envs = h->n_envs; a.mode = mode; a.mask = mask;
+    a.was_reset = mode == 0 ? tc_was_reset(h) : nullptr;
+    a.terminated = mode == 0 ? terminated : nullptr;
+    a.done = mode == 0 ? h->ar_done : nullptr;
+    tc_route_kernel<<<(h->n_envs + TC_ROUTE_THREADS - 1) / TC_ROUTE_THREADS, TC_ROUTE_THREADS, 0, st>>>(a);
+    h->launches++;
+    TC_CUDA(cudaGetLastError());
+    return TC_OK;
+}
+
+int tc_set_route(TcHandle *h, const TcRouteDesc *desc, uint64_t *dev_goal_rng, int32_t *dev_goal_index, double *dev_prev_distance,
+                 const TcRouteOutputs *outs) {
+    if (desc) {   // the description first, so that it can be checked without a device
+        const TcRouteDesc &d = *desc;
+        if (d.n_goals < 1 || d.n_goals > 4096) return tc_fail(TC_ERR_INVALID, "tc_set_route: n_goals must be in 1..4096");
+        if (!d.goals) return tc_fail(TC_ERR_INVALID, "tc_set_route: null goal list");
+        if (!(std::isfinite(d.reach_radius) && d.reach_radius >= 0)) return tc_fail(TC_ERR_INVALID, "tc_set_route: reach_radius must be finite and >= 0");
+        if (d.on_reach != TC_ROUTE_RESAMPLE && d.on_reach != TC_ROUTE_TERMINATE) return tc_fail(TC_ERR_INVALID, "tc_set_route: on_reach must be 0 (resample) or 1 (terminate)");
+    }
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_set_route: null handle");
+    if (desc && (!dev_goal_rng || !dev_goal_index || !dev_prev_distance || !outs || !outs->goal || !outs->goal_position ||
+                 !outs->command || !outs->distance || !outs->progress || !outs->reached))
+        return tc_fail(TC_ERR_INVALID, "tc_set_route: null buffer");
+    const TcTrackTables t = tc_track_tables(h->blob_h.data(), h->layout);
+    const int G = desc ? desc->n_goals : 0, Q = t.lp_n_edges;
+    for (int k = 0; k < G; k++) {
+        const int g = desc->goals[k];
+        if (g < 0 || g >= t.lp_n_nodes) return tc_fail(TC_ERR_INVALID, "tc_set_route: goal node out of range");
+        if (t.prev_off[g] == t.prev_off[g + 1]) return tc_fail(TC_ERR_INVALID, "tc_set_route: goal node " + std::to_string(g) + " has no predecessor");
+    }
+    if ((size_t)G * Q * 9 > ((size_t)256 << 20)) return tc_fail(TC_ERR_INVALID, "tc_set_route: the route table exceeds 256 MiB");
+    TC_CUDA(cudaSetDevice(h->device));
+    TC_CUDA(cudaDeviceSynchronize());   // the old table may still be read by queued kernels
+    h->route_on = false;
+    cudaFree((void *)h->route.D); cudaFree((void *)h->route.cmd); cudaFree((void *)h->route.goals);
+    h->route = TcRoute{};
+    if (!desc) return TC_OK;
+    std::vector<double> D((size_t)G * Q);
+    std::vector<int8_t> cmd((size_t)G * Q);
+    tc_build_route(t, desc->goals, G, D.data(), cmd.data());
+    TcRoute r{};
+    TC_CUDA(cudaMalloc((void **)&r.D, D.size() * sizeof(double)));
+    h->route.D = r.D;
+    TC_CUDA(cudaMalloc((void **)&r.cmd, cmd.size()));
+    h->route.cmd = r.cmd;
+    TC_CUDA(cudaMalloc((void **)&r.goals, (size_t)G * sizeof(int32_t)));
+    h->route.goals = r.goals;
+    TC_CUDA(cudaMemcpy((void *)r.D, D.data(), D.size() * sizeof(double), cudaMemcpyHostToDevice));
+    TC_CUDA(cudaMemcpy((void *)r.cmd, cmd.data(), cmd.size(), cudaMemcpyHostToDevice));
+    TC_CUDA(cudaMemcpy((void *)r.goals, desc->goals, (size_t)G * sizeof(int32_t), cudaMemcpyHostToDevice));
+    if (!h->d_route_was_reset) {
+        TC_TRY(tc_dev_alloc(h, &h->d_route_was_reset, (size_t)h->n_envs));
+        TC_CUDA(cudaMemset(h->d_route_was_reset, 0, (size_t)h->n_envs));
+    }
+    r.G = G; r.Q = Q; r.reach = desc->reach_radius; r.on_reach = desc->on_reach;
+    h->route = r;
+    h->route_rng = dev_goal_rng; h->route_k = dev_goal_index; h->route_prev = dev_prev_distance; h->route_out = *outs;
+    h->route_on = true;
+    return TC_OK;
+}
+
+int tc_update_route(TcHandle *h, const uint8_t *dev_mask, int32_t draw, void *stream) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_update_route: null handle");
+    if (!h->route_on) return tc_fail(TC_ERR_STATE, "tc_update_route: no goals set (tc_set_route)");
+    TC_CUDA(cudaSetDevice(h->device));
+    return tc_launch_route(h, draw ? 1 : 2, dev_mask, nullptr, (cudaStream_t)stream);
+}
+
 int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_nodes, const TcOutputs *outs, void *stream) {
     if (!h) return tc_fail(TC_ERR_INVALID, "tc_reset: null handle");
     if (!dev_spawn_nodes && !h->rng) return tc_fail(TC_ERR_STATE, "tc_reset: no spawn nodes given and no spawn streams set (tc_set_spawn_rng)");
@@ -799,6 +889,7 @@ int tc_reset(TcHandle *h, const uint8_t *dev_mask, const int32_t *dev_spawn_node
         TC_TRY(tc_launch_render(h, tc_view_mask(h, dev_mask), outs->obs, h->obs_format, outs->seg_count, outs->seg_i32, st));
     if (h->bev_out) TC_TRY(tc_launch_bev(h, dev_mask, st));
     if (h->lidar_out) TC_TRY(tc_launch_lidar(h, dev_mask, st));
+    if (h->route_on) TC_TRY(tc_launch_route(h, 1, dev_mask, nullptr, st));
     return TC_OK;
 }
 
@@ -835,6 +926,7 @@ static int tc_step_impl(TcHandle *h, const float *dev_car_control, const double 
     }
     if (h->bev_out) TC_TRY(tc_launch_bev(h, nullptr, st));
     if (h->lidar_out) TC_TRY(tc_launch_lidar(h, nullptr, st));
+    if (h->route_on) TC_TRY(tc_launch_route(h, 0, nullptr, outs ? outs->terminated : nullptr, st));
     return TC_OK;
 }
 

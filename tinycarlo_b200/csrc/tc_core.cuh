@@ -542,6 +542,92 @@ TC_HD int tc_spawn_draw(const TcTrackTables &t, uint64_t *st, const int32_t *cho
     return -1;
 }
 
+// ------------------------------------------------------------------------------------------------ navigation goals
+// tc_set_route's contract (include/tinycarlo_b200.h TcRouteDesc), one env at a time: tc_route_kernel runs it with a thread per
+// env, ht_route_update sequentially. The route table comes from tc_route.h.
+struct TcRoute {
+    const double *D;        // [G][Q]
+    const int8_t *cmd;      // [G][Q]
+    const int32_t *goals;   // [G]
+    int G, Q;
+    double reach;
+    int on_reach;
+};
+// the env's tracked edge pe0, or -1
+TC_HD int tc_route_edge(const TcTrackTables &t, const int32_t *si) {
+    const int pe = si[TC_SI_PATH_EDGES], pn0 = si[TC_SI_PATH_NODES], pn1 = si[TC_SI_PATH_NODES + 1];
+    if (si[TC_SI_PATH_LEN] <= 0 || pe < 0 || pe >= t.lp_n_edges || pn0 < 0 || pn1 < 0 || pn1 >= t.lp_n_nodes) return -1;
+    return pe;
+}
+// distance to goal k (+inf: no route, no tracked edge, no goal), with its command and reached flag
+TC_HD double tc_route_eval(const TcTrackTables &t, const TcRoute &r, int pe, int pn1, double fx, double fy, int k, int &command,
+                           bool &reached) {
+    command = -1;
+    reached = false;
+    if (k < 0 || pe < 0) return INFINITY;
+    const size_t at = (size_t)k * r.Q + pe;
+    const double D = r.D[at];
+    if (!(D < INFINITY)) return INFINITY;
+    command = r.cmd[at];
+    const double d = tc_dist(fx, fy, t.lp_nodes[2 * pn1], t.lp_nodes[2 * pn1 + 1]);
+    reached = pn1 == r.goals[k] && d <= r.reach;
+    return d + D;
+}
+// one draw among the valid goals (list order: finite D_k(pe0), not reached at this pose) on the goal stream; -1 when there is
+// none, and then the stream does not move
+TC_HD int tc_route_draw(const TcTrackTables &t, const TcRoute &r, int pe, int pn1, double fx, double fy, uint64_t *st) {
+    if (pe < 0) return -1;
+    const bool at_pn1 = tc_dist(fx, fy, t.lp_nodes[2 * pn1], t.lp_nodes[2 * pn1 + 1]) <= r.reach;
+    uint32_t n = 0;
+    for (int k = 0; k < r.G; k++) n += r.D[(size_t)k * r.Q + pe] < INFINITY && !(at_pn1 && r.goals[k] == pn1);
+    if (n == 0) return -1;
+    uint32_t j = tc_pcg_bounded(st, n);
+    for (int k = 0; k < r.G; k++)
+        if (r.D[(size_t)k * r.Q + pe] < INFINITY && !(at_pn1 && r.goals[k] == pn1)) {
+            if (j == 0) return k;
+            j--;
+        }
+    return -1;
+}
+// mode 0: after a step (draws where the step autoreset, resamples or terminates on a reach); 1: draw; 2: recompute with
+// progress 0. k and prev are the env's goal index and prev_distance, updated in place; terminate: OR 1 into the done flags.
+TC_HD void tc_route_update(const TcTrackTables &t, const TcRoute &r, int mode, bool was_reset, const int32_t *si, double fx, double fy,
+                           uint64_t *st, int32_t &k, double &prev, int &command, double &distance, double &progress, bool &reached,
+                           bool &terminate) {
+    const int pe = tc_route_edge(t, si), pn1 = si[TC_SI_PATH_NODES + 1];
+    if (k < 0 || k >= r.G) k = -1;
+    progress = 0;
+    reached = terminate = false;
+    bool draw = mode == 1 || (mode == 0 && was_reset);
+    if (!draw) {
+        distance = tc_route_eval(t, r, pe, pn1, fx, fy, k, command, reached);
+        if (mode == 0) {
+            if (isfinite(prev) && isfinite(distance)) progress = prev - distance;
+            if (reached) {
+                if (r.on_reach == TC_ROUTE_TERMINATE) terminate = true;
+                else draw = true;   // progress and reached stay those of the goal just reached
+            }
+        }
+    }
+    if (draw) {
+        bool unused;
+        k = tc_route_draw(t, r, pe, pn1, fx, fy, st);
+        distance = tc_route_eval(t, r, pe, pn1, fx, fy, k, command, unused);   // a drawn goal is never reached where it was drawn
+    }
+    prev = distance;
+}
+TC_HD void tc_route_store(const TcTrackTables &t, const TcRoute &r, const TcRouteOutputs &o, size_t i, int k, int command, double distance,
+                          double progress, bool reached) {
+    const int node = k >= 0 ? r.goals[k] : -1;
+    o.goal[i] = node;
+    o.goal_position[2 * i] = node >= 0 ? (float)t.lp_nodes[2 * node] : NAN;
+    o.goal_position[2 * i + 1] = node >= 0 ? (float)t.lp_nodes[2 * node + 1] : NAN;
+    o.command[i] = command;
+    o.distance[i] = (float)distance;
+    o.progress[i] = (float)progress;
+    o.reached[i] = reached ? 1 : 0;
+}
+
 // ------------------------------------------------------------------------------------------------ blob noise
 // NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) draws from the unseeded global numpy RNG; tc_noise_blobs
 // draws every blob from Philox4x32-10 instead (contract in include/tinycarlo_b200.h), so the noise is a pure function of

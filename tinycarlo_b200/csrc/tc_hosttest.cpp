@@ -13,6 +13,7 @@
 #include "tc_core.cuh"
 #include "tc_cull.h"
 #include "tc_pack.h"
+#include "tc_route.h"
 
 #define HT_API extern "C" __attribute__((visibility("default")))
 
@@ -258,6 +259,39 @@ HT_API int ht_lidar_keep(const TcLidarDesc *d, double ox, double oy, double c, d
     const TcLidarGeom g = {d->rays, d->fov, d->max_range, d->origin_forward, d->origin_right};
     double st[5];
     return tc_lidar_stage(g, ox, oy, c, s, ax, ay, bx, by, st) ? 1 : 0;
+}
+
+// the route table of tc_set_route (tc_route.h) for goals[0..G-1]: D [G][Q], cmd [G][Q]
+HT_API void ht_route_table(const HtMap *m, int G, const int32_t *goals, double *D, int8_t *cmd) {
+    tc_build_route(tc_track_tables(m->pk.blob.data(), m->pk.L), goals, G, D, cmd);
+}
+
+// mirrors tc_route_kernel for n envs at states sf / si (mode, mask, was_reset as there; terminated / done optional, OR-ed)
+HT_API void ht_route_update(const HtMap *m, int G, const int32_t *goals, const double *D, const int8_t *cmd, double reach, int on_reach,
+                            int n, int mode, const double *sf, const int32_t *si, const uint8_t *mask, const uint8_t *was_reset,
+                            uint64_t *rng, int32_t *goal_index, double *prev, int32_t *goal, float *goal_position, int32_t *command,
+                            float *distance, float *progress, uint8_t *reached, uint8_t *terminated, uint8_t *done) {
+    const TcTrackTables t = tc_track_tables(m->pk.blob.data(), m->pk.L);
+    TcRoute r;
+    r.D = D; r.cmd = cmd; r.goals = goals; r.G = G; r.Q = t.lp_n_edges; r.reach = reach; r.on_reach = on_reach;
+    TcRouteOutputs o = {goal, goal_position, command, distance, progress, reached};
+    for (int i = 0; i < n; i++) {
+        if (mode != 0 && mask && !mask[i]) continue;
+        const double *s = sf + (size_t)i * TC_SF_N;
+        int32_t k = goal_index[i];
+        double p = prev[i], dist, prog;
+        int c;
+        bool re, term;
+        tc_route_update(t, r, mode, was_reset && was_reset[i], si + (size_t)i * TC_SI_N, s[TC_SF_FRONT_X], s[TC_SF_FRONT_Y],
+                        rng + (size_t)i * TC_RNG_N, k, p, c, dist, prog, re, term);
+        goal_index[i] = k;
+        prev[i] = p;
+        tc_route_store(t, r, o, i, k, c, dist, prog, re);
+        if (term) {
+            if (terminated) terminated[i] = 1;
+            if (done) done[i] = 1;
+        }
+    }
 }
 
 // the reset paths' spawn draws (tc_spawn_draw): k consecutive draws of n env streams, states advanced in place

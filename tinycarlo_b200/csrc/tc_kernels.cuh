@@ -1820,6 +1820,47 @@ __global__ void __launch_bounds__(TC_LIDAR_THREADS) tc_lidar_kernel(const TcLida
     }
 }
 
+// ------------------------------------------------------------------------------------------------ navigation goals
+// tc_set_route's contract (include/tinycarlo_b200.h TcRouteDesc), a thread per env (tc_route_update in tc_core.cuh). A step
+// reads one route-table entry of D and one of cmd per env (the table stays in L2); only the threads that draw a goal scan the
+// G candidates and touch their goal stream.
+#define TC_ROUTE_THREADS 256
+struct TcRouteArgs {
+    const unsigned char *blob;     // map tables (tc_track_tables)
+    TcBlobLayout layout;
+    const double *sf;              // [N,TC_SF_N]
+    const int32_t *si;             // [N,TC_SI_N]
+    TcRoute r;
+    uint64_t *rng;                 // [N,TC_RNG_N] goal streams
+    int32_t *goal_index;           // [N]
+    double *prev;                  // [N] prev_distance
+    TcRouteOutputs out;
+    int n_envs, mode;              // mode: tc_route_update's
+    const uint8_t *mask;           // optional, modes 1 and 2
+    const uint8_t *was_reset;      // optional, mode 0: the envs the step autoreset
+    uint8_t *terminated, *done;    // optional, mode 0: OR-ed on a reach with TC_ROUTE_TERMINATE
+};
+
+__global__ void __launch_bounds__(TC_ROUTE_THREADS) tc_route_kernel(const TcRouteArgs a) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n_envs || (a.mode != 0 && a.mask && !a.mask[i])) return;
+    const TcTrackTables t = tc_track_tables(a.blob, a.layout);
+    const double *sf = a.sf + (size_t)i * TC_SF_N;
+    int32_t k = a.goal_index[i];
+    double prev = a.prev[i], distance, progress;
+    int command;
+    bool reached, terminate;
+    tc_route_update(t, a.r, a.mode, a.was_reset && a.was_reset[i], a.si + (size_t)i * TC_SI_N, sf[TC_SF_FRONT_X], sf[TC_SF_FRONT_Y],
+                    a.rng + (size_t)i * TC_RNG_N, k, prev, command, distance, progress, reached, terminate);
+    a.goal_index[i] = k;
+    a.prev[i] = prev;
+    tc_route_store(t, a.r, a.out, i, k, command, distance, progress, reached);
+    if (terminate) {
+        if (a.terminated) a.terminated[i] = 1;
+        if (a.done) a.done[i] = 1;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ blob noise
 // NoiseObservationWrapper (tinycarlo/wrapper/observation.py:14-27) on the device: per class, n_blobs filled circles that
 // either erase the class mask or OR in the pixels of a randomly chosen class, applied in the reference's order (classes

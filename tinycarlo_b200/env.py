@@ -178,6 +178,11 @@ class TinyCarloEnv(gc.Env):
             info["bev"] = v.bev[0].cpu().numpy()
         if v.lidar is not None:   # the config's `lidar` section (an extension): this env's range scan [C, R]
             info["lidar"] = v.lidar[0].cpu().numpy()
+        if v.route is not None:   # the config's `navigation` section (an extension): this env's goal and route
+            r = v.route
+            info.update({"goal": int(r["goal"][0].item()), "goal_position": [float(x) for x in r["goal_position"][0].cpu().numpy()],
+                         "route_command": int(r["command"][0].item()), "route_distance": float(r["distance"][0].item()),
+                         "route_progress": float(r["progress"][0].item()), "goal_reached": bool(r["reached"][0].item())})
         return info
 
     def reset(self, seed: Optional[int] = None, options: Optional[Any] = None) -> Tuple[np.ndarray, Dict[str, Any]]:

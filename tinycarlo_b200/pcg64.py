@@ -11,7 +11,7 @@ One numpy Generator per env costs ~4 us per scalar draw in the interpreter; a ve
 
 tests/test_host_logic.py checks the streams against numpy itself (thousands of seeds, ranges that exercise the rejection
 loop) and against the spawn draws recorded from the reference."""
-from typing import Optional
+from typing import Optional, Tuple
 
 import numpy as np
 
@@ -39,8 +39,12 @@ def _mix(x, y):
     return r ^ (r >> XSHIFT)
 
 
-def seed_sequence_state(seeds: np.ndarray) -> np.ndarray:
-    """SeedSequence(int(seed)).generate_state(4, np.uint64) for every non-negative seed < 2^64 -> uint64 [n, 4]."""
+def seed_sequence_state(seeds: np.ndarray, spawn_key: Tuple[int, ...] = ()) -> np.ndarray:
+    """SeedSequence(int(seed), spawn_key=spawn_key).generate_state(4, np.uint64) for every non-negative seed < 2^64 -> uint64
+    [n, 4]. spawn_key (words < 2^32) is what SeedSequence.spawn gives its children: spawn(1)[0] has spawn_key (0,). numpy pads
+    the seed's words to the pool size of 4 and mixes every word beyond the pool into all pool words ("remaining entropy")."""
+    key = [int(k) for k in spawn_key]
+    assert all(0 <= k <= 0xFFFFFFFF for k in key)
     with np.errstate(over="ignore"):
         seeds = np.asarray(seeds, dtype=_U64)
         n = len(seeds)
@@ -56,6 +60,10 @@ def seed_sequence_state(seeds: np.ndarray) -> np.ndarray:
                 if i_src != i_dst:
                     h, hc = _hashmix(pool[i_src].copy(), hc)
                     pool[i_dst] = _mix(pool[i_dst], h)
+        for word in key:
+            for i_dst in range(4):
+                h, hc = _hashmix(np.full(n, word, _U32), hc)
+                pool[i_dst] = _mix(pool[i_dst], h)
         out = np.zeros((8, n), _U32)
         hc = np.full(n, INIT_B, _U32)
         for i_dst in range(8):
@@ -80,15 +88,15 @@ def _mul64(a, b):
 
 
 class VecPCG64:
-    """n independent PCG64 streams; stream i equals numpy's PCG64(SeedSequence(seeds[i]))."""
+    """n independent PCG64 streams; stream i equals numpy's PCG64(SeedSequence(seeds[i], spawn_key=spawn_key))."""
 
-    def __init__(self, seeds: Optional[np.ndarray] = None):
+    def __init__(self, seeds: Optional[np.ndarray] = None, spawn_key: Tuple[int, ...] = ()):
         if seeds is not None:
-            self.seed(seeds)
+            self.seed(seeds, spawn_key)
 
-    def seed(self, seeds):
+    def seed(self, seeds, spawn_key: Tuple[int, ...] = ()):
         with np.errstate(over="ignore"):
-            s = seed_sequence_state(seeds)
+            s = seed_sequence_state(seeds, spawn_key)
             n = len(s)
             init_hi, init_lo, seq_hi, seq_lo = s[:, 0], s[:, 1], s[:, 2], s[:, 3]
             self.inc_hi = (seq_hi << _U64(1)) | (seq_lo >> _U64(63))

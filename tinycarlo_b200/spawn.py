@@ -32,6 +32,16 @@ def spawn_stream_states(num_envs: int, seed: Optional[int], env_index_offset: in
     return VecPCG64(stream_seeds(num_envs, seed, env_index_offset)).device_rows()
 
 
+def goal_stream_states(num_envs: int, seed: Optional[int], env_index_offset: int = 0, seeds: Optional[np.ndarray] = None) -> np.ndarray:
+    """The goal streams of the navigation goals (include/tinycarlo_b200.h TcRouteDesc) in the same row layout: env i gets
+    Generator(PCG64(SeedSequence(seed + offset + i).spawn(1)[0])), the first child of its spawn stream's seed sequence, so the
+    spawn draws stay what they are without goals. seeds: the per-env seeds stream_seeds() returned for the spawn streams (with
+    seed None, the same OS entropy)."""
+    if seeds is None:
+        seeds = stream_seeds(num_envs, seed, env_index_offset)
+    return VecPCG64(seeds, spawn_key=(0,)).device_rows()
+
+
 class SpawnSampler:
     def __init__(self, tables: MapTables, num_envs: int, table_len: int = 16, env_index_offset: int = 0):
         self.tables, self.n, self.K, self.offset = tables, int(num_envs), int(table_len), int(env_index_offset)

@@ -18,9 +18,11 @@ import torch
 
 from . import _lib
 from .camera_params import camera_row, view_rows
-from .config import LINE_THICKNESS_MAX, bev_params, camera_params, lidar_params, camera_rig, car_param_row, load_config, resolve_map_path, sim_params
+from .config import (LINE_THICKNESS_MAX, bev_params, camera_params, lidar_params, camera_rig, car_param_row, load_config, navigation_params,
+                     resolve_map_path, sim_params)
 from .maptables import MapTables
-from .spawn import spawn_stream_states
+from .pcg64 import VecPCG64
+from .spawn import goal_stream_states, stream_seeds
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -129,6 +131,30 @@ class TinyCarloVecEnv:
                 self.lidar = torch.zeros((N, Cn, li["rays"]), dtype=torch.float32, device=dev)
                 ldesc = _lib.TcLidarDesc(li["rays"], li["fov"], li["max_range"], li["origin"][0], li["origin"][1])
                 _lib.check(self._L.tc_set_lidar(self._h, C.byref(ldesc), _ptr(self.lidar)), "tc_set_lidar")
+            # navigation goals (config section `navigation`, tc_set_route): a goal node per env with the route's command,
+            # distance and progress, rewritten by every step() / reset() whatever no_observation says; None without the section
+            self.nav_cfg = navigation_params(self.config, self.map)
+            self.route = None
+            self._goal_rng = None
+            if self.nav_cfg is not None:
+                nv = self.nav_cfg
+                self._nav_goals = np.ascontiguousarray(nv["goals"], np.int32)
+                self._goal_slot = {}   # node id -> its first index in the goal list
+                for k, g in enumerate(nv["goals"]):
+                    self._goal_slot.setdefault(g, k)
+                self._goal_rng = torch.zeros((N, _lib.TC_RNG_N), dtype=torch.int64, device=dev)   # uint64 bit patterns
+                self._goal_index = torch.full((N,), -1, dtype=torch.int32, device=dev)
+                self._prev_distance = torch.full((N,), float("inf"), dtype=torch.float64, device=dev)
+                self.route = {"goal": torch.full((N,), -1, dtype=torch.int32, device=dev),
+                              "goal_position": torch.full((N, 2), float("nan"), dtype=torch.float32, device=dev),
+                              "command": torch.full((N,), -1, dtype=torch.int32, device=dev),
+                              "distance": torch.full((N,), float("inf"), dtype=torch.float32, device=dev),
+                              "progress": f32(N), "reached": torch.zeros(N, dtype=torch.uint8, device=dev)}
+                rdesc = _lib.TcRouteDesc(len(self._nav_goals), self._nav_goals.ctypes.data, nv["reach_radius"],
+                                         1 if nv["on_reach"] == "terminate" else 0)
+                routs = _lib.TcRouteOutputs(*(self.route[k].data_ptr() for k in _lib.ROUTE_OUTPUT_FIELDS))
+                _lib.check(self._L.tc_set_route(self._h, C.byref(rdesc), _ptr(self._goal_rng), _ptr(self._goal_index),
+                                                _ptr(self._prev_distance), C.byref(routs)), "tc_set_route")
             self._spawn_nodes = torch.full((N,), -1, dtype=torch.int32, device=dev)   # node of each env's latest reset
             self._mask_all = torch.ones(N, dtype=torch.uint8, device=dev)
         self._outs = self._make_outputs(with_obs=True)
@@ -321,9 +347,12 @@ class TinyCarloVecEnv:
 
     # ------------------------------------------------------------------------------------------------ spawn draws
     def _seed(self, seed: Optional[int]):
-        st = spawn_stream_states(self.num_envs, seed, self.env_index_offset)
+        seeds = stream_seeds(self.num_envs, seed, self.env_index_offset)
+        st = VecPCG64(seeds).device_rows()
         with torch.cuda.device(self.device):
             self._rng_state.copy_(torch.from_numpy(st.view(np.int64)))   # in place: the library holds the address
+            if self._goal_rng is not None:   # the goal streams: children of the same seeds (OS entropy included)
+                self._goal_rng.copy_(torch.from_numpy(goal_stream_states(self.num_envs, seed, self.env_index_offset, seeds=seeds).view(np.int64)))
         self._seeded = True
 
     # ------------------------------------------------------------------------------------------------ gym-like API
@@ -336,6 +365,10 @@ class TinyCarloVecEnv:
             info["bev"] = self.bev
         if self.lidar is not None:
             info["lidar"] = self.lidar
+        if self.route is not None:
+            r = self.route
+            info.update({"goal": r["goal"], "goal_position": r["goal_position"], "route_command": r["command"],
+                         "route_distance": r["distance"], "route_progress": r["progress"], "goal_reached": r["reached"].view(torch.bool)})
         return info
 
     def reset(self, seed: Optional[int] = None, mask: Optional[torch.Tensor] = None, spawn_nodes: Optional[torch.Tensor] = None):
@@ -504,6 +537,31 @@ class TinyCarloVecEnv:
             _lib.check(self._L.tc_render_lidar(self._h, _ptr(m), self._stream()), "tc_render_lidar")
         return self.lidar
 
+    def _update_route(self, mask: Optional[torch.Tensor], draw: bool):
+        with torch.cuda.device(self.device):
+            m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            _lib.check(self._L.tc_update_route(self._h, _ptr(m), int(draw), self._stream()), "tc_update_route")
+
+    def set_goals(self, nodes, mask: Optional[torch.Tensor] = None):
+        """Sets the goal of the envs in `mask` (None = all) to nodes[i], a lanepath node id from the config's
+        navigation.goals (int [N]), and recomputes their command and distance with progress 0. Raises ValueError for a node
+        that is not in the goal list."""
+        if self.route is None:
+            raise ValueError("set_goals: the config has no `navigation` section")
+        a = nodes.detach().cpu().numpy() if isinstance(nodes, torch.Tensor) else np.asarray(nodes)
+        if a.shape != (self.num_envs,) or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"set_goals: nodes must be {self.num_envs} integer node ids")
+        sel = np.ones(self.num_envs, bool) if mask is None else (mask.detach().cpu().numpy() if isinstance(mask, torch.Tensor)
+                                                                  else np.asarray(mask)).astype(bool).reshape(self.num_envs)
+        bad = sorted({int(v) for v in a[sel]} - set(self._goal_slot))
+        if bad:
+            raise ValueError(f"set_goals: nodes {bad[:8]} are not in navigation.goals")
+        idx = np.array([self._goal_slot[int(v)] if s else 0 for v, s in zip(a, sel)], np.int32)
+        with torch.cuda.device(self.device):
+            sel_t = torch.from_numpy(sel).to(self.device)
+            self._goal_index.copy_(torch.where(sel_t, torch.from_numpy(idx).to(self.device), self._goal_index))
+        self._update_route(sel_t, draw=False)
+
     def render_obs(self, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Re-render self.obs (all views) at the current poses (after load_state_dict / set_camera_params); mask is per env."""
         with torch.cuda.device(self.device):
@@ -523,14 +581,18 @@ class TinyCarloVecEnv:
         return {"sf": sf, "si": si}
 
     def checkpoint(self) -> Dict[str, Any]:
-        """Everything needed to resume a rollout bit for bit: car state, the spawn streams (per-env PCG64 states) and the
-        autoreset flags. The reference has no counterpart (SURVEY section 5)."""
+        """Everything needed to resume a rollout bit for bit: car state, the spawn streams (per-env PCG64 states), the
+        autoreset flags and, with navigation goals, the goal streams, goal indices and previous route distances. The reference has no counterpart (SURVEY section 5)."""
         ck = {k: v.cpu() for k, v in self.state_dict().items()}
         if self._seeded:
             ck["spawn_rng"] = self._rng_state.cpu()
             ck["last_spawn"] = self._spawn_nodes.cpu()
         if self.autoreset:
             ck["done_flags"] = self.done_flags.cpu()
+        if self.route is not None:
+            ck["goal_rng"] = self._goal_rng.cpu()
+            ck["goal_index"] = self._goal_index.cpu()
+            ck["prev_distance"] = self._prev_distance.cpu()
         return ck
 
     def restore(self, ck: Dict[str, Any]):
@@ -546,6 +608,11 @@ class TinyCarloVecEnv:
             self.render_bev()
         if self.lidar is not None:
             self.render_lidar()
+        if self.route is not None and "goal_index" in ck:
+            self._goal_rng.copy_(ck["goal_rng"])
+            self._goal_index.copy_(ck["goal_index"])
+            self._update_route(None, draw=False)          # the outputs at the restored state
+            self._prev_distance.copy_(ck["prev_distance"])
 
     def load_state_dict(self, state: Dict[str, torch.Tensor]):
         with torch.cuda.device(self.device):

@@ -187,8 +187,45 @@ class CTELinearRewardWrapper:
     __new__ = _make(_CTELinearScalar, _CTELinearVec)
 
 
+# ------------------------------------------------------------------------------------------------ route progress
+# An extension (the reference has no navigation task): needs the config's `navigation` section.
+class _RouteProgressScalar(Wrapper):
+    def __init__(self, env, progress_scale: float = 1.0, goal_bonus: float = 0.0):
+        super().__init__(env)
+        self.unwrapped.wrapped = True
+        self.progress_scale, self.goal_bonus = progress_scale, goal_bonus
+
+    def step(self, action):
+        observation, reward, terminated, truncated, info = self.env.step(action)
+        if "route_progress" not in info:
+            raise ValueError("RouteProgressRewardWrapper needs the config's `navigation` section")
+        reward += self.progress_scale * info["route_progress"] + self.goal_bonus * float(info["goal_reached"])
+        return observation, reward, terminated, truncated, info
+
+
+class _RouteProgressVec(_VecWrapper):
+    def __init__(self, env, progress_scale: float = 1.0, goal_bonus: float = 0.0):
+        super().__init__(env)
+        if getattr(self.unwrapped, "route", None) is None:
+            raise ValueError("RouteProgressRewardWrapper needs the config's `navigation` section")
+        self.progress_scale, self.goal_bonus = progress_scale, goal_bonus
+
+    def step(self, action):
+        observation, reward, terminated, truncated, info = self.env.step(action)
+        term = self.progress_scale * info["route_progress"] + self.goal_bonus * info["goal_reached"].to(torch.float32)
+        reward = reward + self._live(term)
+        return observation, reward, terminated, truncated, info
+
+
+class RouteProgressRewardWrapper:
+    """reward += progress_scale * route_progress + goal_bonus * goal_reached: metres gained along the route to the goal, and
+    a bonus on the step a goal is reached (the config's `navigation` section)."""
+    __new__ = _make(_RouteProgressScalar, _RouteProgressVec)
+
+
 for _pub, _impls in ((LanelineSparseRewardWrapper, (_LanelineSparseScalar, _LanelineSparseVec)),
                      (LanelineLinearRewardWrapper, (_LanelineLinearScalar, _LanelineLinearVec)),
-                     (CTESparseRewardWrapper, (_CTESparseScalar, _CTESparseVec)), (CTELinearRewardWrapper, (_CTELinearScalar, _CTELinearVec))):
+                     (CTESparseRewardWrapper, (_CTESparseScalar, _CTESparseVec)), (CTELinearRewardWrapper, (_CTELinearScalar, _CTELinearVec)),
+                     (RouteProgressRewardWrapper, (_RouteProgressScalar, _RouteProgressVec))):
     for _i in _impls:
         _i.__name__ = _pub.__name__
