@@ -208,6 +208,36 @@ TC_API int tc_step_host_obs(TcHandle *h, const float *host_car_control, const in
 TC_API int tc_noise_blobs(TcHandle *h, uint8_t *dev_obs, uint64_t seed, uint32_t step, int32_t n_blobs, int32_t max_radius,
                           int32_t env_index_offset, const uint8_t *dev_mask, void *stream);
 
+/* Tracked observation buffer: renders store only the 32-byte sectors of a frame that can have changed. A class mask is almost
+ * all zeros, and most of its zeros stay zero from one step to the next; the handle keeps one bit per sector that is set when
+ * the sector may hold a non-zero byte, and a render stores a sector only when it holds a set pixel now or its bit is set.
+ * The bytes of the buffer after every render are exactly those of an untracked render.
+ *
+ *   tc_track_obs(h, dev_obs)   dev_obs: a u8 classes buffer [N,(M,)C,H,W] of this handle. The caller declares that between
+ *                              renders nothing but this handle writes it, unless it calls tc_invalidate_obs after such a
+ *                              write. The handle allocates the mask and sets every bit (a set-up call: it synchronises the
+ *                              device). NULL switches tracking off with no CUDA call, so it is allowed inside a stream
+ *                              capture; the mask's memory is released by the next tc_track_obs that keeps no mask, or by
+ *                              tc_destroy. TC_ERR_INVALID for a handle whose obs_format is not TC_OBS_CLASSES or a dev_obs
+ *                              that is not 32-byte aligned.
+ *   tc_invalidate_obs(h, st)   sets every bit again (one memset of the mask on the stream): after any write to the buffer
+ *                              that the handle does not make, e.g. from another kernel, a copy or a collective.
+ *
+ * The mask is kept where the frames are rendered by the per-class kernel (large u8 frames, tc_debug_render_info
+ * block_per_env = 0) and H*W is a multiple of 32; then sector s of a plane is exactly word s of the kernel's bit plane. Elsewhere
+ * tracking is accepted and does nothing: renders store every byte. Mask layout: uint32 [N*M][C][ceil(H*W/1024)], bit b of
+ * word w covers sector 32*w + b of that plane (98.3 MB for 16384 envs at 5x480x640). Renders into the tracked buffer keep the
+ * mask: tc_step / tc_step_f64 / tc_step_host(_obs) / tc_reset / tc_render in TC_OBS_CLASSES without debug segment export.
+ * Every other write of this handle that overlaps it - tc_noise_blobs, tc_render in another format, a segment-export render -
+ * sets every bit, so the next render stores the whole frame once. A CUDA graph captured while tracking is on replays the
+ * captured mask reads and writes: only replay it when nothing else writes the buffer between replays. */
+TC_API int tc_track_obs(TcHandle *h, uint8_t *dev_obs);
+TC_API int tc_invalidate_obs(TcHandle *h, void *stream);
+/* What tracking does for this handle: *host_words = number of mask words kept for the tracked buffer (0: no buffer tracked, or this
+ * handle's renders keep no mask); dev_out, when not NULL and there is a mask, receives a copy of it (uint32 [*host_words],
+ * stream-ordered). */
+TC_API int tc_obs_mask(TcHandle *h, uint32_t *dev_out, int64_t *host_words, void *stream);
+
 /* Ego-centric bird's-eye view (BEV): top-down lane masks around every car, P = C + route planes. For env i with state
  * x = sf[TC_SF_X], y = sf[TC_SF_Y], θ = sf[TC_SF_ROT] (the rear axle, in map metres; map coordinates are image-like, y down):
  *

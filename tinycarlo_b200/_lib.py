@@ -155,6 +155,9 @@ def lib():
     L.tc_debug_render_info.argtypes = [vp, C.POINTER(i32)]
     L.tc_episode_stats.argtypes = [vp, vp, vp, i32, vp, vp]
     L.tc_noise_blobs.argtypes = [vp, vp, C.c_uint64, C.c_uint32, i32, i32, i32, vp, vp]
+    L.tc_track_obs.argtypes = [vp, vp]
+    L.tc_invalidate_obs.argtypes = [vp, vp]
+    L.tc_obs_mask.argtypes = [vp, vp, C.POINTER(i64), vp]
     L.tc_reset.argtypes = [vp, vp, vp, C.POINTER(TcOutputs), vp]
     L.tc_step.argtypes = [vp, vp, vp, C.POINTER(TcOutputs), vp]
     L.tc_step_f64.argtypes = [vp, vp, vp, C.POINTER(TcOutputs), vp]
@@ -168,7 +171,7 @@ def lib():
     L.tc_profile_begin.argtypes = [vp, i32]
     L.tc_profile_end.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32)]
     L.tc_debug_layer_query.argtypes = [vp, i32, C.c_double, C.c_double, C.c_double, i32, i32, vp, vp, vp]
-    for name in ("tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_set_lidar", "tc_render_lidar", "tc_set_route", "tc_update_route", "tc_create", "tc_create_rig", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
+    for name in ("tc_track_obs", "tc_invalidate_obs", "tc_obs_mask", "tc_episode_stats", "tc_set_camera_params_host", "tc_debug_cull_stats", "tc_debug_render_info", "tc_step_host_obs", "tc_set_reset_mask", "tc_debug_cull_info", "tc_set_spawn_rng", "tc_noise_blobs", "tc_step_f64", "tc_debug_set_timeline", "tc_set_autoreset", "tc_set_bev", "tc_render_bev", "tc_set_lidar", "tc_render_lidar", "tc_set_route", "tc_update_route", "tc_create", "tc_create_rig", "tc_destroy", "tc_set_car_params", "tc_set_camera_params", "tc_set_wrapped", "tc_reset", "tc_step",
                  "tc_render", "tc_get_state", "tc_set_state", "tc_step_host", "tc_debug_layer_query", "tc_profile_begin", "tc_profile_end"):
         getattr(L, name).restype = C.c_int
     if L.tc_abi_version() != 1:

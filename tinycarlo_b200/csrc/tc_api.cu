@@ -131,6 +131,10 @@ struct TcHandle {
     bool profiling = false;
     int prof_cap = 0, prof_used = 0; // step slots
     std::vector<cudaEvent_t> prof_ev; // 4 events per slot: before track, after track, after project, after raster
+    // tracked observation buffer (tc_track_obs): per 32-byte sector of every plane, whether it may hold a non-zero byte
+    uint8_t *obs_tracked = nullptr;   // caller-owned; NULL: the renders store every byte
+    uint32_t *obs_mask = nullptr;     // handle-owned [n_views][C][tc_sector_mask_words], allocated whenever obs_tracked is set
+    size_t obs_mask_bytes = 0;
 };
 
 template <typename T>
@@ -250,6 +254,7 @@ int tc_destroy(TcHandle *h) {
     for (TcCullSet &c : h->cull_sets) { cudaFree(c.d_desc); cudaFree(c.d_blob); }
     for (cudaEvent_t e : h->prof_ev) cudaEventDestroy(e);
     cudaFree((void *)h->route.D); cudaFree((void *)h->route.cmd); cudaFree((void *)h->route.goals);
+    cudaFree(h->obs_mask);
     delete h;
     return TC_OK;
 }
@@ -557,6 +562,23 @@ static TcRenderEnvArgs tc_render_env_args(const TcHandle *h, const uint8_t *mask
     return ea;
 }
 
+// bytes of the handle's frames in `format`
+static size_t tc_frame_bytes(const TcHandle *h, int format) {
+    const size_t v = (size_t)h->n_views, hw = (size_t)h->H * h->W;
+    if (format == TC_OBS_RGB) return v * hw * 3;
+    if (format == TC_OBS_CLASSES_BITS) return v * h->C * ((hw + 31) / 32) * 4;
+    return v * h->C * hw * (format == TC_OBS_CLASSES_BF16 ? 2 : 1);
+}
+
+// A write of `bytes` at `p` that does not keep the sector mask: when it touches the tracked buffer, every sector becomes
+// possibly non-zero again (the next tracked render stores the whole frame, and the mask is exact after it).
+static int tc_obs_written(TcHandle *h, const void *p, size_t bytes, cudaStream_t st) {
+    if (!h->obs_tracked || !p) return TC_OK;
+    const uint8_t *a = (const uint8_t *)p, *t = h->obs_tracked;
+    if (a < t + tc_frame_bytes(h, TC_OBS_CLASSES) && t < a + bytes) TC_CUDA(cudaMemsetAsync(h->obs_mask, 0xFF, h->obs_mask_bytes, st));
+    return TC_OK;
+}
+
 // renders the handle's n_views views; mask (NULL = all) is per view
 static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int obs_format, int32_t *seg_count_out, int32_t *seg_out,
                             cudaStream_t st, cudaEvent_t after_project = nullptr) {
@@ -578,6 +600,9 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
         TC_CUDA(cudaMemsetAsync(h->prims.cls_info, 0, (size_t)N * C * 4, st));
         TC_CUDA(cudaMemsetAsync(h->prims.overflow, 0, (size_t)N, st));
     }
+    // the mask is kept by the u8 per-class kernel rendering exactly the tracked buffer; any other render into it resets the mask
+    uint32_t *sector_mask = h->obs_tracked && obs == h->obs_tracked && launch == P::CLASSES && obs_format == TC_OBS_CLASSES ? h->obs_mask : nullptr;
+    if (!sector_mask) TC_TRY(tc_obs_written(h, obs, tc_frame_bytes(h, obs_format), st));
     if (launch != P::UNFUSED && after_project) TC_CUDA(cudaEventRecord(after_project, st));
     switch (launch) {
     case P::ENVS: {
@@ -637,9 +662,10 @@ static int tc_launch_render(TcHandle *h, const uint8_t *mask, uint8_t *obs, int 
         fa.max_nodes = h->max_nodes; fa.max_edges = h->max_edges;
         fa.H = h->H; fa.W = h->W; fa.plane_words = h->plane_words_full;
         fa.pose = h->d_pose; fa.cam = h->d_cam; fa.thickness = h->d_thick; fa.mask = mask; fa.obs = obs;
+        fa.sector_mask = sector_mask;
         fa.timeline = timeline;
         const int grid = N * C;
-        const size_t sm = h->render_smem;
+        const size_t sm = h->render_smem + (sector_mask ? tc_sector_mask_smem_bytes(h->H, h->W) : 0);
         if (obs_format == TC_OBS_CLASSES_BITS) tc_render_classes_kernel<256, TC_FMT_BITS><<<grid, 256, sm, st>>>(fa);
         else if (obs_format == TC_OBS_CLASSES_BF16) tc_render_classes_kernel<256, TC_FMT_BF16><<<grid, 256, sm, st>>>(fa);
         else tc_render_classes_kernel<256, TC_FMT_U8><<<grid, 256, sm, st>>>(fa);
@@ -1043,9 +1069,59 @@ int tc_noise_blobs(TcHandle *h, uint8_t *dev_obs, uint64_t seed, uint32_t step, 
     na.n_envs = h->n_envs; na.n_cams = h->n_cams; na.n_classes = h->C; na.H = h->H; na.W = h->W; na.n_blobs = n_blobs; na.max_radius = max_radius;
     na.seed_lo = (uint32_t)seed; na.seed_hi = (uint32_t)(seed >> 32); na.step = step; na.env_offset = (uint32_t)env_index_offset;
     na.mask = dev_mask; na.obs = dev_obs;
+    TC_TRY(tc_obs_written(h, dev_obs, tc_frame_bytes(h, TC_OBS_CLASSES), (cudaStream_t)stream));
     tc_noise_blobs_kernel<<<h->n_views, 256, 0, (cudaStream_t)stream>>>(na);
     h->launches++;
     TC_CUDA(cudaGetLastError());
+    return TC_OK;
+}
+
+int tc_track_obs(TcHandle *h, uint8_t *dev_obs) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_track_obs: null handle");
+    if (dev_obs && h->obs_format != TC_OBS_CLASSES) return tc_fail(TC_ERR_INVALID, "tc_track_obs: only u8 class observations (TC_OBS_CLASSES) are tracked");
+    if (((uintptr_t)dev_obs & 31) != 0) return tc_fail(TC_ERR_INVALID, "tc_track_obs: dev_obs must be 32-byte aligned");
+    if (!dev_obs) {   // no CUDA call: switching off must work inside a stream capture (the memory goes with the next call or tc_destroy)
+        h->obs_tracked = nullptr;
+        return TC_OK;
+    }
+    TC_CUDA(cudaSetDevice(h->device));
+    TC_CUDA(cudaDeviceSynchronize());   // queued renders may still read or write the mask
+    // the mask is kept only where tc_render_classes_kernel renders these frames and a plane is whole sectors
+    const bool kept = !h->fused_all && h->fused_ok && ((size_t)h->H * h->W) % 32 == 0;
+    const size_t bytes = kept ? (size_t)h->n_views * h->C * tc_sector_mask_words(h->H, h->W) * 4 : 0;
+    if (bytes != h->obs_mask_bytes) {
+        cudaFree(h->obs_mask);
+        h->obs_mask = nullptr;
+        h->obs_mask_bytes = 0;
+        if (bytes) {
+            cudaError_t e = cudaMalloc((void **)&h->obs_mask, bytes);
+            if (e != cudaSuccess) { h->obs_mask = nullptr; h->obs_tracked = nullptr; return tc_fail(TC_ERR_ALLOC, std::string("cudaMalloc: ") + cudaGetErrorString(e)); }
+            h->obs_mask_bytes = bytes;
+        }
+    }
+    h->obs_tracked = kept ? dev_obs : nullptr;
+    if (h->obs_mask) {
+        TC_CUDA(cudaMemset(h->obs_mask, 0xFF, bytes));
+        TC_CUDA(cudaDeviceSynchronize());
+    }
+    return TC_OK;
+}
+
+int tc_invalidate_obs(TcHandle *h, void *stream) {
+    if (!h) return tc_fail(TC_ERR_INVALID, "tc_invalidate_obs: null handle");
+    if (!h->obs_tracked) return TC_OK;
+    TC_CUDA(cudaSetDevice(h->device));
+    TC_CUDA(cudaMemsetAsync(h->obs_mask, 0xFF, h->obs_mask_bytes, (cudaStream_t)stream));
+    return TC_OK;
+}
+
+int tc_obs_mask(TcHandle *h, uint32_t *dev_out, int64_t *host_words, void *stream) {
+    if (!h || !host_words) return tc_fail(TC_ERR_INVALID, "tc_obs_mask: null argument");
+    *host_words = h->obs_tracked ? (int64_t)(h->obs_mask_bytes / 4) : 0;
+    if (dev_out && *host_words) {
+        TC_CUDA(cudaSetDevice(h->device));
+        TC_CUDA(cudaMemcpyAsync(dev_out, h->obs_mask, h->obs_mask_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    }
     return TC_OK;
 }
 

@@ -57,6 +57,11 @@ __device__ __forceinline__ void tc_mbar_wait(uint64_t *bar, uint32_t phase) {
 __device__ __forceinline__ void tc_st_cs(void *p, uint4 v) {
     asm volatile("st.global.cs.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
+// 4-byte global -> shared copy that does not hold the issuing thread (cp.async); tc_cp_async_wait_all before reading it
+__device__ __forceinline__ void tc_cp_async4(void *dst_smem, const void *src_gmem) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(tc_smem_u32(dst_smem)), "l"(src_gmem) : "memory");
+}
+__device__ __forceinline__ void tc_cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // ------------------------------------------------------------------------------------------------ tracking
 struct TcTrackArgs {
@@ -474,6 +479,34 @@ __device__ __forceinline__ void tc_store_plane(uint8_t *out, size_t nbytes, cons
         out[i] = (any && ((plane[i >> 5] >> (i & 31)) & 1)) ? 255 : 0;
 }
 
+// The same for a tracked observation buffer (tc_track_obs): only the 32-byte sectors that hold a set pixel now, or held one
+// after the previous render, are stored; every other sector of `out` is known to be zero already. Sector s of the plane is
+// bytes [32s, 32s + 32) = plane word s; bit b of mask word w stands for sector 32w + b, set when the sector may be non-zero.
+// smask: the plane's mask words, copied to shared memory at kernel start; gmask: the same words in global memory, rewritten
+// where they change. The caller guarantees a 32-byte aligned `out` and nbytes % 32 == 0. A warp takes one mask word (32
+// sectors, 1024 bytes) at a time: lanes 2j and 2j+1 store the halves of sector j, so each store instruction writes whole sectors.
+template <int NT>
+__device__ __forceinline__ void tc_store_plane_tracked(uint8_t *out, uint32_t nbytes, const uint32_t *plane, bool any,
+                                                       const uint32_t *smask, uint32_t *gmask) {
+    const uint32_t lane = threadIdx.x & 31, nsec = nbytes >> 5, words = (nsec + 31) >> 5;
+    for (uint32_t w = threadIdx.x >> 5; w < words; w += NT / 32) {
+        const uint32_t old = smask[w], s0 = w << 5;
+        uint32_t nz = 0;
+        if (any) nz = __ballot_sync(0xffffffffu, s0 + lane < nsec && plane[s0 + lane] != 0u);
+        const uint32_t dirty = old | nz;   // warp-uniform
+        if (dirty == 0u) continue;
+#pragma unroll
+        for (uint32_t k = 0; k < 2; k++) {
+            const uint32_t sec = 16u * k + (lane >> 1);
+            if (((dirty >> sec) & 1u) && s0 + sec < nsec) {
+                const uint32_t b = any ? (plane[s0 + sec] >> (16u * (lane & 1u))) & 0xffffu : 0u;
+                tc_st_cs(out + 32u * (s0 + sec) + 16u * (lane & 1u), tc_expand16(b));
+            }
+        }
+        if (lane == 0 && nz != old) gmask[w] = nz;
+    }
+}
+
 // The same for the block-per-env kernels, whose time goes into instructions rather than into the stores: a frame is mostly
 // background, so the 0x00/0xFF expansion is skipped for the (97 % of) vectors whose 16 plane bits are all clear.
 // (Tried in round 2 and rejected: for aligned output, four half-word loads per thread and a warp ballot that writes 4 x 32 background
@@ -775,6 +808,7 @@ struct TcRenderArgs {
     const int32_t *thickness;  // [N]
     const uint8_t *mask;       // optional
     uint8_t *obs;              // [N,C,H,W]
+    uint32_t *sector_mask;     // u8 only, optional [N*C][ceil(H*W/1024)] (tc_track_obs): obs 32-byte aligned, H*W % 32 == 0
     long long *timeline;       // optional debug [N*C][10]: smid, clock at start / tables landed / geometry done / raster done / end
 };
 
@@ -790,6 +824,9 @@ __host__ __device__ inline size_t tc_render_smem_bytes(int max_nodes, int max_ed
     return tc_render_union_bytes(max_nodes, max_cblob_bytes, plane_words) + tc_render_segs_bytes(max_edges) +
            (size_t)TC_SETUP_CHUNK * TC_MAX_PRIMS_PER_SEG * sizeof(TcPrim) + (size_t)((max_edges + 15) & ~15);
 }
+// words of the sector mask of one plane, and the shared memory a tracked launch adds after tc_render_smem_bytes for them
+__host__ __device__ inline uint32_t tc_sector_mask_words(int H, int W) { return (uint32_t)(((size_t)H * W + 1023) >> 10); }
+__host__ __device__ inline size_t tc_sector_mask_smem_bytes(int H, int W) { return ((size_t)tc_sector_mask_words(H, W) * 4 + 15) & ~(size_t)15; }
 
 // per-block phase clocks for tools/timeline.py (tc_render_classes_kernel, tc_render_env_kernel): compiled in only with
 // -DTC_TIMELINE (the seven 64-bit counters cost registers and spills in the production build). TC_TL runs a statement on
@@ -837,6 +874,13 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
     const int n = cb.n_nodes, m = cb.n_edges;
     int4 *segs = (int4 *)(smem_raw + tc_render_union_bytes(a.max_nodes, a.max_cblob_bytes, a.plane_words));
     uint32_t *plane = (uint32_t *)smem_raw;
+    if (FMT == TC_FMT_U8 && a.sector_mask) {
+        // the plane's mask words travel to shared memory behind the camera pass; a load that the store phase waited for would
+        // stall it for the full memory latency
+        const uint32_t words = tc_sector_mask_words(a.H, a.W);
+        uint32_t *smask = (uint32_t *)(smem_raw + tc_render_smem_bytes(a.max_nodes, a.max_edges, a.max_cblob_bytes, a.plane_words));
+        for (uint32_t i = tid; i < words; i += NT) tc_cp_async4(smask + i, a.sector_mask + (size_t)blockIdx.x * words + i);
+    }
     {
         const size_t np = (size_t)((a.max_nodes + 15) & ~15);
         TcProjScratch sc;
@@ -887,6 +931,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
                 segs[slot] = make_int4(sc.ix[n0], sc.iy[n0], sc.ix[n1], sc.iy[n1]);
             }
         }
+        if (FMT == TC_FMT_U8 && a.sector_mask) tc_cp_async_wait_all();   // the mask words, visible to all after the barrier
         __syncthreads(); // scratch and tables are dead from here on; the plane takes their place
     }
     const int cnt = seg_cnt;
@@ -932,7 +977,11 @@ __global__ void __launch_bounds__(NT, 1024 / NT) tc_render_classes_kernel(const 
         tc_store_bits<NT>((uint32_t *)a.obs + (size_t)blockIdx.x * words, words, plane, cnt > 0);
     } else if (FMT == TC_FMT_BF16)
         tc_store_bf16<NT>((uint16_t *)a.obs + blockIdx.x * hw, (uint32_t)hw, plane, cnt > 0);
-    else tc_store_plane<NT>(a.obs + blockIdx.x * hw, hw, plane, cnt > 0);
+    else if (a.sector_mask) {
+        const uint32_t words = tc_sector_mask_words(a.H, a.W);
+        const uint32_t *smask = (const uint32_t *)(smem_raw + tc_render_smem_bytes(a.max_nodes, a.max_edges, a.max_cblob_bytes, a.plane_words));
+        tc_store_plane_tracked<NT>(a.obs + blockIdx.x * hw, (uint32_t)hw, plane, cnt > 0, smask, a.sector_mask + (size_t)blockIdx.x * words);
+    } else tc_store_plane<NT>(a.obs + blockIdx.x * hw, hw, plane, cnt > 0);
     TC_TL_RECORD(tl1, cnt);
 }
 

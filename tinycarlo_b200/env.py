@@ -150,6 +150,10 @@ class TinyCarloEnv(gc.Env):
         self._wrapped = bool(value)
         self._vec.set_wrapped(self._wrapped)
 
+    def invalidate_obs(self):
+        """TinyCarloVecEnv.invalidate_obs of the one-env vector env behind this env."""
+        self._vec.invalidate_obs()
+
     def _sync_flags(self):
         # env.py:77-81: observations are skipped only when no_observation is set and there is no render mode
         self._vec.no_observation = bool(self.no_observation and self.render_mode is None)

@@ -75,6 +75,11 @@ class TinyCarloGroupedVecEnv:
         for e in self.envs:
             e.set_wrapped(wrapped)
 
+    def invalidate_obs(self):
+        """TinyCarloVecEnv.invalidate_obs for every group's observation tensor."""
+        for e in self.envs:
+            e.invalidate_obs()
+
     def mark_done(self, mask: torch.Tensor):
         for e, sl in zip(self.envs, self._slices()):
             e.mark_done(mask[sl])

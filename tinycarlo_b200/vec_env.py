@@ -8,6 +8,16 @@ host synchronisation inside step() - resets and spawn draws included, so a rollo
 and no CPU implementation.
 
 Returned tensors are owned by the env and are overwritten by the next step()/reset(); clone what must survive.
+
+With large "classes" frames (those the library renders a block per env and class) the env tracks self.obs (tc_track_obs): a
+render stores only the 32-byte sectors of a frame that hold a set pixel now or did after the previous render, and leaves the
+rest, known to be zero, alone. The frames are the same bytes either way. Writes into self.obs that torch records in the
+tensor's version counter (an in-place op on it or on a view of it) are noticed before the next reset / step / step_host /
+render_obs / restore, and so is a new tensor assigned to env.obs. Writes that torch does not record - through `env.obs.data`,
+a raw pointer, a DLPack or __cuda_array_interface__ consumer, a collective into the buffer - must be followed by
+env.invalidate_obs() before the env renders again. Tracking is switched off for good by capture() and by a step inside any
+CUDA graph capture (a replay cannot check the version counter), and never switched on for an inference tensor
+(torch.inference_mode), which has no version counter.
 """
 import ctypes as C
 import os
@@ -159,6 +169,14 @@ class TinyCarloVecEnv:
             self._mask_all = torch.ones(N, dtype=torch.uint8, device=dev)
         self._outs = self._make_outputs(with_obs=True)
         self._outs_noobs = self._make_outputs(with_obs=False)
+        # tracking only where the library keeps a sector mask for these frames and torch records the tensor's writes
+        self._track_obs = False
+        self._obs_seen = (None, None)   # (data_ptr, _version) of self.obs when the env last rendered into it
+        if fmt == _lib.TC_OBS_CLASSES and not self.obs.is_inference() and self.obs.data_ptr() % 32 == 0:
+            with torch.cuda.device(dev):
+                _lib.check(self._L.tc_track_obs(self._h, _ptr(self.obs)), "tc_track_obs")
+            self._track_obs = self.obs_mask_words() > 0
+            self._obs_seen = (self.obs.data_ptr(), self.obs._version)
 
         # ---- parameters
         self._car_rows = np.tile(np.array(car_param_row(self.config["car"], self.T), np.float64), (N, 1))
@@ -206,6 +224,48 @@ class TinyCarloVecEnv:
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _sync_obs(self):
+        """Before every call that renders into self.obs: a new tensor is tracked (a buffer that is not 32-byte aligned is not),
+        and a write torch recorded since the last render (its version counter moved) makes every sector dirty again."""
+        if not self._track_obs:
+            return
+        o = self.obs
+        if o.is_inference() or torch.cuda.is_current_stream_capturing():
+            self._untrack_obs()
+            return
+        seen = (o.data_ptr(), o._version)
+        if seen == self._obs_seen:
+            return
+        if seen[0] != self._obs_seen[0]:
+            _lib.check(self._L.tc_track_obs(self._h, C.c_void_p(seen[0]) if seen[0] % 32 == 0 else None), "tc_track_obs")
+        else:
+            _lib.check(self._L.tc_invalidate_obs(self._h, self._stream()), "tc_invalidate_obs")
+        self._obs_seen = seen
+
+    def _untrack_obs(self):
+        """for good: every later render stores whole frames (tc_track_obs(NULL) makes no CUDA call, so a capture may be running)"""
+        _lib.check(self._L.tc_track_obs(self._h, None), "tc_track_obs")
+        self._track_obs = False
+
+    def obs_mask_words(self, out: Optional[torch.Tensor] = None) -> int:
+        """Words of the sector mask the library keeps for self.obs (0: not tracked); with `out` (int32 CUDA tensor of at least
+        that many elements) a copy of the mask, ordered on the current stream: bit b of word w = sector 32w+b may be non-zero."""
+        n = C.c_int64()
+        _lib.check(self._L.tc_obs_mask(self._h, None, C.byref(n), None), "tc_obs_mask")
+        if out is not None and n.value:
+            if out.device != self.device or out.dtype != torch.int32 or not out.is_contiguous() or out.numel() < n.value:
+                raise ValueError(f"obs_mask_words: out must be a contiguous int32 tensor on {self.device} of at least {n.value} elements")
+            with torch.cuda.device(self.device):
+                _lib.check(self._L.tc_obs_mask(self._h, _ptr(out), C.byref(n), self._stream()), "tc_obs_mask")
+        return int(n.value)
+
+    def invalidate_obs(self):
+        """Declares that something other than this env wrote self.obs in a way torch does not record (raw pointer, DLPack /
+        __cuda_array_interface__ consumer, collective): the next render stores whole frames (ordered on the current stream)."""
+        if self._track_obs:
+            with torch.cuda.device(self.device):
+                _lib.check(self._L.tc_invalidate_obs(self._h, self._stream()), "tc_invalidate_obs")
 
     def _upload_params(self):
         """Car and camera rows to the device. Nothing here waits for the device: the library decides from the host copy of the
@@ -388,6 +448,7 @@ class TinyCarloVecEnv:
             if self.autoreset:
                 self.done_flags.masked_fill_(mask_u8.bool(), 0)
             outs = self._outs if not self.no_observation else self._outs_noobs
+            self._sync_obs()
             _lib.check(self._L.tc_reset(self._h, _ptr(mask_u8), _ptr(nodes), C.byref(outs), self._stream()), "tc_reset")
             self._was_reset = True
         return self.obs, self._info()
@@ -409,6 +470,7 @@ class TinyCarloVecEnv:
         if not self._was_reset:
             raise _lib.TinyCarloError("call reset() before step()")
         fn = self._L.tc_step_f64 if f64 else self._L.tc_step
+        self._sync_obs()
         if self._debug and not torch.cuda.is_current_stream_capturing():
             with torch.cuda.device(self.device):
                 self.profile_begin(1)
@@ -436,6 +498,8 @@ class TinyCarloVecEnv:
         if not self._was_reset:
             raise _lib.TinyCarloError("call reset() before capture()")
         dbg, self._debug = self._debug, False
+        if self._track_obs:   # replays keep full stores: nothing can check the buffer's version between them
+            self._untrack_obs()
 
         def one():
             if policy_fn is None:
@@ -484,6 +548,7 @@ class TinyCarloVecEnv:
                 raise ValueError(f"step_host: {name} must be a contiguous host tensor of dtype {dt} and shape {shape}")
         outs = self._outs if not self.no_observation else self._outs_noobs
         with torch.cuda.device(self.device):
+            self._sync_obs()
             if obs_host is None:
                 _lib.check(self._L.tc_step_host(self._h, _ptr(car_control), _ptr(maneuver), C.byref(outs), _ptr(reward), _ptr(terminated),
                                                 _ptr(truncated), _ptr(cte), _ptr(heading_error), self._stream()), "tc_step_host")
@@ -566,6 +631,7 @@ class TinyCarloVecEnv:
         """Re-render self.obs (all views) at the current poses (after load_state_dict / set_camera_params); mask is per env."""
         with torch.cuda.device(self.device):
             m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            self._sync_obs()
             _lib.check(self._L.tc_render(self._h, _ptr(m), _ptr(self.obs), self._fmt, _ptr(self.out.get("seg_count")),
                                          _ptr(self.out.get("seg_i32")), self._stream()), "tc_render")
         return self.obs
